@@ -3,7 +3,7 @@
 shadow)" and "SPPM iterations/sec"; one invocation measures one workload as THE line and (for the default workload)
 carries the SPPM workloads as complete sub-lines under "sppm".
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 Whitted workloads (metric Mrays/s; a step = one full render):
   tess-1M   BASELINE.json configs[2] (C3): 1920x1080, 16 spp, depth 5, 999 840 triangles, Glass/Matte/Mirror  [default]
@@ -23,6 +23,11 @@ communicator id, the barriers and the max-over-ranks of the timings.
 
 --impl reference: the CPU restatement of the reference (oracle/, C++, std::thread over tiles / photons, all host cores)
 on the same workload; the product's native library is not loaded in that process.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what each timed path handed its caller after its last timed step
+as DIR/<name>.npy (float32): film_<workload>.npy, the Whitted film (H, W, 4: X, Y, Z, filter weight), and
+image_<workload>.npy, the SPPM image (H, W, 3).  Scenes and seeds depend on the arguments only, so two builds run with
+the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -52,6 +57,7 @@ SPPM_WORKLOADS = {
     "sppm-caustic-moving": ("caustic_moving", dict(resolution=1024), 25),
     "sppm-shadows-small": ("shadows", dict(resolution=96), 8),
 }
+DUMP_BYTES = 64_000_000                     # --dump-outputs: all files together, .npy headers included
 METRIC_WHITTED = "Mrays/sec (closest-hit + shadow)"
 METRIC_SPPM = "SPPM iterations/sec"
 L2_NOTE_WHITTED = "inputs larger than L2 (ray queues + BVH > 126 MB per step)"
@@ -74,6 +80,25 @@ def load_profile_table(name):
         return json.load(open(p))
     except Exception:
         return {}
+
+
+def dump_outputs(outputs, path):
+    """Write {name: (H, W, C) array} as path/<name>.npy in float32, DUMP_BYTES in all.  Smallest first, each array gets at
+    most an equal share of what is left; one larger than its share is replaced by a seeded sample of its pixels (rows of
+    the (H * W, C) view, in raster order), the same sample for the same shape."""
+    os.makedirs(path, exist_ok=True)
+    items = sorted(outputs.items(), key=lambda kv: kv[1].nbytes)
+    left = DUMP_BYTES
+    for k, (name, a) in enumerate(items):
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        share = left // (len(items) - k) - 1024                  # (room for the .npy header)
+        if a.nbytes > share:
+            px = a.reshape(a.shape[0] * a.shape[1], -1)
+            keep = np.random.default_rng(0).choice(len(px), share // px[0].nbytes, replace=False)
+            a = px[np.sort(keep)]
+        f = os.path.join(path, name + ".npy")
+        np.save(f, a)
+        left -= os.path.getsize(f)
 
 
 class ClockSampler:
@@ -261,6 +286,7 @@ class Env:
         from trace_jl_b200 import distributed as D
         self.torch, self.dist, self.T, self.D, self.args = torch, dist, T, D, args
         self.t_start = time.perf_counter()
+        self.outputs = {}                                   # --dump-outputs: name -> array after the last timed step
         self.world = int(os.environ.get("WORLD_SIZE", "1"))
         self.rank = int(os.environ.get("RANK", "0"))
         self.local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -355,6 +381,8 @@ def bench_whitted(env, workload, with_extras=True):
     ms_total, _ = env.timed(lambda i: step(args.warmup + i), args.steps)
     st = ctx.stats()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:              # (later passes keep accumulating into the same film)
+        env.outputs[f"film_{workload}"] = film_dev.cpu().numpy()
     rays_e, rays_s, launches, prim_rays, prim_hits = env.sum_over_ranks(
         [st["rays_extend"], st["rays_shadow"], st["kernel_launches"], st["primary_rays"], st["primary_hits"]])
     total_rays = rays_e + rays_s
@@ -518,6 +546,8 @@ def bench_sppm(env, workload, steps, warmup, cpu_baseline=True):
     ms, _ = env.timed(lambda i: sess.step(steps), 1)
     clocks = sampler.stop() if rank == 0 else None
     st = ctx.stats()
+    if args.dump_outputs:                           # (every rank: with several ranks the image is an all-gather)
+        env.outputs[f"image_{workload}"] = sess.image()
     launches = sum(env.sum_over_ranks([st["kernel_launches"]]))
     value = steps / (ms * 1e-3)
     env.note(f"{workload}: timed iterations done ({value:.0f} it/s)")
@@ -681,8 +711,12 @@ def main():
     ap.add_argument("--no-optin", action="store_true", help="skip the extra measurement on the opt-in SAH tree")
     ap.add_argument("--sppm-workloads", default="sppm-shadows-1024,sppm-caustic-moving,sppm-caustic-glass-d8",
                     help="SPPM sub-lines carried by the default Whitted line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, 64 MB in all; GPU arm)")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the GPU arm; it has no meaning with --impl reference")
         return run_reference(args)
     env = Env(args)
     if args.workload in SPPM_WORKLOADS:
@@ -692,12 +726,14 @@ def main():
     else:
         out = bench_whitted(env, args.workload)
         if not args.no_sppm:
-            # the metric's second half: every SPPM workload as a complete line of its own (value, e2e, roofline, cpu_baseline)
-            # (30 iterations per timed call: with sppm_pipeline iterations in flight, fill and drain are part of the timed region)
-            out["sppm"] = [bench_sppm(env, wl, 30, 4, cpu_baseline=True) for wl in args.sppm_workloads.split(",") if wl]
+            # the metric's second half: every SPPM workload as a complete line of its own (value, e2e, roofline, cpu_baseline),
+            # K timed iterations each (with sppm_pipeline iterations in flight, fill and drain are part of the timed region)
+            out["sppm"] = [bench_sppm(env, wl, args.steps, args.warmup, cpu_baseline=True) for wl in args.sppm_workloads.split(",") if wl]
             if env.world > 1:
                 out["sppm"].append({"sharded_vs_single_gpu_check": sppm_sharding_check(env)})
     if env.rank == 0:
+        if args.dump_outputs:
+            dump_outputs(env.outputs, args.dump_outputs)
         print(json.dumps(out))
     env.ctx.close()
     if env.world > 1:

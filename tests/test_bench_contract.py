@@ -1,10 +1,15 @@
 """bench.py contract pieces that can be checked without a GPU: the reference arm prints one JSON line with the agreed keys
 (it times the CPU restatement on a bounded sample), ranks other than 0 stay silent, and our own arm refuses to run
-without a CUDA device instead of falling back to anything."""
+without a CUDA device instead of falling back to anything.  With a GPU (-m gpu): --dump-outputs writes what the timed
+steps computed."""
+import ctypes as C
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -73,3 +78,62 @@ def test_both_arms_share_one_config():
     import bench
     src = open(os.path.join(ROOT, "bench.py")).read()
     assert src.count('"config": whitted_config(') == 2 and src.count('"config": sppm_config(') == 2
+
+
+def test_dump_outputs_budget_and_sample(tmp_path):
+    """Outputs that fit are written whole; one that does not is replaced by the same seeded sample of whole pixels on
+    every run, and all files together stay within DUMP_BYTES."""
+    sys.path.insert(0, ROOT)
+    import bench
+    big = np.random.default_rng(3).random((2048, 2048, 4), dtype=np.float32)      # 64 MiB on its own
+    big[..., 0] = np.arange(2048 * 2048, dtype=np.float32).reshape(2048, 2048)     # channel 0 names the pixel
+    small = np.random.default_rng(4).random((64, 48, 3), dtype=np.float32)
+    for d in ("a", "b"):
+        bench.dump_outputs({"big": big, "small": small}, str(tmp_path / d))
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["big.npy", "small.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= bench.DUMP_BYTES
+    assert np.array_equal(np.load(tmp_path / "a" / "small.npy"), small)
+    a, b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert a.dtype == np.float32 and a.shape[1] == 4 and len(a) > 3_000_000 and np.array_equal(a, b)
+    idx = a[:, 0].astype(np.int64)
+    assert np.all(np.diff(idx) > 0) and np.array_equal(a, big.reshape(-1, 4)[idx])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_step(T, tmp_path):
+    """The dumped Whitted film is the film after warm-up + K renders (seeds 1000, 1001, ...; it accumulates), the dumped
+    SPPM image the image after max(3, W) + K iterations; both equal the same work done directly through the library, up to
+    the order of the float atomics."""
+    steps, warmup = 3, 2
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "tess-small", "--steps", str(steps),
+                        "--warmup", str(warmup), "--no-cpu-baseline", "--no-optin", "--sppm-workloads", "sppm-shadows-small",
+                        "--dump-outputs", str(tmp_path)], cwd=ROOT, capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-3000:]
+    d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])
+    assert d["steps"] == steps and d["sppm"][0]["steps"] == steps
+    assert sorted(os.listdir(tmp_path)) == ["film_tess-small.npy", "image_sppm-shadows-small.npy"]
+    sys.path.insert(0, ROOT)
+    import bench
+    from trace_jl_b200 import distributed as D
+    ctx = T.Context(0)
+    try:
+        scene, camera, spp, depth = bench.build_scene(T, "tess-small")
+        ctx.upload(scene)
+        cam, fd = camera.pod(), camera.film.desc()
+        want = np.zeros_like(camera.film.pixels)
+        for i in range(warmup + steps):
+            ctx.check(ctx.lib.trace_render_whitted(ctx.h, C.byref(cam), C.byref(fd), spp, depth, C.c_uint64(1000 + i), T._lib.ptr(want)))
+        film = np.load(tmp_path / "film_tess-small.npy")
+        assert film.dtype == np.float32 and film.shape == want.shape and float(want[..., 3].min()) > 0
+        assert np.allclose(film, want, rtol=1e-5, atol=1e-6), float(np.abs(film - want).max())
+        scene, camera, p = bench.build_sppm_scene(T, "sppm-shadows-small")
+        sess = D.SPPMSession(ctx, scene, camera, p["r0"], p["max_depth"], p["photons"], 0x5EED0001)
+        sess.step(max(3, warmup) + steps)
+        want = sess.image()
+        sess.close()
+        img = np.load(tmp_path / "image_sppm-shadows-small.npy")
+        assert img.dtype == np.float32 and img.shape == want.shape and float(want.max()) > 0
+        assert np.allclose(img, want, rtol=2e-4, atol=1e-6), float(np.abs(img - want).max())
+    finally:
+        ctx.close()
