@@ -157,6 +157,14 @@ int     trace_bvh_build(const float* prim_bounds /* [n][6] = min xyz, max xyz */
 /* opt-in: conventional binned SAH (primitive-count weighted, empty buckets, leaves up to max_node_primitives) in the same
  * node format.  Not the reference's tree: closest hits agree except for ties between equal t (SURVEY.md §8f.2). */
 int     trace_bvh_build_sah(const float* prim_bounds, int64_t n, int max_node_primitives, trace_bvh** out);
+/* opt-in: LBVH (Karras 2012 radix tree over 63-bit Morton codes of the centroids) built on GPU `device`, in the same
+ * node format; the tree comes back as an ordinary host trace_bvh handle (trace_bvh_num_nodes / _copy / _free apply).
+ * Not the reference's tree: closest hits agree except for ties between equal t.  max_node_primitives is clamped to
+ * 1..255; a range of at most that many primitives is one leaf.  Synchronous; the caller's current device is restored;
+ * TRACE_BVH_PROFILE=1 prints per-phase CUDA-event times to stderr.  Return codes as trace_bvh_build, plus 6: the tree
+ * is deeper than the traversal stack (64 levels; builder "sah" handles such inputs), 7: CUDA error / no device (there
+ * is no CPU fallback). */
+int     trace_bvh_build_gpu(int device, const float* prim_bounds, int64_t n, int max_node_primitives, trace_bvh** out);
 int64_t trace_bvh_num_nodes(const trace_bvh* bvh);
 int64_t trace_bvh_num_prims(const trace_bvh* bvh);
 int     trace_bvh_copy(const trace_bvh* bvh, trace_bvh_node* nodes_out, uint32_t* prim_order_out);

@@ -72,6 +72,7 @@ _P = C.c_void_p
 SIGNATURES = {
     "trace_bvh_build": (C.c_int, [_P, C.c_int64, C.c_int, C.POINTER(_P)]),
     "trace_bvh_build_sah": (C.c_int, [_P, C.c_int64, C.c_int, C.POINTER(_P)]),
+    "trace_bvh_build_gpu": (C.c_int, [C.c_int, _P, C.c_int64, C.c_int, C.POINTER(_P)]),
     "trace_bvh_num_nodes": (C.c_int64, [_P]),
     "trace_bvh_num_prims": (C.c_int64, [_P]),
     "trace_bvh_copy": (C.c_int, [_P, _P, _P]),

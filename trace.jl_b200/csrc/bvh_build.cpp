@@ -637,6 +637,19 @@ extern "C" int trace_bvh_build_sah(const float* pb, int64_t n, int max_node_prim
     return build_entry<SahSplitter>(pb, n, m, out);
 }
 
+// The handle for builders outside this file (bvh_gpu.cu): arrays of the given sizes, left uninitialised for the caller
+// to fill; nullptr when out of memory.
+trace_bvh* bvh_alloc(int64_t n_nodes, int64_t n_prims, trace_bvh_node** nodes, uint32_t** order) {
+    try {
+        std::unique_ptr<trace_bvh> bvh(new trace_bvh());
+        bvh->nodes.resize((size_t)n_nodes);
+        bvh->order.resize((size_t)n_prims);
+        *nodes = bvh->nodes.data();
+        *order = bvh->order.data();
+        return bvh.release();
+    } catch (...) { return nullptr; }
+}
+
 extern "C" int64_t trace_bvh_num_nodes(const trace_bvh* b) { return b ? (int64_t)b->nodes.size() : 0; }
 extern "C" int64_t trace_bvh_num_prims(const trace_bvh* b) { return b ? (int64_t)b->order.size() : 0; }
 extern "C" int trace_bvh_copy(const trace_bvh* b, trace_bvh_node* nodes_out, uint32_t* order_out) {

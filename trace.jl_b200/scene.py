@@ -332,11 +332,13 @@ class BVHAccel:
     """BVHAccel(primitives, max_node_primitives = 1), src/accel/bvh.jl:50-80.  The build itself is
     trace_bvh_build in libtrace_cuda.so's host part (the reference's SAH split logic)."""
 
-    def __init__(self, primitives, max_node_primitives=1, builder="reference"):
+    def __init__(self, primitives, max_node_primitives=1, builder="reference", device=0):
         """builder = "reference": the reference's split logic, bit-identical tree (src/accel/bvh.jl:55-206).
-        builder = "sah": opt-in conventional binned SAH (trace_bvh_build_sah) - same hits, ties aside; less traversal."""
-        if builder not in ("reference", "sah"):
-            raise ValueError("builder must be 'reference' or 'sah'")
+        builder = "sah": opt-in conventional binned SAH (trace_bvh_build_sah) - same hits, ties aside; less traversal.
+        builder = "lbvh": opt-in LBVH built on GPU `device` (trace_bvh_build_gpu) - same hits, ties aside; `device` is
+        used by this builder only (multi-rank callers pass their own GPU)."""
+        if builder not in ("reference", "sah", "lbvh"):
+            raise ValueError("builder must be 'reference', 'sah' or 'lbvh'")
         self.builder = builder
         self.max_node_primitives = min(255, int(max_node_primitives))
         self.items = _expand(primitives)
@@ -366,10 +368,18 @@ class BVHAccel:
             return
         lib = _lib.load()
         h = C.c_void_p()
-        build = lib.trace_bvh_build if builder == "reference" else lib.trace_bvh_build_sah
-        rc = build(_lib.ptr(self.prim_bounds), self.n_primitives, self.max_node_primitives, C.byref(h))
-        if rc != 0:
-            raise RuntimeError(f"trace_bvh_build failed ({rc})")
+        if builder == "lbvh":
+            rc = lib.trace_bvh_build_gpu(int(device), _lib.ptr(self.prim_bounds), self.n_primitives,
+                                         self.max_node_primitives, C.byref(h))
+            if rc != 0:
+                cause = {5: "NaN bounds", 6: "tree deeper than 64 levels: use builder='sah'",
+                         7: f"CUDA error or no CUDA device (device {device}); there is no CPU fallback"}.get(rc, "")
+                raise RuntimeError(f"trace_bvh_build_gpu failed ({rc}): {cause}")
+        else:
+            build = lib.trace_bvh_build if builder == "reference" else lib.trace_bvh_build_sah
+            rc = build(_lib.ptr(self.prim_bounds), self.n_primitives, self.max_node_primitives, C.byref(h))
+            if rc != 0:
+                raise RuntimeError(f"trace_bvh_build failed ({rc})")
         try:
             self.nodes = np.zeros(lib.trace_bvh_num_nodes(h), dtype=_lib.node_dtype)
             self.order = np.zeros(lib.trace_bvh_num_prims(h), dtype=np.uint32)
