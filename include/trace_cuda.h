@@ -225,6 +225,37 @@ int trace_comm_info(const trace_ctx* ctx, int* rank, int* world, int* nccl_versi
 
 int trace_scene_upload(trace_ctx* ctx, const trace_scene_desc* scene);
 
+/* ---- refit (extension: the reference has no counterpart; it rebuilds BVHAccel).  New positions for the triangles of
+ * the last upload, with the tree's topology kept (node structure, primitive order, materials, spheres, lights) and every
+ * box recomputed on the GPU.  The result is exactly the scene trace_scene_upload would build from the same nodes and
+ * primitives with the new vertices and these boxes:
+ *   tri_vertices  [n_tris][3][3] world space, the triangle order of trace_scene_desc.tri_vertices; n_tris must be the
+ *                 uploaded count.  The degenerate test is decided again (upload's unfused dot(g, g) == 0).
+ *   tri_normals   same layout or NULL (keep the current normals); applied only to triangles uploaded with
+ *                 TRACE_TRI_HAS_NORMALS.
+ *   sphere_bounds [n_spheres][6] = min xyz, max xyz, host memory: the bounds the tree was built with (the spheres do not
+ *                 move).  Required when the scene holds spheres, NULL otherwise.
+ *   leaf box      Julia min / max (-0.0 < +0.0) union of its primitives' bounds (a triangle: its three vertices); a
+ *                 zero-primitive leaf keeps its box and adds nothing to its parent's;
+ *   interior box  Julia min / max union of its two children's boxes.  A refit with unchanged vertices therefore gives
+ *                 back the uploaded boxes of the reference, sah and lbvh trees (float ==; the sign of a zero may differ);
+ *   scene_scale   recomputed from the new root box with the upload's rule.
+ * Refused, with the scene untouched: no scene uploaded, another triangle count, a scene with spheres and no (or the
+ * wrong number of) sphere bounds, NaN in any vertex, normal or sphere bound.  The call first waits for all of the
+ * context's work (an asynchronous SPPM session included) and ends any SPPM session, as trace_scene_upload does; it is
+ * synchronous, so the caller may reuse its buffers on return.  Device buffers are rewritten in place: a captured Whitted
+ * graph stays valid and replays over the new data (a changed scene_scale recaptures it).  Deterministic (bit-identical
+ * for the same input); local to the context (no collectives: every rank refits with the same vertices).
+ * TRACE_BVH_PROFILE=1 prints per-phase CUDA-event times to stderr. */
+int trace_scene_refit(trace_ctx* ctx, int64_t n_tris, const float* tri_vertices, const float* tri_normals,
+                      int64_t n_spheres, const float* sphere_bounds);
+/* the same with vertices (and normals, or NULL) in device memory on the context's GPU, read on the context's stream:
+ * the caller orders the work that wrote them before this call.  sphere_bounds stays in host memory. */
+int trace_scene_refit_device(trace_ctx* ctx, int64_t n_tris, const void* tri_vertices_device,
+                             const void* tri_normals_device, int64_t n_spheres, const float* sphere_bounds);
+/* the uploaded scene's current nodes (n_nodes of the last upload), boxes as refit last left them */
+int trace_scene_copy_nodes(trace_ctx* ctx, trace_bvh_node* nodes_out);
+
 /* ---- ray queries, host buffers. o,d: [n][3]; tmax_inout: [n] (t of the hit on return, unchanged on a miss);
  * prim_out: [n] original index + 1, 0 = miss; b0b1_out: [n][2] barycentrics (triangles) or 0; may be NULL. ---- */
 int trace_intersect(trace_ctx* ctx, const float* o, const float* d, float* tmax_inout, int64_t n,

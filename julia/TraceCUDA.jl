@@ -168,8 +168,11 @@ mutable struct FlatScene
     lights::Vector{LightP}
     material_ids::IdDict{Any,UInt32}
     n_original::UInt32                 # running "caller's order" primitive number
+    triangles::Vector{Any}             # the Trace.Triangle behind each tri_vertices entry (refit! gathers from them)
+    sphere_bounds::Vector{Float32}     # [n_spheres][6] world bounds the tree was built with
 end
-FlatScene() = FlatScene(BVHNode[], Prim[], Float32[], Float32[], UInt8[], SphereP[], MaterialP[], LightP[], IdDict{Any,UInt32}(), 0)
+FlatScene() = FlatScene(BVHNode[], Prim[], Float32[], Float32[], UInt8[], SphereP[], MaterialP[], LightP[], IdDict{Any,UInt32}(), 0,
+                        Any[], Float32[])
 
 function material_id!(fs::FlatScene, m)
     m === nothing && return NO_MATERIAL          # fine for intersect!/intersect_p; the integrators refuse such scenes
@@ -191,6 +194,7 @@ function prim_row!(fs::FlatScene, p::Trace.GeometricPrimitive{Trace.Triangle})
         append!(fs.tri_normals, has_n ? Float32.(Tuple(t.mesh.normals[k])) : ZERO3)
     end
     push!(fs.tri_flags, UInt8(flips(t.core)) | (UInt8(has_n) << 1))
+    push!(fs.triangles, t)
     row = Prim(PRIM_TRIANGLE, UInt32(length(fs.tri_flags) - 1), material_id!(fs, p.material), fs.n_original)
     fs.n_original += 1
     row
@@ -199,6 +203,8 @@ function prim_row!(fs::FlatScene, p::Trace.GeometricPrimitive{Trace.Sphere})
     s = p.shape
     push!(fs.spheres, SphereP(rowmajor(s.core.object_to_world.m), rowmajor(s.core.object_to_world.inv_m), s.radius,
                               s.z_min, s.z_max, s.θ_min, s.θ_max, s.ϕ_max, UInt32(flips(s.core)), 0))
+    b = Trace.world_bound(s)
+    append!(fs.sphere_bounds, Float32.((b.p_min..., b.p_max...)))
     row = Prim(PRIM_SPHERE, UInt32(length(fs.spheres) - 1), material_id!(fs, p.material), fs.n_original)
     fs.n_original += 1
     row
@@ -252,6 +258,23 @@ function upload!(ctx::Context, scene::Trace.Scene)
                      length(fs.lights), pointer(fs.lights))
     GC.@preserve fs check(ctx, ccall((:trace_scene_upload, LIB), Cint, (Ptr{Cvoid}, Ref{SceneDesc}), ctx.h, desc))
     UPLOADED[ctx] = (scene, fs)
+    nothing
+end
+
+# Animation: move the vertices of the scene's meshes (mesh.vertices[k] = ...), then refit!(ctx, scene) instead of
+# building a new BVHAccel.  The tree's topology stays; the library recomputes every box on the GPU (trace_scene_refit).
+# Every context that holds the scene (one per GPU) is refit with the same vertices.  A deformation computed on the GPU
+# can skip the gather and pass a device buffer to trace_scene_refit_device instead.
+function refit!(ctx::Context, scene::Trace.Scene)
+    haskey(UPLOADED, ctx) && UPLOADED[ctx][1] === scene || error("TraceCUDA.refit!: this scene is not the one uploaded to ctx")
+    fs = UPLOADED[ctx][2]
+    v = Vector{Float32}(undef, 9 * length(fs.triangles))
+    for (j, t) in enumerate(fs.triangles), (c, k) in enumerate(t.mesh.indices[t.i:t.i + 2])
+        v[9 * (j - 1) + 3 * (c - 1) .+ (1:3)] .= Float32.(Tuple(t.mesh.vertices[k]))
+    end
+    GC.@preserve v fs check(ctx, ccall((:trace_scene_refit, LIB), Cint,
+        (Ptr{Cvoid}, Int64, Ptr{Float32}, Ptr{Float32}, Int64, Ptr{Float32}),
+        ctx.h, length(fs.triangles), v, C_NULL, length(fs.spheres), isempty(fs.spheres) ? C_NULL : pointer(fs.sphere_bounds)))
     nothing
 end
 

@@ -90,6 +90,9 @@ SIGNATURES = {
     "trace_comm_destroy": (C.c_int, [_P]),
     "trace_comm_info": (C.c_int, [_P, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "trace_scene_upload": (C.c_int, [_P, C.POINTER(SceneDesc)]),
+    "trace_scene_refit": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int64, _P]),
+    "trace_scene_refit_device": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int64, _P]),
+    "trace_scene_copy_nodes": (C.c_int, [_P, _P]),
     "trace_intersect": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P]),
     "trace_occluded": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P]),
     "trace_intersect_device": (C.c_int, [_P, _P, _P, C.c_int64, _P]),

@@ -89,7 +89,8 @@ extern "C" void trace_destroy(trace_ctx* c) {
     cudaStreamSynchronize(c->stream);
     sppm_free(c);
     trace_comm_destroy(c);
-    DevBuf* all[] = {&c->b_nodes, &c->b_pairs, &c->b_prims, &c->b_tnorm, &c->b_spheres, &c->b_materials, &c->b_lights, &c->b_counters};
+    DevBuf* all[] = {&c->b_nodes, &c->b_pairs, &c->b_prims, &c->b_tnorm, &c->b_spheres, &c->b_materials, &c->b_lights, &c->b_counters,
+                     &c->refit.topo, &c->refit.stage, &c->refit.sphere_bounds};
     for (DevBuf* b : all) b->release();
     for (auto& b : c->b_query) b.release();
     for (auto& b : c->b_queue) b.release();
@@ -226,6 +227,7 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
         }
     }
     std::vector<float4> prims((size_t)d->n_prims * 3), tnorm((size_t)d->n_prims * 3);
+    std::vector<uint32_t> tri_index((size_t)d->n_prims, 0u);        // kept for trace_scene_refit
     for (int64_t i = 0; i < d->n_prims; ++i) {
         const trace_prim& p = d->prims[i];
         float4 A = make_float4(0, 0, 0, 0), B = A, C = A, N0 = A, N1 = A, N2 = A;
@@ -238,6 +240,7 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
             const float3 p0 = f3(v[0], v[1], v[2]), p1 = f3(v[3], v[4], v[5]), p2 = f3(v[6], v[7], v[8]);
             const float3 g = cross3(p2 - p0, p1 - p0);
             if (dot3(g, g) == 0.0f) tag = TR_PRIM_DEGENERATE_BIT;
+            tri_index[i] = p.index;
             flags = d->tri_flags ? d->tri_flags[p.index] : 0;
             if (!d->tri_normals) flags &= ~(uint32_t)TRACE_TRI_HAS_NORMALS;
             if (flags & TRACE_TRI_HAS_NORMALS) {
@@ -258,9 +261,9 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
     // Preorder numbering: interior node i gets pair index = number of interior nodes before it.
     std::vector<float4> pairs;
     uint32_t root_ref = 0;
+    uint32_t n_pairs = 0;
     {
         std::vector<uint32_t> pair_of((size_t)d->n_nodes, 0);
-        uint32_t n_pairs = 0;
         for (int64_t i = 0; i < d->n_nodes; ++i) if ((d->nodes[i].meta >> 30) != 3) pair_of[i] = n_pairs++;
         if (n_pairs >= 0x40000000u) return c->fail("scene: too many interior nodes");
         pairs.resize((size_t)n_pairs * 4);
@@ -369,6 +372,9 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
         }
     }
     c->have_scene = true;
+    c->refit.tri_index.swap(tri_index);
+    c->refit.n_tris = d->n_tris; c->refit.n_spheres = d->n_spheres; c->refit.n_pairs = n_pairs;
+    c->refit.topo_ready = false;
     sppm_end_session(c);
     return 0;
 }

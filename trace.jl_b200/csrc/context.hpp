@@ -116,6 +116,25 @@ struct trace_ctx {
     DeviceScene scene{};
     DevBuf b_nodes, b_pairs, b_prims, b_tnorm, b_spheres, b_materials, b_lights;
 
+    // refit (refit.cu): what trace_scene_refit needs of the last upload.  The host keeps only the BVH-slot -> triangle
+    // map; the device topology (parents, pair slots, leaf list) is derived from b_nodes at the first refit after an
+    // upload, so scenes that are never refit pay no device memory for it.
+    struct Refit {
+        std::vector<uint32_t> tri_index;   // [n_prims] trace_prim.index of triangle slots (0 for spheres)
+        int64_t n_tris = 0, n_spheres = 0, n_pairs = 0;
+        bool topo_ready = false;
+        DevBuf topo, stage, sphere_bounds;
+        // carved out of `topo` (refit.cu)
+        int32_t* parent = nullptr;         // [n_nodes] parent node, -1 at the root
+        uint32_t* up = nullptr;            // [n_nodes] 2 * parent's pair index + child slot (0: first, 1: second)
+        uint32_t* pair_of = nullptr;       // [n_nodes] interior: its pair index (exclusive scan of "is interior")
+        uint32_t* leaves = nullptr;        // [n_nodes - n_pairs] leaf node ids
+        uint8_t* empty = nullptr;          // [n_nodes] subtree holds no primitive (per call)
+        uint32_t* arrive = nullptr;        // [n_pairs] arrival counters (reset per call)
+        uint32_t* slot_tri = nullptr;      // [n_prims] tri_index on the device
+        uint32_t* status = nullptr;        // [0] NaN vertex seen
+    } refit;
+
     // scratch
     DevBuf b_query[4];            // ray query staging
     DevBuf b_queue[16];           // wavefront queues
@@ -277,3 +296,5 @@ int whitted_render_device(trace_ctx* ctx, const trace_camera* cam, const trace_f
 void sppm_free(trace_ctx* ctx);
 void sppm_end_session(trace_ctx* ctx);
 void whitted_film_range(const trace_ctx* ctx, long long npix, long long* p0, long long* p1);
+// implemented in refit.cu: waits for every stream of the context (caller's, lanes, SPPM chain / collectives, copies)
+int ctx_drain(trace_ctx* ctx);

@@ -164,6 +164,7 @@ class Context:
 
     def __init__(self, device=0, stream=None):
         self.lib = _lib.load()
+        self.device = int(device)
         self.h = C.c_void_p()
         self.stream_handle = int(stream) if stream else 0
         rc = self.lib.trace_create(C.byref(self.h), int(device), C.c_void_p(stream) if stream else None)
@@ -198,10 +199,64 @@ class Context:
     def upload(self, scene):
         flat = scene.flatten()
         if self._scene is not flat:
+            if flat.stale:
+                raise RuntimeError("this scene was refit on a context and its host nodes / vertices are stale: upload it "
+                                   "before refitting and refit every context with the same vertices, or build a new "
+                                   "BVHAccel for the moved geometry")
             d = flat.desc()
             self.check(self.lib.trace_scene_upload(self.h, C.byref(d)))
             self._scene = flat
         return flat
+
+    def refit(self, scene, vertices=None, normals=None):
+        """Move the triangles of the scene uploaded to this context and refit its tree on the GPU (trace_scene_refit):
+        same topology, every box recomputed.  `vertices` is [n_tris, 3, 3] in the triangle order of the scene's
+        flattening (`FlatScene.tri_vertices`):
+          None                   the meshes' current `vertices` (move a mesh's vertices, then refit);
+          numpy array            through host memory;
+          float32 CUDA tensor    (contiguous, on this context's device) read in place on the GPU: no host traffic.
+        `normals` (same layout and kind as `vertices`, or None to keep the current ones) apply to triangles uploaded
+        with normals.  Afterwards the host FlatScene's nodes are stale: it cannot be uploaded to another context."""
+        flat = scene.flatten() if scene._flat is not None else None
+        if flat is None or flat is not self._scene:
+            raise ValueError("refit: this scene is not the one uploaded to this context")
+        n = len(flat.tri_vertices)
+        sb = np.ascontiguousarray(flat.sphere_bounds, dtype=np.float32)
+        sb_ptr = _lib.ptr(sb) if len(sb) else None
+        if vertices is None:
+            vertices = flat.gather_vertices()
+        if hasattr(vertices, "is_cuda"):                      # a torch tensor
+            def dev_ptr(t, what):
+                if t is None:
+                    return None
+                if not (hasattr(t, "is_cuda") and t.is_cuda and t.device.index == self.device):
+                    raise ValueError(f"refit: {what} must be a CUDA tensor on device {self.device}")
+                if str(t.dtype) != "torch.float32" or not t.is_contiguous() or t.numel() != 9 * n:
+                    raise ValueError(f"refit: {what} must be a contiguous float32 tensor of {n} x 3 x 3")
+                return t.data_ptr()
+            vp, np_ = dev_ptr(vertices, "vertices"), dev_ptr(normals, "normals")
+            import torch
+            torch.cuda.current_stream(self.device).synchronize()    # the work that wrote them is done
+            self.check(self.lib.trace_scene_refit_device(self.h, n, vp, np_, len(sb), sb_ptr))
+        else:
+            def host(a, what):
+                if a is None:
+                    return None
+                a = np.ascontiguousarray(a, dtype=np.float32)
+                if a.size != 9 * n:
+                    raise ValueError(f"refit: {what} must be {n} x 3 x 3")
+                return a
+            v, nn = host(vertices, "vertices"), host(normals, "normals")
+            self.check(self.lib.trace_scene_refit(self.h, n, _lib.ptr(v), _lib.ptr(nn), len(sb), sb_ptr))
+        flat.stale = True
+
+    def scene_nodes(self):
+        """The uploaded scene's nodes as the device holds them now (trace_scene_copy_nodes), node_dtype."""
+        if self._scene is None:
+            raise ValueError("no scene uploaded")
+        nodes = np.zeros(len(self._scene.nodes), dtype=_lib.node_dtype)
+        self.check(self.lib.trace_scene_copy_nodes(self.h, _lib.ptr(nodes)))
+        return nodes
 
     def stats(self):
         s = _lib.Stats()

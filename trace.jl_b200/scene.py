@@ -476,6 +476,9 @@ class FlatScene:
         spheres = []
         self.n_tris = 0
         self._orig = 0
+        self.tri_sources = []       # where the triangles come from, in triangle order: a batch's mesh or one Triangle
+        self.sphere_bounds = []     # world_bound() of each sphere (the bounds its tree was built with)
+        self.stale = False          # Context.refit moved the vertices on the device: nodes / tri_vertices are old
         nodes, prims = self._flatten_bvh(scene.aggregate, tri_v, tri_n, tri_f, spheres)
         self.nodes = nodes
         self.prims = prims
@@ -488,6 +491,7 @@ class FlatScene:
             self.tri_normals = np.zeros((0, 3, 3), np.float32)
             self.tri_flags = np.zeros(0, np.uint8)
         self.spheres = np.array(spheres, dtype=_lib.sphere_dtype) if spheres else np.zeros(0, _lib.sphere_dtype)
+        self.sphere_bounds = np.array(self.sphere_bounds, dtype=np.float32).reshape(-1, 6)
         mats = np.zeros(max(1, len(self.materials)), dtype=_lib.material_dtype)
         for i, m in enumerate(self.materials):
             mats[i] = m.pod()
@@ -528,6 +532,7 @@ class FlatScene:
                 tri_v.append(tv)
                 tri_n.append(tn if tn is not None else np.zeros_like(tv))
                 tri_f.append(np.full(cnt, flags, dtype=np.uint8))
+                self.tri_sources.append(mesh)
                 kinds[pos:pos + cnt] = _lib.PRIM_TRIANGLE
                 index[pos:pos + cnt] = np.arange(self.n_tris, self.n_tris + cnt, dtype=np.uint32)
                 mat[pos:pos + cnt] = self._material_id(p.material)
@@ -542,6 +547,7 @@ class FlatScene:
                 tri_v.append(tv)
                 tri_n.append(t.mesh.normals[idx][None] if has_n else np.zeros_like(tv))
                 tri_f.append(np.array([(1 if t.core.flip else 0) | (2 if has_n else 0)], dtype=np.uint8))
+                self.tri_sources.append(t)
                 kinds[pos] = _lib.PRIM_TRIANGLE
                 index[pos] = self.n_tris
                 mat[pos] = self._material_id(p.material)
@@ -553,6 +559,7 @@ class FlatScene:
                 o2w = s.core.object_to_world
                 spheres.append((o2w.m.reshape(-1), o2w.inv_m.reshape(-1), s.radius, s.z_min, s.z_max, s.theta_min,
                                 s.theta_max, s.phi_max, 1 if s.core.flip else 0, 0))
+                self.sphere_bounds.append(s.world_bound().as6())
                 kinds[pos] = _lib.PRIM_SPHERE
                 index[pos] = len(spheres) - 1
                 mat[pos] = self._material_id(p.material)
@@ -609,6 +616,14 @@ class FlatScene:
         for i, r in enumerate(out_prims):
             prims[i] = tuple(int(x) for x in r)
         return nodes, prims
+
+    def gather_vertices(self):
+        """[n_tris, 3, 3] float32: the current world-space vertices of the meshes this scene was flattened from, in the
+        order of `tri_vertices` (what Context.refit(scene) uploads after the caller moved mesh vertices)."""
+        if not self.tri_sources:
+            return np.zeros((0, 3, 3), np.float32)
+        parts = [src.triangle_vertices() if isinstance(src, TriangleMesh) else src.vertices()[None] for src in self.tri_sources]
+        return np.ascontiguousarray(np.concatenate(parts, axis=0), dtype=np.float32)
 
     def desc(self):
         d = _lib.SceneDesc()
