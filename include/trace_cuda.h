@@ -195,7 +195,11 @@ const char* trace_last_error(const trace_ctx* ctx);
  *          src/accel/bvh.jl:221-257; "leaf_wait" 0/4/8/16/32 warp-synchronous variant of loop 0 with batched leaf
  *          tests (measured slower, kept for the record); "film_mode" see trace_comm_init; "persist" 0/1
  *          persistent-warp traversal kernels (default 0); "count_nodes" 0/1; "time_kernels" 0/1 (per-launch CUDA
- *          events; with TRACE_CUDA_TIMELINE=<file> they are also dumped); "rank"/"world" shard selection (Whitted: tiles
+ *          events; with TRACE_CUDA_TIMELINE=<file> they are also dumped); "shadow_tree" 0/1 (default 1): any-hit queries
+ *          (trace_occluded*, Whitted and SPPM shadow rays) walk the scene's shadow tree, an LBVH built on the device at
+ *          upload, and check every occluder they find against the reference tree: the same answers bit for bit, 0 =
+ *          walk the reference tree only (it applies with "slab" 2 and "walk" 1; a scene uploaded with 0 gets no shadow
+ *          tree, which saves its 64 B per primitive); "rank"/"world" shard selection (Whitted: tiles
  *          k % world; SPPM: image rows and, through the photon range arguments, photons). */
 int         trace_set_option(trace_ctx* ctx, const char* key, int64_t value);
 int         trace_get_stats(trace_ctx* ctx, trace_stats* out);
@@ -255,6 +259,15 @@ int trace_scene_refit_device(trace_ctx* ctx, int64_t n_tris, const void* tri_ver
                              const void* tri_normals_device, int64_t n_spheres, const float* sphere_bounds);
 /* the uploaded scene's current nodes (n_nodes of the last upload), boxes as refit last left them */
 int trace_scene_copy_nodes(trace_ctx* ctx, trace_bvh_node* nodes_out);
+/* the uploaded scene's shadow tree: *n_pairs = its pair records (n_prims - 1), 0 when the scene has none (analytic
+ * spheres, fewer than 2 primitives, a NaN vertex, deeper than 64 levels).  pairs_out (NULL: count only) receives
+ * n_pairs x 64 bytes: per child {bmin.xyz, bmax.x} {bmax.y, bmax.z, reference, split-axis bit (first child) or 0};
+ * reference = pair index, or 0x80000000 | primitive slot for a leaf.  Boxes as the last refit left them. */
+int trace_scene_shadow_tree(trace_ctx* ctx, int64_t* n_pairs, void* pairs_out);
+/* any-hit rays since the last trace_reset_stats that found a candidate occluder on the shadow tree which the exact
+ * check could not confirm (or had a zero, tiny or non-finite direction component), and so were answered by the
+ * reference tree's walk */
+int trace_get_shadow_fallbacks(trace_ctx* ctx, uint64_t* out);
 
 /* ---- ray queries, host buffers. o,d: [n][3]; tmax_inout: [n] (t of the hit on return, unchanged on a miss);
  * prim_out: [n] original index + 1, 0 = miss; b0b1_out: [n][2] barycentrics (triangles) or 0; may be NULL. ---- */

@@ -25,7 +25,7 @@ __global__ void __launch_bounds__(128, 8) k_intersect(DeviceScene sc, const floa
         hits[i] = make_float4(h.prim ? h.t : o.w, __uint_as_float(orig), h.b0, h.b1);
     }
 }
-template <int SLAB, bool COUNT, int WAIT>
+template <int SLAB, bool COUNT, int WAIT, bool TREE>       // TREE: walk the shadow tree (wavefront.cuh k_wh_shadow)
 __global__ void __launch_bounds__(128, 8) k_occluded(DeviceScene sc, const float4* __restrict__ ro, const float4* __restrict__ rd,
                                                   long long n, uint8_t* __restrict__ out, unsigned long long* counters,
                                                   int* error_flag) {
@@ -34,8 +34,12 @@ __global__ void __launch_bounds__(128, 8) k_occluded(DeviceScene sc, const float
         const long long i = base + lane;
         const bool valid = i < n;
         const float4 o = valid ? ro[i] : make_float4(0.0f, 0.0f, 0.0f, 0.0f), d = valid ? rd[i] : make_float4(1.0f, 1.0f, 1.0f, 0.0f);
-        HitRecord h;
-        const bool occ = traverse_any<SLAB, true, COUNT, WAIT>(sc, valid, xyz(o), xyz(d), o.w, h, counters, error_flag);
+        bool occ;
+        if (TREE) occ = valid && traverse_shadow<COUNT>(sc, xyz(o), xyz(d), o.w, counters, error_flag);
+        else {
+            HitRecord h;
+            occ = traverse_any<SLAB, true, COUNT, WAIT>(sc, valid, xyz(o), xyz(d), o.w, h, counters, error_flag);
+        }
         if (valid) out[i] = occ ? 1 : 0;
     }
 }
@@ -90,7 +94,7 @@ extern "C" void trace_destroy(trace_ctx* c) {
     sppm_free(c);
     trace_comm_destroy(c);
     DevBuf* all[] = {&c->b_nodes, &c->b_pairs, &c->b_prims, &c->b_tnorm, &c->b_spheres, &c->b_materials, &c->b_lights, &c->b_counters,
-                     &c->refit.topo, &c->refit.stage, &c->refit.sphere_bounds};
+                     &c->b_shadow, &c->refit.topo, &c->refit.stage, &c->refit.sphere_bounds, &c->refit.shadow_topo};
     for (DevBuf* b : all) b->release();
     for (auto& b : c->b_query) b.release();
     for (auto& b : c->b_queue) b.release();
@@ -132,6 +136,7 @@ extern "C" int trace_set_option(trace_ctx* c, const char* key, int64_t v) {
     else if (!strcmp(key, "lanes")) { if (v < 1 || v > trace_ctx::MAX_LANES) return c->fail("lanes must be in [1, 16]"); c->lanes = (int)v; }
     else if (!strcmp(key, "cap_percent")) { if (v < 100 || v > 1600) return c->fail("cap_percent must be in [100, 1600]"); c->cap_percent = (int)v; }
     else if (!strcmp(key, "time_kernels")) c->time_kernels = v != 0;
+    else if (!strcmp(key, "shadow_tree")) c->shadow_tree = v != 0;
     else if (!strcmp(key, "graph")) c->graph = v != 0;
     else if (!strcmp(key, "sppm_lanes")) { if (v < 0 || v > trace_ctx::MAX_LANES / 2) return c->fail("sppm_lanes must be in [0, 8]"); c->sppm_lanes = (int)v; }
     else if (!strcmp(key, "sppm_chain_priority")) c->sppm_chain_priority = v != 0;
@@ -158,6 +163,7 @@ int ctx_pull_stats(trace_ctx* c) {
     c->stats.sppm_grid_items = h[ST_GRID_ITEMS];
     c->stats.primary_rays = h[ST_PRIMARY_RAYS];
     c->stats.primary_hits = h[ST_PRIMARY_HITS];
+    c->shadow_fallbacks = h[ST_SHADOW_FALLBACKS];
     return 0;
 }
 
@@ -371,11 +377,42 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
             if (std::isfinite(b)) s.scene_scale = fmaxf(s.scene_scale, b);
         }
     }
+    // the shadow tree (traverse.cuh, traverse_shadow): built on the device from the uploaded primitive records.  Scenes
+    // with analytic spheres have none (the guard its walk admits nodes with is off below spheres); neither has a scene
+    // uploaded with option shadow_tree 0
+    s.shadow_pairs = nullptr;
+    if (c->shadow_tree && d->n_spheres == 0 && d->n_prims >= 2) {
+        TR_CUDA(c, c->b_shadow.ensure((size_t)(d->n_prims - 1) * 4 * sizeof(float4)));
+        const int rc = shadow_tree_build(c->stream, c->b_prims.p, d->n_prims, c->b_shadow.p);
+        if (rc == 0) s.shadow_pairs = c->b_shadow.as<float4>();
+        else if (rc != 5 && rc != 6) return c->fail("scene: shadow tree build failed (CUDA error)");
+    }
     c->have_scene = true;
     c->refit.tri_index.swap(tri_index);
     c->refit.n_tris = d->n_tris; c->refit.n_spheres = d->n_spheres; c->refit.n_pairs = n_pairs;
     c->refit.topo_ready = false;
+    c->refit.shadow_topo_ready = false;
     sppm_end_session(c);
+    return 0;
+}
+
+extern "C" int trace_scene_shadow_tree(trace_ctx* c, int64_t* n_pairs, void* pairs_out) {
+    if (!c || !n_pairs) return 1;
+    cudaSetDevice(c->device);
+    if (!c->have_scene) return c->fail("no scene uploaded");
+    *n_pairs = c->scene.shadow_pairs ? c->scene.n_prims - 1 : 0;
+    if (pairs_out && *n_pairs) {
+        TR_CUDA(c, cudaMemcpyAsync(pairs_out, c->scene.shadow_pairs, (size_t)*n_pairs * 4 * sizeof(float4), cudaMemcpyDeviceToHost, c->stream));
+        TR_CUDA(c, cudaStreamSynchronize(c->stream));
+    }
+    return 0;
+}
+
+extern "C" int trace_get_shadow_fallbacks(trace_ctx* c, uint64_t* out) {
+    if (!c || !out) return 1;
+    cudaSetDevice(c->device);
+    if (ctx_pull_stats(c)) return 1;
+    *out = c->shadow_fallbacks;
     return 0;
 }
 
@@ -427,9 +464,13 @@ static int launch_occluded(trace_ctx* c, const float4* ro, const float4* rd, int
     unsigned long long* cnt = ctx_stats64(c) + ST_NODES;
     const int grid = (int)std::min<int64_t>((n + 127) / 128, (int64_t)persistent_grid(c, 16));
     if (c->time_kernels) cudaEventRecord(c->evk0, c->stream);
+    const DeviceScene sc = shadow_launch_scene(c, c->scene);
     trav_dispatch(c, [&](auto S, auto C_, auto W) {
-        auto k = k_occluded<decltype(S)::value, decltype(C_)::value, decltype(W)::value>;
-        k<<<std::min(grid, occupancy_grid(c, k, 128)), 128, 0, c->stream>>>(c->scene, ro, rd, n, out, cnt, err);
+        constexpr int s = decltype(S)::value, w = decltype(W)::value;
+        constexpr bool cn = decltype(C_)::value;
+        auto k = k_occluded<s, cn, w, false>;
+        if constexpr (shadow_walk_capable<s, cn, w>) if (sc.shadow_pairs) k = k_occluded<s, cn, w, true>;
+        k<<<std::min(grid, occupancy_grid(c, k, 128)), 128, 0, c->stream>>>(sc, ro, rd, n, out, cnt, err);
     });
     if (c->time_kernels) cudaEventRecord(c->evk1, c->stream);
     TR_CUDA(c, cudaGetLastError());

@@ -214,12 +214,13 @@ __global__ void lbvh_emit(int64_t n, int m, const uint32_t* __restrict__ child, 
 inline unsigned blocks_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
 
 // The build's device buffers, carved out of one allocation: carve() with base == 0 sizes it, then again on the real one.
+// `pb` (the primitive bounds) and the node array are carved only when asked for.
 struct Buffers {
-    float* pb; Status* st;
+    float* pb = nullptr; Status* st;
     uint64_t *keys, *keys_sorted; uint32_t *ids, *ids_sorted;                  // sort in / out
     uint32_t *child, *first, *count; int32_t* parent; uint8_t* axis;           // hierarchy (parent: every node)
     uint32_t* arrive; float* box; uint32_t *size, *depth;                      // bottom-up, every node
-    trace_bvh_node* nodes; void* sort_tmp;
+    trace_bvh_node* nodes = nullptr; void* sort_tmp;
     size_t used = 0;
     char* base = nullptr;
     template <class T> T* take(int64_t count) {
@@ -227,16 +228,26 @@ struct Buffers {
         used = off + (size_t)count * sizeof(T);
         return reinterpret_cast<T*>(base + off);
     }
-    void carve(int64_t n, size_t sort_bytes) {
+    void carve(int64_t n, size_t sort_bytes, bool with_pb, bool with_nodes) {
         const int64_t nn = 2 * n - 1;
         used = 0;
-        pb = take<float>(6 * n); st = take<Status>(1);
+        if (with_pb) pb = take<float>(6 * n);
+        st = take<Status>(1);
         keys = take<uint64_t>(n); keys_sorted = take<uint64_t>(n); ids = take<uint32_t>(n); ids_sorted = take<uint32_t>(n);
         child = take<uint32_t>(2 * (n - 1)); first = take<uint32_t>(n - 1); count = take<uint32_t>(n - 1);
         parent = take<int32_t>(nn); axis = take<uint8_t>(n - 1);
         arrive = take<uint32_t>(n - 1); box = take<float>(6 * nn); size = take<uint32_t>(nn); depth = take<uint32_t>(nn);
-        nodes = take<trace_bvh_node>(nn); sort_tmp = take<char>((int64_t)sort_bytes);
+        if (with_nodes) nodes = take<trace_bvh_node>(nn);
+        sort_tmp = take<char>((int64_t)sort_bytes);
     }
+    // one allocation for everything; freed by the destructor
+    int alloc(int64_t n, size_t sort_bytes, bool with_pb, bool with_nodes) {
+        carve(n, sort_bytes, with_pb, with_nodes);
+        if (cudaMalloc(&base, used) != cudaSuccess) { cudaGetLastError(); base = nullptr; return 7; }
+        carve(n, sort_bytes, with_pb, with_nodes);
+        return 0;
+    }
+    ~Buffers() { if (base) cudaFree(base); }
 };
 
 struct Phases {
@@ -246,22 +257,20 @@ struct Phases {
     void mark(cudaStream_t s) { if (on && n < 8) cudaEventRecord(ev[n++], s); }
 };
 
-int build(cudaStream_t s, const float* hb, int64_t n, int m, trace_bvh** out, Phases& ph) {
-    const int64_t nn = 2 * n - 1;
-    size_t sort_bytes = 0;
-    if (cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (const uint64_t*)nullptr, (uint64_t*)nullptr,
-                                        (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)n, 0, 63, s) != cudaSuccess)
-        return 7;
-    Buffers b;
-    b.carve(n, sort_bytes);
-    if (cudaMalloc(&b.base, b.used) != cudaSuccess) { cudaGetLastError(); return 7; }
-    struct Free { void* p; ~Free() { cudaFree(p); } } free_buffers{b.base};
-    b.carve(n, sort_bytes);
+size_t sort_bytes_for(int64_t n, cudaStream_t s) {
+    size_t bytes = 0;
+    if (cub::DeviceRadixSort::SortPairs(nullptr, bytes, (const uint64_t*)nullptr, (uint64_t*)nullptr, (const uint32_t*)nullptr,
+                                        (uint32_t*)nullptr, (int)n, 0, 63, s) != cudaSuccess)
+        return 0;
+    return bytes;
+}
 
+// The device-resident core: bounds b.pb (device, [n][6]) -> keys, sorted order, hierarchy, boxes, subtree sizes and
+// depths in `b`, and the status on the host.  Returns 0, 5 (a NaN bound), 6 (deeper than the 64-entry traversal
+// stack) or 7 (CUDA error).
+int build_core(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, Status& hs, Phases& ph) {
+    const int64_t nn = 2 * n - 1;
     const int T = 256;
-    ph.mark(s);
-    if (cudaMemcpyAsync(b.pb, hb, (size_t)n * 6 * sizeof(float), cudaMemcpyHostToDevice, s) != cudaSuccess) return 7;
-    ph.mark(s);
     cudaMemsetAsync(b.st, 0xFF, sizeof(b.st->cmin), s);
     cudaMemsetAsync(&b.st->cmax, 0, sizeof(Status) - sizeof(b.st->cmin), s);
     cudaMemsetAsync(b.parent, 0xFF, (size_t)nn * sizeof(int32_t), s);
@@ -277,7 +286,6 @@ int build(cudaStream_t s, const float* hb, int64_t n, int m, trace_bvh** out, Ph
     ph.mark(s);
     lbvh_bottom_up<<<blocks_for(n, T), T, 0, s>>>(b.pb, b.ids_sorted, n, m, b.child, b.parent, b.count, b.arrive, b.box,
                                                    b.size, b.depth, b.st);
-    Status hs;
     if (cudaGetLastError() != cudaSuccess ||
         cudaMemcpyAsync(&hs, b.st, sizeof(Status), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
         cudaStreamSynchronize(s) != cudaSuccess)
@@ -285,6 +293,21 @@ int build(cudaStream_t s, const float* hb, int64_t n, int m, trace_bvh** out, Ph
     ph.mark(s);
     if (hs.nan) return 5;
     if (hs.root_depth > 64) return 6;                        // TR_STACK_SIZE (traverse.cuh): the walks' stacks would overflow
+    return 0;
+}
+
+int build(cudaStream_t s, const float* hb, int64_t n, int m, trace_bvh** out, Phases& ph) {
+    const int64_t nn = 2 * n - 1;
+    const size_t sort_bytes = sort_bytes_for(n, s);
+    if (!sort_bytes) return 7;
+    Buffers b;
+    if (b.alloc(n, sort_bytes, true, true)) return 7;
+    const int T = 256;
+    ph.mark(s);
+    if (cudaMemcpyAsync(b.pb, hb, (size_t)n * 6 * sizeof(float), cudaMemcpyHostToDevice, s) != cudaSuccess) return 7;
+    ph.mark(s);
+    Status hs;
+    if (const int rc = build_core(s, n, m, b, sort_bytes, hs, ph)) return rc;
     const int64_t n_nodes = hs.root_size;
     lbvh_emit<<<blocks_for(nn, T), T, 0, s>>>(n, m, b.child, b.parent, b.first, b.count, b.axis, b.box, b.size, b.nodes);
     if (cudaGetLastError() != cudaSuccess) return 7;
@@ -304,7 +327,62 @@ int build(cudaStream_t s, const float* hb, int64_t n, int m, trace_bvh** out, Ph
     return 0;
 }
 
+// ------------------------------------------------------------------ the shadow tree (traverse.cuh, traverse_shadow)
+// A primitive's box: Julia min / max over its three vertices (the refit's leaf rule, refit.cu).  A NaN coordinate makes
+// the whole box NaN, so the centroid pass refuses the input.
+__global__ void lbvh_prim_bounds(const float4* __restrict__ prims, int64_t n, float* __restrict__ pb) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float4 A = prims[3 * i], B = prims[3 * i + 1], C = prims[3 * i + 2];
+    float lo[3] = {jl_min(jl_min(jl_min(INFINITY, A.x), B.x), C.x), jl_min(jl_min(jl_min(INFINITY, A.y), B.y), C.y),
+                   jl_min(jl_min(jl_min(INFINITY, A.z), B.z), C.z)};
+    float hi[3] = {jl_max(jl_max(jl_max(-INFINITY, A.x), B.x), C.x), jl_max(jl_max(jl_max(-INFINITY, A.y), B.y), C.y),
+                   jl_max(jl_max(jl_max(-INFINITY, A.z), B.z), C.z)};
+    const bool nan = A.x != A.x || A.y != A.y || A.z != A.z || B.x != B.x || B.y != B.y || B.z != B.z || C.x != C.x ||
+                     C.y != C.y || C.z != C.z;
+    for (int c = 0; c < 3; ++c) {
+        pb[6 * i + c] = nan ? NAN : lo[c];
+        pb[6 * i + 3 + c] = nan ? NAN : hi[c];
+    }
+}
+
+// One 64-byte pair record per internal node, in Karras numbering (the root is pair 0): both children's boxes, their
+// references (a pair index, or 0x80000000 | primitive slot for a leaf: TR_REF_LEAF, traverse.cuh) and the split axis as
+// a bit in the first half - the layout of the upload's pair records (api.cu).
+__global__ void lbvh_emit_pairs(int64_t n, const uint32_t* __restrict__ child, const uint32_t* __restrict__ sorted_ids,
+                                const uint8_t* __restrict__ axis, const float* __restrict__ box, float4* __restrict__ pairs) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= n - 1) return;
+    for (int k = 0; k < 2; ++k) {
+        const int64_t v = child[2 * i + k];
+        const float* bx = box + 6 * v;
+        const uint32_t ref = v < n - 1 ? (uint32_t)v : (0x80000000u | sorted_ids[v - (n - 1)]);
+        const uint32_t extra = k == 0 ? (1u << axis[i]) : 0u;
+        pairs[4 * i + 2 * k] = make_float4(bx[0], bx[1], bx[2], bx[3]);
+        pairs[4 * i + 2 * k + 1] = make_float4(bx[4], bx[5], __uint_as_float(ref), __uint_as_float(extra));
+    }
+}
+
 }  // namespace
+
+// The shadow tree of an uploaded scene (api.cu): an LBVH with one primitive per leaf over the n >= 2 uploaded primitive
+// records `prims` (device, BVH slot order, triangles only), written as n - 1 pair records to `pairs` (device).  Nothing
+// crosses to the host but the build's status.  Returns 0, 5 (a NaN vertex), 6 (deeper than 64 levels) or 7 (CUDA error).
+int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs) {
+    if (n < 2 || n >= 0x40000000ll) return 1;
+    const size_t sort_bytes = sort_bytes_for(n, s);
+    if (!sort_bytes) return 7;
+    Buffers b;
+    if (b.alloc(n, sort_bytes, true, false)) return 7;
+    const int T = 256;
+    lbvh_prim_bounds<<<blocks_for(n, T), T, 0, s>>>(static_cast<const float4*>(prims), n, b.pb);
+    Phases ph;
+    Status hs;
+    if (const int rc = build_core(s, n, 1, b, sort_bytes, hs, ph)) return rc;
+    lbvh_emit_pairs<<<blocks_for(n - 1, T), T, 0, s>>>(n, b.child, b.ids_sorted, b.axis, b.box, static_cast<float4*>(pairs));
+    if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess) return 7;
+    return 0;
+}
 
 extern "C" int trace_bvh_build_gpu(int device, const float* pb, int64_t n, int max_node_primitives, trace_bvh** out) {
     if (!out || n < 0 || (n > 0 && !pb)) return 1;

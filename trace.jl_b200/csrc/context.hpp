@@ -84,6 +84,7 @@ struct trace_ctx {
     int work_slot = 0;
     int leaf_wait = -1;           // walk selector: -1 pair nodes (default, option "walk" 1), 0 the reference loop ("walk" 0), 4/8/16/32 batched leaves
     int time_kernels = 0;
+    int shadow_tree = 1;          // any-hit queries walk the scene's shadow tree (traverse_shadow) when it has one; 0 = the reference tree only
     int rank = 0, world = 1;
     void* comm = nullptr;         // ncclComm_t of this rank (comm.cpp), null until trace_comm_init
     int nccl_version = 0;
@@ -115,6 +116,7 @@ struct trace_ctx {
     bool have_scene = false;
     DeviceScene scene{};
     DevBuf b_nodes, b_pairs, b_prims, b_tnorm, b_spheres, b_materials, b_lights;
+    DevBuf b_shadow;              // the shadow tree's pair records (scene.shadow_pairs), 64 B per primitive
 
     // refit (refit.cu): what trace_scene_refit needs of the last upload.  The host keeps only the BVH-slot -> triangle
     // map; the device topology (parents, pair slots, leaf list) is derived from b_nodes at the first refit after an
@@ -133,6 +135,12 @@ struct trace_ctx {
         uint32_t* arrive = nullptr;        // [n_pairs] arrival counters (reset per call)
         uint32_t* slot_tri = nullptr;      // [n_prims] tri_index on the device
         uint32_t* status = nullptr;        // [0] NaN vertex seen
+        // the shadow tree's topology, derived from its pair records at the first refit after an upload (refit.cu)
+        bool shadow_topo_ready = false;
+        DevBuf shadow_topo;
+        uint32_t* shadow_up_pair = nullptr;   // [n_prims - 1] 2 * parent pair + slot, ~0 at the root
+        uint32_t* shadow_up_prim = nullptr;   // [n_prims] 2 * pair + slot holding the primitive's leaf
+        uint32_t* shadow_arrive = nullptr;    // [n_prims - 1] arrival counters (reset per call)
     } refit;
 
     // scratch
@@ -143,6 +151,7 @@ struct trace_ctx {
     int* h_flags = nullptr;       // pinned host mirror of [overflow, error]
 
     trace_stats stats{};
+    unsigned long long shadow_fallbacks = 0;   // any-hit rays the shadow walk handed to the reference walk (trace_get_shadow_fallbacks)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evk0 = nullptr, evk1 = nullptr;
     // per-launch CUDA-event timing of the traversal kernels (option "time_kernels"), resolved after a stream sync
     struct KernelEvent { cudaEvent_t a, b; int kind, lane; };
@@ -206,7 +215,9 @@ struct trace_ctx {
     } while (0)
 
 // u64 device stats block layout (ctx->b_counters, after the int counters)
-enum { ST_RAYS_EXTEND = 0, ST_RAYS_SHADOW = 1, ST_NODES = 2, ST_PRIMS = 3, ST_DEPOSITS = 4, ST_CANDIDATES = 5, ST_REQUESTS = 6, ST_GRID_ITEMS = 7, ST_PRIMARY_RAYS = 8, ST_PRIMARY_HITS = 9, ST_COUNT = 12 };
+enum { ST_RAYS_EXTEND = 0, ST_RAYS_SHADOW = 1, ST_NODES = 2, ST_PRIMS = 3, ST_DEPOSITS = 4, ST_CANDIDATES = 5, ST_REQUESTS = 6, ST_GRID_ITEMS = 7, ST_PRIMARY_RAYS = 8, ST_PRIMARY_HITS = 9, ST_SHADOW_FALLBACKS = 10, ST_COUNT = 12 };
+// the traversal kernels get `counters` = stats + ST_NODES; the shadow walk counts its fallbacks at this offset from it
+static_assert(ST_SHADOW_FALLBACKS - ST_NODES == 8, "TR_COUNTER_SHADOW_FALLBACKS (traverse.cuh)");
 static const int TR_INT_COUNTERS = 128;    // ints at the start of b_counters (64..127: work counters of persistent launches)
 // int counter slots: [1 .. TR_MAX_DEPTH] ray-queue length per bounce level, [32] shadow / deposit-request queue
 enum { IC_OVERFLOW = 60, IC_ERROR = 61, IC_OVERFLOW_SHADOW = 62, IC_OVERFLOW_DEPOSIT = 63 };
@@ -275,6 +286,13 @@ static void trav_dispatch(const trace_ctx* c, F f) {
     else f(integral_constant<int, 2>{}, integral_constant<bool, false>{}, integral_constant<int, 0>{});
 }
 
+// The scene as an any-hit launch sees it: the shadow tree only with the option on, the guarded test and the pair walk
+// (the walk it falls back to, and the guard its admission test relies on)
+inline DeviceScene shadow_launch_scene(const trace_ctx* c, DeviceScene sc) {
+    if (!(c->shadow_tree && c->slab == 2 && c->leaf_wait == -1 /* TR_WALK_PAIR */)) sc.shadow_pairs = nullptr;
+    return sc;
+}
+
 // implemented in api.cu
 int ctx_device_film(trace_ctx* ctx, const trace_film_desc* film, DeviceFilm* out, DevBuf* table_buf);
 void ctx_device_camera(const trace_camera* cam, DeviceCamera* out);
@@ -296,5 +314,7 @@ int whitted_render_device(trace_ctx* ctx, const trace_camera* cam, const trace_f
 void sppm_free(trace_ctx* ctx);
 void sppm_end_session(trace_ctx* ctx);
 void whitted_film_range(const trace_ctx* ctx, long long npix, long long* p0, long long* p1);
+// implemented in bvh_gpu.cu: the shadow tree over uploaded primitive records (0, 5 NaN, 6 too deep, 7 CUDA error)
+int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs);
 // implemented in refit.cu: waits for every stream of the context (caller's, lanes, SPPM chain / collectives, copies)
 int ctx_drain(trace_ctx* ctx);

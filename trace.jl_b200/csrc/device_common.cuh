@@ -93,6 +93,10 @@ struct DeviceScene {
     const DeviceLight* lights;
     int n_nodes, n_prims, n_spheres, n_materials, n_lights;
     float scene_scale;        // largest |coordinate| of the root bounds (slack of the guarded slab test)
+    // the shadow tree (api.cu, traverse.cuh traverse_shadow): an LBVH over the same primitive slots, one primitive per
+    // leaf, n_prims - 1 pair records in the layout of `pairs`, root = pair 0.  Null: no shadow tree (analytic spheres,
+    // fewer than 2 primitives, NaN vertices, deeper than 64 levels), or the launch does not use it (option shadow_tree)
+    const float4* shadow_pairs;
 };
 struct DeviceCamera {
     float r2c[16], c2w[16];

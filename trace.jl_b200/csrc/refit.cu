@@ -153,6 +153,57 @@ __global__ void refit_climb(const float4* __restrict__ prims, const float* __res
     }
 }
 
+// ------------------------------------------------------------------ the shadow tree (api.cu, traverse.cuh traverse_shadow)
+// Its pair records hold both children's boxes, so a pair's box is the union of its own two halves: one thread per
+// primitive writes the primitive's vertex box into its leaf's half, then climbs while it is the second to arrive at a
+// pair, writing the pair's union into the parent's half.  Same rules as above (Julia min / max, exact, deterministic)
+// and as the build (bvh_gpu.cu), so a refit with unchanged vertices gives back the uploaded records.
+
+// topology: every reference's (parent pair, slot)
+__global__ void shadow_topology(const float4* __restrict__ pairs, int64_t n_pairs, uint32_t* __restrict__ up_pair,
+                                uint32_t* __restrict__ up_prim) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= n_pairs) return;
+    for (uint32_t k = 0; k < 2; ++k) {
+        const uint32_t ref = __float_as_uint(pairs[4 * i + 2 * k + 1].z), u = 2u * (uint32_t)i + k;
+        if (ref & TR_REF_LEAF) up_prim[ref & TR_REF_INDEX_MASK] = u;
+        else up_pair[ref] = u;
+    }
+}
+
+__device__ __forceinline__ void put_half(float4* pairs, uint32_t u, const float lo[3], const float hi[3]) {
+    float4* q = pairs + 4 * (size_t)(u >> 1) + 2 * (u & 1u);
+    q[0] = make_float4(lo[0], lo[1], lo[2], hi[0]);
+    *reinterpret_cast<float2*>(&q[1]) = make_float2(hi[1], hi[2]);
+}
+
+__global__ void shadow_climb(const float4* __restrict__ prims, int64_t n_prims, const uint32_t* __restrict__ up_pair,
+                             const uint32_t* __restrict__ up_prim, uint32_t* arrive, const uint32_t* __restrict__ status,
+                             float4* pairs) {
+    const int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (s >= n_prims || *status) return;
+    const float4 A = prims[3 * s], B = prims[3 * s + 1], C = prims[3 * s + 2];
+    float lo[3] = {jl_min(jl_min(jl_min(TR_INF, A.x), B.x), C.x), jl_min(jl_min(jl_min(TR_INF, A.y), B.y), C.y),
+                   jl_min(jl_min(jl_min(TR_INF, A.z), B.z), C.z)};
+    float hi[3] = {jl_max(jl_max(jl_max(-TR_INF, A.x), B.x), C.x), jl_max(jl_max(jl_max(-TR_INF, A.y), B.y), C.y),
+                   jl_max(jl_max(jl_max(-TR_INF, A.z), B.z), C.z)};
+    uint32_t u = up_prim[s];
+    put_half(pairs, u, lo, hi);
+    for (;;) {
+        const uint32_t p = u >> 1;
+        __threadfence();
+        if (atomicAdd(&arrive[p], 1u) == 0) return;               // the sibling's thread continues
+        __threadfence();
+        const float4 a0 = __ldcg(&pairs[4 * (size_t)p]), a1 = __ldcg(&pairs[4 * (size_t)p + 1]);
+        const float4 b0 = __ldcg(&pairs[4 * (size_t)p + 2]), b1 = __ldcg(&pairs[4 * (size_t)p + 3]);
+        lo[0] = jl_min(a0.x, b0.x); lo[1] = jl_min(a0.y, b0.y); lo[2] = jl_min(a0.z, b0.z);
+        hi[0] = jl_max(a0.w, b0.w); hi[1] = jl_max(a1.x, b1.x); hi[2] = jl_max(a1.y, b1.y);
+        u = up_pair[p];
+        if (u == ~0u) return;                                      // the root: pair 0 has no parent half
+        put_half(pairs, u, lo, hi);
+    }
+}
+
 inline unsigned blocks_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
 
 struct Phases {
@@ -194,6 +245,24 @@ int derive_topology(trace_ctx* c) {
         TR_CUDA(c, cudaMemcpyAsync(R.slot_tri, R.tri_index.data(), (size_t)n_prims * 4, cudaMemcpyHostToDevice, c->stream));
     TR_CUDA(c, cudaStreamSynchronize(c->stream));       // (tri_index is pageable host memory)
     R.topo_ready = true;
+    return 0;
+}
+
+// first refit after an upload that built a shadow tree: its parents, from the pair records
+int derive_shadow_topology(trace_ctx* c) {
+    auto& R = c->refit;
+    const int64_t n_prims = c->scene.n_prims, n_pairs = n_prims - 1;
+    size_t used = 0;
+    auto take = [&](size_t bytes) { const size_t off = (used + 255) & ~(size_t)255; used = off + bytes; return off; };
+    const size_t o_up_pair = take(n_pairs * 4), o_up_prim = take(n_prims * 4), o_arrive = take(n_pairs * 4);
+    TR_CUDA(c, R.shadow_topo.ensure(used));
+    char* base = R.shadow_topo.as<char>();
+    R.shadow_up_pair = (uint32_t*)(base + o_up_pair); R.shadow_up_prim = (uint32_t*)(base + o_up_prim);
+    R.shadow_arrive = (uint32_t*)(base + o_arrive);
+    TR_CUDA(c, cudaMemsetAsync(R.shadow_up_pair, 0xFF, n_pairs * 4, c->stream));
+    shadow_topology<<<blocks_for(n_pairs, 256), 256, 0, c->stream>>>(c->scene.shadow_pairs, n_pairs, R.shadow_up_pair, R.shadow_up_prim);
+    TR_CUDA(c, cudaGetLastError());
+    R.shadow_topo_ready = true;
     return 0;
 }
 
@@ -263,6 +332,15 @@ int refit_run(trace_ctx* c, int64_t n_tris, const float* v, const float* nrm, bo
                                                                   c->b_pairs.as<float4>());
     TR_CUDA(c, cudaGetLastError());
     ph.mark(c->stream, "climb");
+    if (c->scene.shadow_pairs) {                           // the shadow tree: same primitives, its own topology
+        if (!R.shadow_topo_ready && derive_shadow_topology(c)) return 1;
+        TR_CUDA(c, cudaMemsetAsync(R.shadow_arrive, 0, (size_t)(n_prims - 1) * 4, c->stream));
+        shadow_climb<<<blocks_for(n_prims, T), T, 0, c->stream>>>(c->b_prims.as<float4>(), n_prims, R.shadow_up_pair,
+                                                                  R.shadow_up_prim, R.shadow_arrive, R.status,
+                                                                  c->b_shadow.as<float4>());
+        TR_CUDA(c, cudaGetLastError());
+        ph.mark(c->stream, "shadow tree");
+    }
     uint32_t nan = 0;
     float4 root[2] = {};
     TR_CUDA(c, cudaMemcpyAsync(&nan, R.status, 4, cudaMemcpyDeviceToHost, c->stream));

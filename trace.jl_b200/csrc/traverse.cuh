@@ -464,6 +464,125 @@ done:
     return found;
 }
 
+// ------------------------------------------------------------------ any-hit walk on the shadow tree
+// An any-hit query returns one bit and never changes t_max, so the reference's answer does not depend on the order in
+// which its walk visits nodes: it is "some primitive passes triangle_test(r, t_max), and every reference-tree ancestor
+// of that primitive passes the reference's box test".  traverse_shadow computes that bit on the shadow tree (an LBVH
+// with one primitive per leaf, built at upload, DeviceScene::shadow_pairs), which costs about half the box tests of
+// the reference tree, and ties every occluder it reports back to the reference tree with one exact check:
+//   walk       every pair fetch tests both children with the guard of slab_child<2> (the interval widened by the slack
+//              r.m*, with the t_max term of slab_test<2>); a child is entered iff that guard admits it.  t_max is fixed,
+//              so every verdict is final when a child is pushed: the stack holds references only, nearer entry first.
+//   candidate  a primitive whose triangle_test(r, t_max) passes (same RayPrep, same scene_scale as the reference walk);
+//   check      the candidate triangle's own vertex box textbook-accepts: t_enter <= t_exit, t_exit > 0 and
+//              t_enter < t_max, on the six products slab_child_fast forms.  Then the answer is "occluded".
+//   end        no candidate: "not occluded"; only unconfirmed candidates: the reference walk (traverse_pair<2, true>)
+//              answers, which is the answer without a shadow tree.
+// Why this is the reference's bit:
+//   * No false "not occluded".  The guarded reference walk already relies on the guard never rejecting a box that
+//     contains the vertices of a triangle the ray passes (triangle_test) - the slack covers the rounding of the
+//     watertight test; otherwise the guarded walk (the default) would differ from the literal one.  Shadow-tree boxes
+//     are exact unions of their primitives' vertex boxes, so every reference candidate is admitted here all the way
+//     down to its leaf and becomes a shadow-tree candidate.
+//   * No false "occluded".  Every reference-tree ancestor box of a primitive contains the primitive's vertex box,
+//     coordinate by coordinate (tests/test_shadow_tree_host.py checks it on the uploaded trees).  Subtracting o and
+//     multiplying by inv are monotone under round-to-nearest, so on each axis the ancestor's two products bracket the
+//     vertex box's: its textbook entry is <= the vertex box's entry and its exit is >= its exit.  A textbook ACCEPT
+//     of the vertex box is therefore a textbook ACCEPT of every ancestor, the root included, with entry <= the vertex
+//     box's entry < t_max.  By slab_child_fast's three-way argument that is the reference's literal and guarded
+//     verdict with tx_min < t_max (so neither the far-child cull nor the pop test of traverse_pair drops it): the
+//     reference walk reaches the candidate's leaf and tests the same triangle with the same t_max - "occluded".
+//   * NaN never enters: the walk runs only for rays with a finite origin and a finite, non-zero 1/d on every axis
+//     (the shadow tree's boxes hold no NaN: a NaN vertex means no shadow tree), so the min / max form of the six
+//     products below is exactly the sign-selected form of slab_child<2>.  Other rays (a zero, tiny or non-finite
+//     direction component: +Inf thresholds, never a fast accept) go to the reference walk directly.
+// Deviation: the shadow tree is at most 64 levels deep (the upload refuses deeper ones), so this stack cannot
+// overflow; a reference-tree overflow (64 box-hit pending far children) is reported only when the fallback runs.
+#define TR_COUNTER_SHADOW_FALLBACKS 8      // offset of ST_SHADOW_FALLBACKS from `counters` (= stats + ST_NODES, context.hpp)
+
+// the kernel instantiations that can walk the shadow tree: the guarded pair walk (the default), and the counting passes,
+// which run the plain loop for closest hits but count the shadow walk the default path runs.  The launch picks them
+// when the scene it passes has a shadow tree (shadow_launch_scene, context.hpp); every other launch runs a kernel
+// without this walk, compiled exactly as before it existed
+template <int SLAB, bool COUNT, int WAIT>
+constexpr bool shadow_walk_capable = SLAB == 2 && (WAIT == TR_WALK_PAIR || COUNT);
+
+// kept out of line: it runs for a few rays per thousand and would otherwise double the kernel's code
+template <bool COUNT>
+static __device__ __noinline__ bool shadow_fallback(const DeviceScene sc, float3 o, float3 d, float tmax,
+                                                    unsigned long long* counters, int* error_flag) {
+    if (counters) atomicAdd(&counters[TR_COUNTER_SHADOW_FALLBACKS], 1ull);
+    HitRecord h;
+    return traverse_pair<2, true, COUNT>(sc, o, d, tmax, h, counters, error_flag);
+}
+
+// textbook entry / exit of a box (lo.xyz, hi.xyz) for a ray with finite, non-zero inv (no NaN: min / max pick the
+// same numbers as the sign-selected products)
+__device__ __forceinline__ void slab_interval(float lx, float ly, float lz, float hx, float hy, float hz, const RayPrep& r,
+                                              float slack_x, float slack_y, float slack_z, float& t_enter, float& t_exit) {
+    const float x0 = (lx - r.o.x) * r.inv.x, x1 = (hx - r.o.x) * r.inv.x;
+    const float y0 = (ly - r.o.y) * r.inv.y, y1 = (hy - r.o.y) * r.inv.y;
+    const float z0 = (lz - r.o.z) * r.inv.z, z1 = (hz - r.o.z) * r.inv.z;
+    t_enter = fmaxf(fmaxf(fminf(x0, x1) - slack_x, fminf(y0, y1) - slack_y), fminf(z0, z1) - slack_z);
+    t_exit = fminf(fminf(fmaxf(x0, x1) + slack_x, fmaxf(y0, y1) + slack_y), fmaxf(z0, z1) + slack_z);
+}
+
+template <bool COUNT>
+__device__ __forceinline__ bool traverse_shadow(const DeviceScene& sc, float3 o, float3 d, float tmax,
+                                                unsigned long long* counters, int* error_flag) {
+    const RayPrep r = prepare_ray(o, d, sc.scene_scale);
+    const bool regular = isfinite(o.x) & isfinite(o.y) & isfinite(o.z) & isfinite(r.inv.x) & isfinite(r.inv.y) &
+                         isfinite(r.inv.z) & (r.inv.x != 0.0f) & (r.inv.y != 0.0f) & (r.inv.z != 0.0f);
+    if (!regular) return shadow_fallback<COUNT>(sc, o, d, tmax, counters, error_flag);
+    const float tmax_guard = tmax + fabsf(tmax) * TR_GUARD_REL;        // slab_test<2>'s t_max term
+    uint32_t stack[TR_STACK_SIZE];
+    int sp = 0;
+    uint32_t item = 0;                      // the root: pair 0
+    unsigned n_nodes = 0, n_prims = 0;
+    bool occluded = false, candidate = false;
+    for (;;) {
+        if (item & TR_REF_LEAF) {
+            const uint32_t pi = item & TR_REF_INDEX_MASK;
+            const float4 a = __ldg(&sc.prims[3 * pi]);
+            if (COUNT) n_prims++;
+            if ((__float_as_uint(a.w) & ~TR_PRIM_LAST_BIT) == 0u) {        // degenerate triangles never hit
+                const float4 b = __ldg(&sc.prims[3 * pi + 1]), c = __ldg(&sc.prims[3 * pi + 2]);
+                float t, b0, b1, b2;
+                if (triangle_test(a, b, c, r, tmax, t, b0, b1, b2)) {
+                    float t_enter, t_exit;
+                    slab_interval(fminf(fminf(a.x, b.x), c.x), fminf(fminf(a.y, b.y), c.y), fminf(fminf(a.z, b.z), c.z),
+                                  fmaxf(fmaxf(a.x, b.x), c.x), fmaxf(fmaxf(a.y, b.y), c.y), fmaxf(fmaxf(a.z, b.z), c.z), r,
+                                  0.0f, 0.0f, 0.0f, t_enter, t_exit);
+                    if ((t_enter <= t_exit) & (t_exit > 0.0f) & (t_enter < tmax)) { occluded = true; break; }
+                    candidate = true;
+                }
+            }
+        } else {
+            const float4* np = sc.shadow_pairs + 4u * item;
+            const float4 q0 = __ldg(np), q1 = __ldg(np + 1), q2 = __ldg(np + 2), q3 = __ldg(np + 3);
+            if (COUNT) n_nodes += 2;
+            float e0, x0, e1, x1;
+            slab_interval(q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, r, r.mx, r.my, r.mz, e0, x0);
+            slab_interval(q2.x, q2.y, q2.z, q2.w, q3.x, q3.y, r, r.mx, r.my, r.mz, e1, x1);
+            const bool in0 = !((e0 > x0) | (x0 < 0.0f) | (e0 > tmax_guard));
+            const bool in1 = !((e1 > x1) | (x1 < 0.0f) | (e1 > tmax_guard));
+            const uint32_t ref0 = __float_as_uint(q1.z), ref1 = __float_as_uint(q3.z);
+            if (in0 & in1) {
+                const bool second_first = e1 < e0;
+                stack[sp++] = second_first ? ref0 : ref1;
+                item = second_first ? ref1 : ref0;
+                continue;
+            }
+            if (in0 | in1) { item = in0 ? ref0 : ref1; continue; }
+        }
+        if (sp == 0) break;
+        item = stack[--sp];
+    }
+    if (COUNT && counters) { atomicAdd(&counters[0], (unsigned long long)n_nodes); atomicAdd(&counters[1], (unsigned long long)n_prims); }
+    if (occluded || !candidate) return occluded;
+    return shadow_fallback<COUNT>(sc, o, d, tmax, counters, error_flag);
+}
+
 // ------------------------------------------------------------------ warp-synchronous traversal with batched leaves
 // Same walk, same order, same tests as traverse<>() per ray - only WHEN a lane runs the primitive tests of a leaf changes.
 // In the plain loop a warp executes the ~120-instruction triangle test whenever ANY of its lanes stands on a leaf;

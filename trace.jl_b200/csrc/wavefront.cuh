@@ -45,7 +45,8 @@ __global__ void __launch_bounds__(128, TR_TRAV_MIN_BLOCKS) k_wh_extend(DeviceSce
     }
 }
 
-template <int SLAB, bool COUNT, int WAIT>
+// TREE: walk the shadow tree (traverse_shadow; sc.shadow_pairs is set), else the reference tree
+template <int SLAB, bool COUNT, int WAIT, bool TREE>
 __global__ void __launch_bounds__(128, TR_TRAV_MIN_BLOCKS) k_wh_shadow(DeviceScene sc, const float4* __restrict__ so, const float4* __restrict__ sd,
                                                    const float4* __restrict__ contrib, const int* __restrict__ count, int cap,
                                                    float4* __restrict__ accum, unsigned long long* counters, int* error_flag) {
@@ -55,8 +56,13 @@ __global__ void __launch_bounds__(128, TR_TRAV_MIN_BLOCKS) k_wh_shadow(DeviceSce
         const int i = base + lane;
         const bool valid = i < n;
         const float4 o = valid ? q_load(&so[i]) : make_float4(0.0f, 0.0f, 0.0f, 0.0f), d = valid ? q_load(&sd[i]) : make_float4(1.0f, 1.0f, 1.0f, 0.0f);
-        HitRecord h;
-        if (!traverse_any<SLAB, true, COUNT, WAIT>(sc, valid, xyz(o), xyz(d), o.w, h, counters, error_flag) && valid) {
+        bool occ;
+        if (TREE) occ = !valid || traverse_shadow<COUNT>(sc, xyz(o), xyz(d), o.w, counters, error_flag);
+        else {
+            HitRecord h;
+            occ = traverse_any<SLAB, true, COUNT, WAIT>(sc, valid, xyz(o), xyz(d), o.w, h, counters, error_flag);
+        }
+        if (!occ && valid) {
             const float4 c = q_load(&contrib[i]);
             atomicAdd(&accum[__float_as_int(d.w)], make_float4(c.x, c.y, c.z, 0.0f));   // 128-bit vector atomic (sm_90+)
         }
@@ -83,16 +89,19 @@ static void launch_extend_plain(trace_ctx* c, int grid, Args... args) {
     c->stats.kernel_launches++;
     c->kev_end();
 }
-template <class... Args>
-static void launch_shadow_plain(trace_ctx* c, int grid, Args... args) {
+static void launch_shadow_plain(trace_ctx* c, DeviceScene sc, const float4* so, const float4* sd, const float4* contrib,
+                                const int* count, int cap, float4* accum, unsigned long long* counters, int* err) {
     c->kev_begin(1);
     trav_dispatch(c, [&](auto S, auto C_, auto W) {
-        k_wh_shadow<decltype(S)::value, decltype(C_)::value, decltype(W)::value><<<persistent_grid(c, 16), 128, 0, c->cur_stream>>>(args...);
+        constexpr int s = decltype(S)::value, w = decltype(W)::value;
+        constexpr bool cn = decltype(C_)::value;
+        auto k = k_wh_shadow<s, cn, w, false>;
+        if constexpr (shadow_walk_capable<s, cn, w>) if (sc.shadow_pairs) k = k_wh_shadow<s, cn, w, true>;
+        k<<<persistent_grid(c, 16), 128, 0, c->cur_stream>>>(sc, so, sd, contrib, count, cap, accum, counters, err);
     });
     c->stats.kernel_launches++;
     c->kev_end();
 }
-
 
 static void launch_extend(trace_ctx* c, int grid, DeviceScene sc, const float4* ro, const float4* rd, const int* count, int cap,
                           float4* hits, unsigned long long* counters, int* err, const int* count_back = nullptr) {
@@ -100,5 +109,5 @@ static void launch_extend(trace_ctx* c, int grid, DeviceScene sc, const float4* 
 }
 static void launch_shadow(trace_ctx* c, int grid, DeviceScene sc, const float4* so, const float4* sd, const float4* contrib,
                           const int* count, int cap, float4* accum, unsigned long long* counters, int* err) {
-    launch_shadow_plain(c, grid, sc, so, sd, contrib, count, cap, accum, counters, err);
+    launch_shadow_plain(c, shadow_launch_scene(c, sc), so, sd, contrib, count, cap, accum, counters, err);
 }

@@ -647,7 +647,7 @@ int whitted_render_device(trace_ctx* c, const trace_camera* cam, const trace_fil
     if (c->graph && !c->time_kernels && (size_t)c->stream > 2) {       // (legacy / per-thread default streams cannot be captured)
         std::string key((const char*)lane.data(), lane.size() * sizeof(WhittedLaunch));
         key.append((const char*)b_count.data(), b_count.size() * sizeof(long long));
-        const long long extra[] = {nb, batch, K, total_slots, (long long)(size_t)d_flags, c->slab, c->persist, c->count_nodes, c->leaf_wait, c->fuse_primary,
+        const long long extra[] = {nb, batch, K, total_slots, (long long)(size_t)d_flags, c->slab, c->persist, c->count_nodes, c->leaf_wait, c->fuse_primary, c->shadow_tree,
                                    (long long)(size_t)c->stream};
         key.append((const char*)extra, sizeof(extra));
         if (!c->wh_graph || key != c->wh_graph_key) {

@@ -258,10 +258,25 @@ class Context:
         self.check(self.lib.trace_scene_copy_nodes(self.h, _lib.ptr(nodes)))
         return nodes
 
+    def shadow_tree(self):
+        """The uploaded scene's shadow tree as its pair records (trace_scene_shadow_tree): float32 [n_prims - 1, 16]
+        (viewed as uint32, columns 6, 7, 14, 15 are references and split-axis bits), or None when the scene has none."""
+        n = C.c_int64()
+        self.check(self.lib.trace_scene_shadow_tree(self.h, C.byref(n), None))
+        if n.value == 0:
+            return None
+        pairs = np.zeros((n.value, 16), dtype=np.float32)
+        self.check(self.lib.trace_scene_shadow_tree(self.h, C.byref(n), _lib.ptr(pairs)))
+        return pairs
+
     def stats(self):
         s = _lib.Stats()
         self.check(self.lib.trace_get_stats(self.h, C.byref(s)))
-        return s.as_dict()
+        out = s.as_dict()
+        fb = C.c_uint64()
+        self.check(self.lib.trace_get_shadow_fallbacks(self.h, C.byref(fb)))
+        out["shadow_fallbacks"] = fb.value
+        return out
 
     def reset_stats(self):
         self.check(self.lib.trace_reset_stats(self.h))
