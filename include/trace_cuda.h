@@ -6,6 +6,7 @@
  *
  *   trace_bvh_build            <- BVHAccel(primitives, max_node_primitives)   src/accel/bvh.jl:55-80 (+ _init :87-185, _unroll :187-206)
  *   trace_scene_upload         <- Scene(lights, aggregate)                    src/Trace.jl:176-187
+ *   trace_scene_upload_mesh_device  (extension: a triangle scene built and packed on the GPU from device arrays)
  *   trace_intersect            <- intersect!(bvh|scene, ray)                  src/accel/bvh.jl:212-258, src/Trace.jl:189-191
  *   trace_occluded             <- intersect_p(bvh|scene, ray)                 src/accel/bvh.jl:260-299, src/Trace.jl:192-194
  *   trace_render_whitted       <- (i::SamplerIntegrator)(scene)               src/integrators/sampler.jl:12-56
@@ -228,6 +229,37 @@ int trace_comm_destroy(trace_ctx* ctx);
 int trace_comm_info(const trace_ctx* ctx, int* rank, int* world, int* nccl_version /* 0: no communicator */);
 
 int trace_scene_upload(trace_ctx* ctx, const trace_scene_desc* scene);
+
+/* ---- device mesh upload (extension: the reference has no counterpart).  A triangle-only scene whose per-triangle
+ * arrays are already in device memory on the context's GPU: the GPU builds its tree (the LBVH of trace_bvh_build_gpu)
+ * and writes every scene buffer; no array proportional to n_tris crosses to the host (the host reads the build's
+ * status block and the root box).  The resulting device scene is bit for bit the one trace_scene_upload builds from
+ *   nodes     = trace_bvh_build_gpu(device, B, n_tris, max_node_primitives), B[i] = Julia min / max (-0.0 < +0.0) of
+ *               triangle i's three vertices (the refit's leaf rule);
+ *   prims[k]  = {TRACE_PRIM_TRIANGLE, order[k], tri_materials[order[k]], order[k]}: `original` is the triangle index;
+ *   the same triangle arrays (tri_normals NULL: zeros, TRACE_TRI_HAS_NORMALS cleared), no spheres, these materials
+ *   and lights
+ * - nodes, pair records, primitive records, normals and flags, shadow tree, scene_scale and counts alike.
+ * Refused, before any scene buffer is written (the previous scene stays uploaded and usable): NaN in a vertex or a
+ * normal, a material index >= n_materials, a tree deeper than 64 levels, n_tris >= 2^30, a NULL vertex array with
+ * n_tris > 0, an unknown material or light kind.  n_tris == 0 uploads the empty scene, n_tris == 1 a single leaf.
+ * The arrays are read on the context's stream: the caller orders the work that wrote them before this call.  Like
+ * trace_scene_upload the call waits for all of the context's work, ends any SPPM session and is synchronous.  Its
+ * scratch (the build's and the shadow tree's) lives in grow-only context buffers: a repeated upload of the same size
+ * allocates nothing.  trace_scene_refit[_device] applies afterwards (the slot -> triangle map stays on the device).
+ * *n_nodes_out (may be NULL) receives the node count.  TRACE_BVH_PROFILE=1 prints per-phase CUDA-event times. */
+typedef struct trace_mesh_device_desc {
+    int64_t n_tris;
+    const void* tri_vertices;     /* device [n_tris][3][3] float32, world space */
+    const void* tri_normals;      /* device [n_tris][3][3] float32, or NULL */
+    const void* tri_flags;        /* device [n_tris] uint8 TRACE_TRI_*, or NULL (all 0) */
+    const void* tri_materials;    /* device [n_tris] uint32 index into materials, or NULL (all 0) */
+    int32_t max_node_primitives;  /* clamped to 1..255 as trace_bvh_build_gpu */
+    int32_t pad;
+    int64_t n_materials;  const trace_material* materials;   /* host */
+    int64_t n_lights;     const trace_light* lights;         /* host */
+} trace_mesh_device_desc;
+int trace_scene_upload_mesh_device(trace_ctx* ctx, const trace_mesh_device_desc* mesh, int64_t* n_nodes_out);
 
 /* ---- refit (extension: the reference has no counterpart; it rebuilds BVHAccel).  New positions for the triangles of
  * the last upload, with the tree's topology kept (node structure, primitive order, materials, spheres, lights) and every

@@ -278,6 +278,36 @@ function refit!(ctx::Context, scene::Trace.Scene)
     nothing
 end
 
+# Geometry made on the GPU (CUDA.jl arrays of a simulation, a procedural mesh, a change of topology): upload it without a
+# round trip through host memory.  The library builds the LBVH and packs every scene buffer on the device
+# (trace_scene_upload_mesh_device); the scene is the one BVHAccel(builder="lbvh") + Scene would give, with the triangle
+# index as the primitive index.  Pointers are raw device addresses on ctx's GPU (e.g. UInt(pointer(cu_array))), read on
+# the context's stream: synchronise the work that wrote them first.  `materials` / `lights` are host pods
+# (material_pod / light_pod).  Returns the node count; refit! does not apply (call trace_scene_refit_device directly).
+struct MeshDeviceDesc
+    n_tris::Int64
+    tri_vertices::UInt          # device Float32 [9, n_tris] (x y z of p0 p1 p2 per triangle)
+    tri_normals::UInt           # same layout, or 0
+    tri_flags::UInt             # device UInt8 [n_tris] (bit 0 flip, bit 1 has normals), or 0
+    tri_materials::UInt         # device UInt32 [n_tris], 0-based into materials, or 0 (all 0)
+    max_node_primitives::Int32
+    pad::Int32
+    n_materials::Int64; materials::Ptr{Cvoid}
+    n_lights::Int64; lights::Ptr{Cvoid}
+end
+function upload_mesh_device!(ctx::Context, n_tris, vertices, normals, flags, material_ids, materials::Vector, lights::Vector;
+                             max_node_primitives = 1)
+    GC.@preserve materials lights begin
+        d = MeshDeviceDesc(n_tris, UInt(vertices), UInt(normals), UInt(flags), UInt(material_ids), Int32(max_node_primitives),
+                           Int32(0), length(materials), pointer(materials), length(lights), pointer(lights))
+        n_nodes = Ref{Int64}(0)
+        check(ctx, ccall((:trace_scene_upload_mesh_device, LIB), Cint, (Ptr{Cvoid}, Ref{MeshDeviceDesc}, Ref{Int64}),
+                         ctx.h, d, n_nodes))
+    end
+    delete!(UPLOADED, ctx)         # the uploaded scene is no Trace.Scene of this shim
+    n_nodes[]
+end
+
 # ---- the two functors ------------------------------------------------------------------------------------------------
 struct GPU{I<:Trace.Integrator,C}
     integrator::I

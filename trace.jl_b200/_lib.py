@@ -37,6 +37,15 @@ class SceneDesc(C.Structure):
                 ("n_lights", C.c_int64), ("lights", C.c_void_p)]
 
 
+class MeshDeviceDesc(C.Structure):
+    """trace_mesh_device_desc: per-triangle arrays in device memory (raw pointers), materials and lights in host memory"""
+    _fields_ = [("n_tris", C.c_int64), ("tri_vertices", C.c_void_p), ("tri_normals", C.c_void_p),
+                ("tri_flags", C.c_void_p), ("tri_materials", C.c_void_p),
+                ("max_node_primitives", C.c_int32), ("pad", C.c_int32),
+                ("n_materials", C.c_int64), ("materials", C.c_void_p),
+                ("n_lights", C.c_int64), ("lights", C.c_void_p)]
+
+
 class Camera(C.Structure):
     _fields_ = [("raster_to_camera", C.c_float * 16), ("camera_to_world", C.c_float * 16),
                 ("lens_radius", C.c_float), ("focal_distance", C.c_float),
@@ -90,6 +99,7 @@ SIGNATURES = {
     "trace_comm_destroy": (C.c_int, [_P]),
     "trace_comm_info": (C.c_int, [_P, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "trace_scene_upload": (C.c_int, [_P, C.POINTER(SceneDesc)]),
+    "trace_scene_upload_mesh_device": (C.c_int, [_P, C.POINTER(MeshDeviceDesc), C.POINTER(C.c_int64)]),
     "trace_scene_refit": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int64, _P]),
     "trace_scene_refit_device": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int64, _P]),
     "trace_scene_copy_nodes": (C.c_int, [_P, _P]),

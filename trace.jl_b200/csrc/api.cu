@@ -94,7 +94,8 @@ extern "C" void trace_destroy(trace_ctx* c) {
     sppm_free(c);
     trace_comm_destroy(c);
     DevBuf* all[] = {&c->b_nodes, &c->b_pairs, &c->b_prims, &c->b_tnorm, &c->b_spheres, &c->b_materials, &c->b_lights, &c->b_counters,
-                     &c->b_shadow, &c->refit.topo, &c->refit.stage, &c->refit.sphere_bounds, &c->refit.shadow_topo};
+                     &c->b_shadow, &c->refit.topo, &c->refit.stage, &c->refit.sphere_bounds, &c->refit.shadow_topo,
+                     &c->refit.slot_tri_dev, &c->b_build};
     for (DevBuf* b : all) b->release();
     for (auto& b : c->b_query) b.release();
     for (auto& b : c->b_queue) b.release();
@@ -310,9 +311,34 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
         static_assert(sizeof(DeviceSphere) == sizeof(trace_sphere), "sphere layout");
         memcpy(&spheres[i], &d->spheres[i], sizeof(trace_sphere));
     }
-    std::vector<DeviceMaterial> mats((size_t)d->n_materials);
-    for (int64_t i = 0; i < d->n_materials; ++i) {
-        const trace_material& m = d->materials[i];
+    std::vector<DeviceMaterial> mats;
+    std::vector<DeviceLight> lights;
+    if (ctx_pack_materials(c, d->n_materials, d->materials, mats) || ctx_pack_lights(c, d->n_lights, d->lights, lights)) return 1;
+    // --- upload
+    TR_CUDA(c, cudaStreamSynchronize(c->stream));
+    if (ctx_put(c, c->b_nodes, nodes.data(), nodes.size() * sizeof(float4)) ||
+        ctx_put(c, c->b_pairs, pairs.data(), pairs.size() * sizeof(float4)) ||
+        ctx_put(c, c->b_prims, prims.data(), prims.size() * sizeof(float4)) ||
+        ctx_put(c, c->b_tnorm, tnorm.data(), tnorm.size() * sizeof(float4)) ||
+        ctx_put(c, c->b_spheres, spheres.data(), spheres.size() * sizeof(DeviceSphere)) ||
+        ctx_put(c, c->b_materials, mats.data(), mats.size() * sizeof(DeviceMaterial)) ||
+        ctx_put(c, c->b_lights, lights.data(), lights.size() * sizeof(DeviceLight)))
+        return 1;
+    TR_CUDA(c, cudaStreamSynchronize(c->stream));      // host staging vectors die at return
+    float root_box[6] = {};
+    if (d->n_nodes > 0)
+        for (int k = 0; k < 3; ++k) { root_box[k] = d->nodes[0].bmin[k]; root_box[3 + k] = d->nodes[0].bmax[k]; }
+    c->refit.tri_index.swap(tri_index);
+    c->refit.slot_tri_on_device = false;
+    return ctx_commit_scene(c, d->n_nodes, d->n_prims, d->n_spheres, d->n_materials, d->n_lights, d->n_tris, n_pairs,
+                            root_ref, root_box, nullptr);
+}
+
+int ctx_pack_materials(trace_ctx* c, int64_t n, const trace_material* in, std::vector<DeviceMaterial>& out) {
+    if (n < 0 || (n > 0 && !in)) return c->fail("scene: bad material array");
+    out.resize((size_t)n);
+    for (int64_t i = 0; i < n; ++i) {
+        const trace_material& m = in[i];
         DeviceMaterial dm;
         memset(&dm, 0, sizeof(dm));
         dm.kind = m.kind;
@@ -333,11 +359,16 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
             float r = m.remap ? remap_alpha(m.rough_u) : m.rough_u;
             dm.alpha_u = dm.alpha_v = fmaxf(1e-3f, r);           // TrowbridgeReitzDistribution clamps, microfacet.jl:58-62
         } else if (m.kind != TRACE_MAT_MIRROR) return c->fail("material %lld: unknown kind %u", (long long)i, m.kind);
-        mats[i] = dm;
+        out[i] = dm;
     }
-    std::vector<DeviceLight> lights((size_t)d->n_lights);
-    for (int64_t i = 0; i < d->n_lights; ++i) {
-        const trace_light& l = d->lights[i];
+    return 0;
+}
+
+int ctx_pack_lights(trace_ctx* c, int64_t n, const trace_light* in, std::vector<DeviceLight>& out) {
+    if (n < 0 || (n > 0 && !in)) return c->fail("scene: bad light array");
+    out.resize((size_t)n);
+    for (int64_t i = 0; i < n; ++i) {
+        const trace_light& l = in[i];
         DeviceLight dl;
         dl.kind = l.kind;
         memcpy(dl.m, l.m, sizeof(dl.m)); memcpy(dl.inv_m, l.inv_m, sizeof(dl.inv_m));
@@ -345,51 +376,49 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
         dl.cos_total = l.cos_total_width; dl.cos_falloff = l.cos_falloff_start;
         if (l.kind != TRACE_LIGHT_POINT && l.kind != TRACE_LIGHT_SPOT && l.kind != TRACE_LIGHT_DIRECTIONAL)
             return c->fail("light %lld: unknown kind", (long long)i);
-        lights[i] = dl;
+        out[i] = dl;
     }
-    // --- upload
-    auto put = [&](DevBuf& b, const void* src, size_t bytes) -> cudaError_t {
-        cudaError_t e = b.ensure(bytes ? bytes : 16);
-        if (e != cudaSuccess) return e;
-        if (bytes) e = cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, c->stream);
-        return e;
-    };
-    TR_CUDA(c, cudaStreamSynchronize(c->stream));
-    TR_CUDA(c, put(c->b_nodes, nodes.data(), nodes.size() * sizeof(float4)));
-    TR_CUDA(c, put(c->b_pairs, pairs.data(), pairs.size() * sizeof(float4)));
-    TR_CUDA(c, put(c->b_prims, prims.data(), prims.size() * sizeof(float4)));
-    TR_CUDA(c, put(c->b_tnorm, tnorm.data(), tnorm.size() * sizeof(float4)));
-    TR_CUDA(c, put(c->b_spheres, spheres.data(), spheres.size() * sizeof(DeviceSphere)));
-    TR_CUDA(c, put(c->b_materials, mats.data(), mats.size() * sizeof(DeviceMaterial)));
-    TR_CUDA(c, put(c->b_lights, lights.data(), lights.size() * sizeof(DeviceLight)));
-    TR_CUDA(c, cudaStreamSynchronize(c->stream));      // host staging vectors die at return
+    return 0;
+}
+
+// host -> device into a grow-only scene buffer (16 bytes for an empty array), on the context's stream
+int ctx_put(trace_ctx* c, DevBuf& b, const void* src, size_t bytes) {
+    TR_CUDA(c, b.ensure(bytes ? bytes : 16));
+    if (bytes) TR_CUDA(c, cudaMemcpyAsync(b.p, src, bytes, cudaMemcpyHostToDevice, c->stream));
+    return 0;
+}
+
+// The tail of every upload, once the scene buffers hold the new scene: the DeviceScene, scene_scale from the root box
+// (min xyz, max xyz), the shadow tree, the refit state and the end of any SPPM session.  The caller sets the refit's
+// slot -> triangle map.
+int ctx_commit_scene(trace_ctx* c, int64_t n_nodes, int64_t n_prims, int64_t n_spheres, int64_t n_materials,
+                     int64_t n_lights, int64_t n_tris, int64_t n_pairs, uint32_t root_ref, const float* root_box,
+                     void* shadow_scratch) {
     DeviceScene& s = c->scene;
     s.nodes = c->b_nodes.as<float4>(); s.pairs = c->b_pairs.as<float4>(); s.root_ref = root_ref; s.prims = c->b_prims.as<float4>(); s.tnorm = c->b_tnorm.as<float4>();
     s.spheres = c->b_spheres.as<DeviceSphere>(); s.materials = c->b_materials.as<DeviceMaterial>();
     s.lights = c->b_lights.as<DeviceLight>();
-    s.n_nodes = (int)d->n_nodes; s.n_prims = (int)d->n_prims; s.n_spheres = (int)d->n_spheres;
-    s.n_materials = (int)d->n_materials; s.n_lights = (int)d->n_lights;
+    s.n_nodes = (int)n_nodes; s.n_prims = (int)n_prims; s.n_spheres = (int)n_spheres;
+    s.n_materials = (int)n_materials; s.n_lights = (int)n_lights;
     s.scene_scale = 0.0f;
-    if (d->n_nodes > 0) {
-        for (int k = 0; k < 3; ++k) {
-            const float a = fabsf(d->nodes[0].bmin[k]), b = fabsf(d->nodes[0].bmax[k]);
+    if (n_nodes > 0) {
+        for (int k = 0; k < 6; ++k) {
+            const float a = fabsf(root_box[k]);
             if (std::isfinite(a)) s.scene_scale = fmaxf(s.scene_scale, a);
-            if (std::isfinite(b)) s.scene_scale = fmaxf(s.scene_scale, b);
         }
     }
     // the shadow tree (traverse.cuh, traverse_shadow): built on the device from the uploaded primitive records.  Scenes
     // with analytic spheres have none (the guard its walk admits nodes with is off below spheres); neither has a scene
     // uploaded with option shadow_tree 0
     s.shadow_pairs = nullptr;
-    if (c->shadow_tree && d->n_spheres == 0 && d->n_prims >= 2) {
-        TR_CUDA(c, c->b_shadow.ensure((size_t)(d->n_prims - 1) * 4 * sizeof(float4)));
-        const int rc = shadow_tree_build(c->stream, c->b_prims.p, d->n_prims, c->b_shadow.p);
+    if (c->shadow_tree && n_spheres == 0 && n_prims >= 2) {
+        TR_CUDA(c, c->b_shadow.ensure((size_t)(n_prims - 1) * 4 * sizeof(float4)));
+        const int rc = shadow_tree_build(c->stream, c->b_prims.p, n_prims, c->b_shadow.p, shadow_scratch);
         if (rc == 0) s.shadow_pairs = c->b_shadow.as<float4>();
         else if (rc != 5 && rc != 6) return c->fail("scene: shadow tree build failed (CUDA error)");
     }
     c->have_scene = true;
-    c->refit.tri_index.swap(tri_index);
-    c->refit.n_tris = d->n_tris; c->refit.n_spheres = d->n_spheres; c->refit.n_pairs = n_pairs;
+    c->refit.n_tris = n_tris; c->refit.n_spheres = n_spheres; c->refit.n_pairs = n_pairs;
     c->refit.topo_ready = false;
     c->refit.shadow_topo_ready = false;
     sppm_end_session(c);

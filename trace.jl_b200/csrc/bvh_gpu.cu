@@ -33,6 +33,7 @@ struct Status {
     uint32_t cmin[3], cmax[3];      // centroid box as order-preserving keys (ord_key)
     uint32_t nan;                   // a centroid is NaN
     uint32_t root_size, root_depth; // emitted nodes, levels (root = 1)
+    uint32_t bad;                   // mesh builds: a NaN normal (bit 0), a material index out of range (bit 1)
 };
 
 // float <-> uint32 in Julia's total order on non-NaN floats (-0.0 sorts below +0.0), so atomicMin / atomicMax pick it
@@ -244,10 +245,17 @@ struct Buffers {
     int alloc(int64_t n, size_t sort_bytes, bool with_pb, bool with_nodes) {
         carve(n, sort_bytes, with_pb, with_nodes);
         if (cudaMalloc(&base, used) != cudaSuccess) { cudaGetLastError(); base = nullptr; return 7; }
+        owned = true;
         carve(n, sort_bytes, with_pb, with_nodes);
         return 0;
     }
-    ~Buffers() { if (base) cudaFree(base); }
+    // the caller's allocation of at least lbvh_scratch_bytes(n) bytes (with pb, without nodes); kept by the caller
+    void borrow(void* scratch, int64_t n, size_t sort_bytes) {
+        base = static_cast<char*>(scratch);
+        carve(n, sort_bytes, true, false);
+    }
+    bool owned = false;
+    ~Buffers() { if (owned) cudaFree(base); }
 };
 
 struct Phases {
@@ -268,13 +276,16 @@ size_t sort_bytes_for(int64_t n, cudaStream_t s) {
 // The device-resident core: bounds b.pb (device, [n][6]) -> keys, sorted order, hierarchy, boxes, subtree sizes and
 // depths in `b`, and the status on the host.  Returns 0, 5 (a NaN bound), 6 (deeper than the 64-entry traversal
 // stack) or 7 (CUDA error).
-int build_core(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, Status& hs, Phases& ph) {
-    const int64_t nn = 2 * n - 1;
-    const int T = 256;
+void core_reset(cudaStream_t s, int64_t n, Buffers& b) {
     cudaMemsetAsync(b.st, 0xFF, sizeof(b.st->cmin), s);
     cudaMemsetAsync(&b.st->cmax, 0, sizeof(Status) - sizeof(b.st->cmin), s);
-    cudaMemsetAsync(b.parent, 0xFF, (size_t)nn * sizeof(int32_t), s);
+    cudaMemsetAsync(b.parent, 0xFF, (size_t)(2 * n - 1) * sizeof(int32_t), s);
     if (n > 1) cudaMemsetAsync(b.arrive, 0, (size_t)(n - 1) * sizeof(uint32_t), s);
+}
+
+// build_core without the reset: what runs after core_reset (and anything that reports into the status block)
+int core_run(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, Status& hs, Phases& ph) {
+    const int T = 256;
     lbvh_centroid_box<<<(unsigned)std::min<int64_t>(blocks_for(n, T), 4096), T, 0, s>>>(b.pb, n, b.st);
     lbvh_keys<<<blocks_for(n, T), T, 0, s>>>(b.pb, n, b.st, b.keys, b.ids);
     ph.mark(s);
@@ -294,6 +305,11 @@ int build_core(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, 
     if (hs.nan) return 5;
     if (hs.root_depth > 64) return 6;                        // TR_STACK_SIZE (traverse.cuh): the walks' stacks would overflow
     return 0;
+}
+
+int build_core(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, Status& hs, Phases& ph) {
+    core_reset(s, n, b);
+    return core_run(s, n, m, b, sort_bytes, hs, ph);
 }
 
 int build(cudaStream_t s, const float* hb, int64_t n, int m, trace_bvh** out, Phases& ph) {
@@ -363,17 +379,57 @@ __global__ void lbvh_emit_pairs(int64_t n, const uint32_t* __restrict__ child, c
     }
 }
 
+// ------------------------------------------------------------------ mesh builds (trace_scene_upload_mesh_device, upload_device.cu)
+// The inputs a triangle array brings beyond its vertices: any NaN normal (bit 0) and any material index >= n_materials
+// (bit 1) into the status block, which the build reads back before anything is emitted.
+__global__ void lbvh_mesh_validate(const float* __restrict__ nrm, const uint32_t* __restrict__ mat, int64_t n,
+                                   uint32_t n_materials, Status* st) {
+    uint32_t bad = 0;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        if (nrm)
+            for (int k = 0; k < 9; ++k) { const float x = nrm[9 * i + k]; if (x != x) bad |= 1u; }
+        if ((mat ? mat[i] : 0u) >= n_materials) bad |= 2u;
+    }
+    bad = __reduce_or_sync(0xFFFFFFFFu, bad);
+    if ((threadIdx.x & 31) == 0 && bad) atomicOr(&st->bad, bad);
+}
+
+// A triangle's box from the [n][3][3] vertex array: the rule of lbvh_prim_bounds (a NaN vertex makes the box NaN)
+__global__ void lbvh_tri_bounds(const float* __restrict__ v, int64_t n, float* __restrict__ pb) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float* p = v + 9 * i;
+    bool nan = false;
+    for (int k = 0; k < 9; ++k) nan |= p[k] != p[k];
+    for (int c = 0; c < 3; ++c) {
+        pb[6 * i + c] = nan ? NAN : jl_min(jl_min(jl_min(INFINITY, p[c]), p[3 + c]), p[6 + c]);
+        pb[6 * i + 3 + c] = nan ? NAN : jl_max(jl_max(jl_max(-INFINITY, p[c]), p[3 + c]), p[6 + c]);
+    }
+}
+
 }  // namespace
+
+// Scratch of one LBVH build over n primitives (bounds, keys, sort, hierarchy, boxes) in a caller-owned allocation;
+// 0 when CUB cannot size its sort.  The shadow tree's build of the same n fits the same bytes.
+size_t lbvh_scratch_bytes(int64_t n, cudaStream_t s) {
+    const size_t sort_bytes = sort_bytes_for(n, s);
+    if (!sort_bytes) return 0;
+    Buffers b;
+    b.carve(n, sort_bytes, true, false);
+    return b.used;
+}
 
 // The shadow tree of an uploaded scene (api.cu): an LBVH with one primitive per leaf over the n >= 2 uploaded primitive
 // records `prims` (device, BVH slot order, triangles only), written as n - 1 pair records to `pairs` (device).  Nothing
-// crosses to the host but the build's status.  Returns 0, 5 (a NaN vertex), 6 (deeper than 64 levels) or 7 (CUDA error).
-int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs) {
+// crosses to the host but the build's status.  `scratch` (lbvh_scratch_bytes(n)) or nullptr: an allocation of its own.
+// Returns 0, 5 (a NaN vertex), 6 (deeper than 64 levels) or 7 (CUDA error).
+int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs, void* scratch) {
     if (n < 2 || n >= 0x40000000ll) return 1;
     const size_t sort_bytes = sort_bytes_for(n, s);
     if (!sort_bytes) return 7;
     Buffers b;
-    if (b.alloc(n, sort_bytes, true, false)) return 7;
+    if (scratch) b.borrow(scratch, n, sort_bytes);
+    else if (b.alloc(n, sort_bytes, true, false)) return 7;
     const int T = 256;
     lbvh_prim_bounds<<<blocks_for(n, T), T, 0, s>>>(static_cast<const float4*>(prims), n, b.pb);
     Phases ph;
@@ -382,6 +438,65 @@ int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs)
     lbvh_emit_pairs<<<blocks_for(n - 1, T), T, 0, s>>>(n, b.child, b.ids_sorted, b.axis, b.box, static_cast<float4*>(pairs));
     if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess) return 7;
     return 0;
+}
+
+// The tree of trace_scene_upload_mesh_device, in steps over `scratch` (lbvh_scratch_bytes(n), n >= 1):
+//   lbvh_mesh_validate  reset the status block, check normals (NULL: none) and material indices (NULL: all 0) into it;
+//   lbvh_mesh_bounds    the triangles' boxes (no host wait so far);
+//   lbvh_mesh_build     the LBVH core and its status read back: 0, 5 a NaN vertex, 6 deeper than 64 levels, 7 CUDA
+//                       error, 8 a NaN normal, 9 a material index out of range; *n_nodes, and *order = the sorted
+//                       triangle ids (slot -> triangle, device, inside the scratch);
+//   lbvh_mesh_emit      the preorder node records (trace_bvh_node, 32 B) into `nodes` (device).
+// Nothing is written outside the scratch before lbvh_mesh_emit, so a refused input leaves the caller's buffers intact.
+int lbvh_mesh_validate(cudaStream_t s, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n, void* scratch) {
+    const size_t sort_bytes = sort_bytes_for(n, s);
+    if (!sort_bytes) return 7;
+    Buffers b;
+    b.borrow(scratch, n, sort_bytes);
+    core_reset(s, n, b);
+    const int T = 256;
+    const uint32_t nm = n_materials > 0xFFFFFFFFll ? 0xFFFFFFFFu : (uint32_t)n_materials;
+    lbvh_mesh_validate<<<(unsigned)std::min<int64_t>(blocks_for(n, T), 4096), T, 0, s>>>(nrm, mat, n, nm, b.st);
+    return cudaGetLastError() == cudaSuccess ? 0 : 7;
+}
+
+int lbvh_mesh_bounds(cudaStream_t s, const float* v, int64_t n, void* scratch) {
+    const size_t sort_bytes = sort_bytes_for(n, s);
+    if (!sort_bytes) return 7;
+    Buffers b;
+    b.borrow(scratch, n, sort_bytes);
+    const int T = 256;
+    lbvh_tri_bounds<<<blocks_for(n, T), T, 0, s>>>(v, n, b.pb);
+    return cudaGetLastError() == cudaSuccess ? 0 : 7;
+}
+
+int lbvh_mesh_build(cudaStream_t s, int64_t n, int m, void* scratch, int64_t* n_nodes, const uint32_t** order) {
+    const size_t sort_bytes = sort_bytes_for(n, s);
+    if (!sort_bytes) return 7;
+    Buffers b;
+    b.borrow(scratch, n, sort_bytes);
+    Phases ph;
+    Status hs;
+    const int rc = core_run(s, n, m, b, sort_bytes, hs, ph);
+    if (rc == 7) return 7;
+    if (hs.nan) return 5;                  // the order of the refusals: vertices, normals, materials, depth
+    if (hs.bad & 1u) return 8;
+    if (hs.bad & 2u) return 9;
+    if (rc) return rc;
+    *n_nodes = hs.root_size;
+    *order = b.ids_sorted;
+    return 0;
+}
+
+int lbvh_mesh_emit(cudaStream_t s, int64_t n, int m, void* scratch, void* nodes) {
+    const size_t sort_bytes = sort_bytes_for(n, s);
+    if (!sort_bytes) return 7;
+    Buffers b;
+    b.borrow(scratch, n, sort_bytes);
+    const int T = 256;
+    lbvh_emit<<<blocks_for(2 * n - 1, T), T, 0, s>>>(n, m, b.child, b.parent, b.first, b.count, b.axis, b.box, b.size,
+                                                    static_cast<trace_bvh_node*>(nodes));
+    return cudaGetLastError() == cudaSuccess ? 0 : 7;
 }
 
 extern "C" int trace_bvh_build_gpu(int device, const float* pb, int64_t n, int max_node_primitives, trace_bvh** out) {

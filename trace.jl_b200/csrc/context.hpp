@@ -117,12 +117,17 @@ struct trace_ctx {
     DeviceScene scene{};
     DevBuf b_nodes, b_pairs, b_prims, b_tnorm, b_spheres, b_materials, b_lights;
     DevBuf b_shadow;              // the shadow tree's pair records (scene.shadow_pairs), 64 B per primitive
+    // trace_scene_upload_mesh_device (upload_device.cu): the LBVH build's scratch, then the pair numbering's and the
+    // shadow tree build's (grow-only, so a per-frame rebuild of the same size allocates nothing)
+    DevBuf b_build;
 
     // refit (refit.cu): what trace_scene_refit needs of the last upload.  The host keeps only the BVH-slot -> triangle
     // map; the device topology (parents, pair slots, leaf list) is derived from b_nodes at the first refit after an
     // upload, so scenes that are never refit pay no device memory for it.
     struct Refit {
         std::vector<uint32_t> tri_index;   // [n_prims] trace_prim.index of triangle slots (0 for spheres)
+        DevBuf slot_tri_dev;               // the same map already on the device (a device mesh upload), used when
+        bool slot_tri_on_device = false;   // slot_tri_on_device: then tri_index is empty
         int64_t n_tris = 0, n_spheres = 0, n_pairs = 0;
         bool topo_ready = false;
         DevBuf topo, stage, sphere_bounds;
@@ -314,7 +319,49 @@ int whitted_render_device(trace_ctx* ctx, const trace_camera* cam, const trace_f
 void sppm_free(trace_ctx* ctx);
 void sppm_end_session(trace_ctx* ctx);
 void whitted_film_range(const trace_ctx* ctx, long long npix, long long* p0, long long* p1);
-// implemented in bvh_gpu.cu: the shadow tree over uploaded primitive records (0, 5 NaN, 6 too deep, 7 CUDA error)
-int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs);
+// implemented in bvh_gpu.cu: the shadow tree over uploaded primitive records (0, 5 NaN, 6 too deep, 7 CUDA error), in
+// `scratch` (lbvh_scratch_bytes(n) bytes) or, with nullptr, an allocation of its own; the device mesh build's steps
+int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs, void* scratch);
+size_t lbvh_scratch_bytes(int64_t n, cudaStream_t s);
+int lbvh_mesh_validate(cudaStream_t s, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n, void* scratch);
+int lbvh_mesh_bounds(cudaStream_t s, const float* v, int64_t n, void* scratch);
+int lbvh_mesh_build(cudaStream_t s, int64_t n, int m, void* scratch, int64_t* n_nodes, const uint32_t** order);
+int lbvh_mesh_emit(cudaStream_t s, int64_t n, int m, void* scratch, void* nodes);
+// implemented in api.cu: the parts of a scene upload that do not depend on where the tree was built
+int ctx_pack_materials(trace_ctx* ctx, int64_t n, const trace_material* in, std::vector<DeviceMaterial>& out);
+int ctx_pack_lights(trace_ctx* ctx, int64_t n, const trace_light* in, std::vector<DeviceLight>& out);
+int ctx_put(trace_ctx* ctx, DevBuf& b, const void* src, size_t bytes);
+int ctx_commit_scene(trace_ctx* ctx, int64_t n_nodes, int64_t n_prims, int64_t n_spheres, int64_t n_materials,
+                     int64_t n_lights, int64_t n_tris, int64_t n_pairs, uint32_t root_ref, const float* root_box,
+                     void* shadow_scratch);
 // implemented in refit.cu: waits for every stream of the context (caller's, lanes, SPPM chain / collectives, copies)
 int ctx_drain(trace_ctx* ctx);
+// implemented in refit.cu: the upload's preorder pair numbering of a device node array (2 float4 per node), pair_of[i] =
+// interior nodes before node i, as an exclusive scan of "is interior" (`flag`: n words of scratch; `tmp`:
+// pair_scan_bytes(n) bytes of scan scratch)
+size_t pair_scan_bytes(int64_t n, cudaStream_t s);
+cudaError_t pair_numbering(cudaStream_t s, const float4* nodes, int64_t n, uint32_t* flag, uint32_t* pair_of, void* tmp,
+                           size_t tmp_bytes);
+
+// TRACE_BVH_PROFILE=1: CUDA events between the phases of an upload / refit call, printed as one stderr line
+struct PhaseTimer {
+    bool on = false;
+    cudaEvent_t ev[12] = {};
+    const char* name[12] = {};
+    int n = 0;
+    void mark(cudaStream_t s, const char* what) {      // `what` names the phase that ends here
+        if (!on || n >= 12) return;
+        if (!ev[n]) cudaEventCreate(&ev[n]);
+        name[n] = what;
+        cudaEventRecord(ev[n++], s);
+    }
+    void print(const char* head, double wall_ms) {     // after the last mark's work is done
+        fprintf(stderr, "%s, wall %.3f ms;", head, wall_ms);
+        for (int i = 1; i < n; ++i) {
+            float ms = 0.0f;
+            cudaEventElapsedTime(&ms, ev[i - 1], ev[i]);
+            fprintf(stderr, " %s %.3f ms%s", name[i], ms, i + 1 < n ? "," : "\n");
+        }
+    }
+    ~PhaseTimer() { for (auto e : ev) if (e) cudaEventDestroy(e); }
+};

@@ -206,42 +206,30 @@ __global__ void shadow_climb(const float4* __restrict__ prims, int64_t n_prims, 
 
 inline unsigned blocks_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
 
-struct Phases {
-    bool on = false;
-    cudaEvent_t ev[8] = {};
-    const char* name[8] = {};
-    int n = 0;
-    void mark(cudaStream_t s, const char* what) {      // `what` names the phase that ends here
-        if (!on || n >= 8) return;
-        if (!ev[n]) cudaEventCreate(&ev[n]);
-        name[n] = what;
-        cudaEventRecord(ev[n++], s);
-    }
-    ~Phases() { for (auto e : ev) if (e) cudaEventDestroy(e); }
-};
-
-// first refit after an upload: parents, pair slots and leaves from b_nodes, the slot -> triangle map from the host
+// first refit after an upload: parents, pair slots and leaves from b_nodes, the slot -> triangle map from the host (or,
+// after a device mesh upload, the one it left on the device)
 int derive_topology(trace_ctx* c) {
     auto& R = c->refit;
     const int64_t n = c->scene.n_nodes, n_prims = c->scene.n_prims, n_leaves = n - R.n_pairs;
-    size_t scan_bytes = 0;
-    TR_CUDA(c, cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)n, c->stream));
+    const size_t scan_bytes = pair_scan_bytes(n, c->stream);
+    if (!scan_bytes) return c->fail("scene refit: cannot size the pair scan");
     size_t used = 0;
     auto take = [&](size_t bytes) { const size_t off = (used + 255) & ~(size_t)255; used = off + bytes; return off; };
     const size_t o_parent = take(n * 4), o_up = take(n * 4), o_pair = take(n * 4), o_leaves = take(n_leaves * 4),
-                 o_empty = take(n), o_arrive = take(R.n_pairs * 4), o_tri = take(n_prims * 4), o_status = take(16),
+                 o_empty = take(n), o_arrive = take(R.n_pairs * 4), o_tri = take(R.slot_tri_on_device ? 0 : n_prims * 4),
+                 o_status = take(16),
                  o_scan = take(scan_bytes);
     TR_CUDA(c, R.topo.ensure(used));
     char* base = R.topo.as<char>();
     R.parent = (int32_t*)(base + o_parent); R.up = (uint32_t*)(base + o_up); R.pair_of = (uint32_t*)(base + o_pair);
     R.leaves = (uint32_t*)(base + o_leaves); R.empty = (uint8_t*)(base + o_empty); R.arrive = (uint32_t*)(base + o_arrive);
-    R.slot_tri = (uint32_t*)(base + o_tri); R.status = (uint32_t*)(base + o_status);
+    R.slot_tri = R.slot_tri_on_device ? R.slot_tri_dev.as<uint32_t>() : (uint32_t*)(base + o_tri);
+    R.status = (uint32_t*)(base + o_status);
     const int T = 256;
-    refit_is_interior<<<blocks_for(n, T), T, 0, c->stream>>>(c->scene.nodes, n, R.up);   // (`up` holds the flags until the scan)
-    TR_CUDA(c, cub::DeviceScan::ExclusiveSum(base + o_scan, scan_bytes, R.up, R.pair_of, (int)n, c->stream));
+    TR_CUDA(c, pair_numbering(c->stream, c->scene.nodes, n, R.up, R.pair_of, base + o_scan, scan_bytes));   // (`up` holds the flags until the scan)
     refit_topology<<<blocks_for(n, T), T, 0, c->stream>>>(c->scene.nodes, n, R.pair_of, R.parent, R.up, R.leaves);
     TR_CUDA(c, cudaGetLastError());
-    if (n_prims)
+    if (n_prims && !R.slot_tri_on_device)
         TR_CUDA(c, cudaMemcpyAsync(R.slot_tri, R.tri_index.data(), (size_t)n_prims * 4, cudaMemcpyHostToDevice, c->stream));
     TR_CUDA(c, cudaStreamSynchronize(c->stream));       // (tri_index is pageable host memory)
     R.topo_ready = true;
@@ -287,7 +275,7 @@ int refit_run(trace_ctx* c, int64_t n_tris, const float* v, const float* nrm, bo
     if (check_args(c, n_tris, v, n_spheres, sb)) return 1;
     if (c->scene.n_nodes == 0) return 0;                   // an empty scene: no triangle, no box
     auto& R = c->refit;
-    Phases ph;
+    PhaseTimer ph;
     ph.on = getenv("TRACE_BVH_PROFILE") != nullptr;
     const auto t0 = std::chrono::steady_clock::now();
     if (ctx_drain(c)) return 1;
@@ -356,19 +344,29 @@ int refit_run(trace_ctx* c, int64_t n_tris, const float* v, const float* nrm, bo
     }
     if (ph.on) {
         cudaEventSynchronize(ph.ev[ph.n - 1]);
-        const double wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-        fprintf(stderr, "scene refit: %lld triangles, %lld nodes, %s input, wall %.3f ms;", (long long)n_tris,
-                (long long)n_nodes, host_input ? "host" : "device", wall);
-        for (int i = 1; i < ph.n; ++i) {
-            float ms = 0.0f;
-            cudaEventElapsedTime(&ms, ph.ev[i - 1], ph.ev[i]);
-            fprintf(stderr, " %s %.3f ms%s", ph.name[i], ms, i + 1 < ph.n ? "," : "\n");
-        }
+        char head[160];
+        snprintf(head, sizeof(head), "scene refit: %lld triangles, %lld nodes, %s input", (long long)n_tris, (long long)n_nodes,
+                 host_input ? "host" : "device");
+        ph.print(head, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
     }
     return 0;
 }
 
 }  // namespace
+
+size_t pair_scan_bytes(int64_t n, cudaStream_t s) {
+    size_t bytes = 0;
+    if (cub::DeviceScan::ExclusiveSum(nullptr, bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)n, s) != cudaSuccess)
+        return 0;
+    return bytes ? bytes : 1;
+}
+
+cudaError_t pair_numbering(cudaStream_t s, const float4* nodes, int64_t n, uint32_t* flag, uint32_t* pair_of, void* tmp,
+                           size_t tmp_bytes) {
+    refit_is_interior<<<blocks_for(n, 256), 256, 0, s>>>(nodes, n, flag);
+    const cudaError_t e = cudaGetLastError();
+    return e != cudaSuccess ? e : cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, flag, pair_of, (int)n, s);
+}
 
 int ctx_drain(trace_ctx* c) {
     TR_CUDA(c, cudaStreamSynchronize(c->stream));

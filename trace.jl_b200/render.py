@@ -11,6 +11,7 @@ import numpy as np
 
 from . import _lib
 from .geometry import Bounds2, Point2f, Transformation, _v3, f32, perspective, scale, translate
+from .scene import DeviceMeshScene
 
 
 class LanczosSincFilter:
@@ -171,6 +172,7 @@ class Context:
         if rc != 0:
             raise RuntimeError(f"trace_create failed ({rc}): no usable CUDA device; there is no CPU fallback")
         self._scene = None
+        self._n_nodes = 0
 
     def check(self, rc):
         if rc != 0:
@@ -197,6 +199,10 @@ class Context:
         return {"rank": r.value, "world": w.value, "nccl_version": v.value}
 
     def upload(self, scene):
+        if isinstance(scene, DeviceMeshScene):
+            if self._scene is not scene:
+                self._upload_mesh(scene)
+            return scene
         flat = scene.flatten()
         if self._scene is not flat:
             if flat.stale:
@@ -205,8 +211,17 @@ class Context:
                                    "BVHAccel for the moved geometry")
             d = flat.desc()
             self.check(self.lib.trace_scene_upload(self.h, C.byref(d)))
-            self._scene = flat
+            self._scene, self._n_nodes = flat, len(flat.nodes)
         return flat
+
+    def _upload_mesh(self, scene):
+        """trace_scene_upload_mesh_device: tree and scene buffers built on the GPU from the scene's device arrays"""
+        d, keep = scene.desc(self.device)
+        import torch
+        torch.cuda.current_stream(self.device).synchronize()       # the work that wrote the arrays is done
+        n_nodes = C.c_int64()
+        self.check(self.lib.trace_scene_upload_mesh_device(self.h, C.byref(d), C.byref(n_nodes)))
+        self._scene, self._n_nodes = scene, n_nodes.value
 
     def refit(self, scene, vertices=None, normals=None):
         """Move the triangles of the scene uploaded to this context and refit its tree on the GPU (trace_scene_refit):
@@ -216,15 +231,26 @@ class Context:
           numpy array            through host memory;
           float32 CUDA tensor    (contiguous, on this context's device) read in place on the GPU: no host traffic.
         `normals` (same layout and kind as `vertices`, or None to keep the current ones) apply to triangles uploaded
-        with normals.  Afterwards the host FlatScene's nodes are stale: it cannot be uploaded to another context."""
-        flat = scene.flatten() if scene._flat is not None else None
-        if flat is None or flat is not self._scene:
-            raise ValueError("refit: this scene is not the one uploaded to this context")
-        n = len(flat.tri_vertices)
-        sb = np.ascontiguousarray(flat.sphere_bounds, dtype=np.float32)
+        with normals.  Afterwards the host FlatScene's nodes are stale: it cannot be uploaded to another context.
+        A DeviceMeshScene: `vertices` in its triangle order; None re-reads the scene's own tensors (vertices, and
+        normals if it has them) after the caller changed them in place."""
+        if isinstance(scene, DeviceMeshScene):
+            if scene is not self._scene:
+                raise ValueError("refit: this scene is not the one uploaded to this context")
+            flat, n, sb = None, scene.n_tris, np.zeros((0, 6), np.float32)
+            if vertices is None:
+                vertices = scene.vertices
+            if normals is None and hasattr(vertices, "is_cuda"):
+                normals = scene.normals
+        else:
+            flat = scene.flatten() if scene._flat is not None else None
+            if flat is None or flat is not self._scene:
+                raise ValueError("refit: this scene is not the one uploaded to this context")
+            n = len(flat.tri_vertices)
+            sb = np.ascontiguousarray(flat.sphere_bounds, dtype=np.float32)
+            if vertices is None:
+                vertices = flat.gather_vertices()
         sb_ptr = _lib.ptr(sb) if len(sb) else None
-        if vertices is None:
-            vertices = flat.gather_vertices()
         if hasattr(vertices, "is_cuda"):                      # a torch tensor
             def dev_ptr(t, what):
                 if t is None:
@@ -248,13 +274,14 @@ class Context:
                 return a
             v, nn = host(vertices, "vertices"), host(normals, "normals")
             self.check(self.lib.trace_scene_refit(self.h, n, _lib.ptr(v), _lib.ptr(nn), len(sb), sb_ptr))
-        flat.stale = True
+        if flat is not None:
+            flat.stale = True
 
     def scene_nodes(self):
         """The uploaded scene's nodes as the device holds them now (trace_scene_copy_nodes), node_dtype."""
         if self._scene is None:
             raise ValueError("no scene uploaded")
-        nodes = np.zeros(len(self._scene.nodes), dtype=_lib.node_dtype)
+        nodes = np.zeros(self._n_nodes, dtype=_lib.node_dtype)
         self.check(self.lib.trace_scene_copy_nodes(self.h, _lib.ptr(nodes)))
         return nodes
 

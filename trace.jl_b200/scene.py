@@ -464,6 +464,121 @@ class Scene:
         return self._flat
 
 
+def _is_tensor(a):
+    return hasattr(a, "is_cuda") and hasattr(a, "data_ptr")
+
+
+class DeviceMeshScene:
+    """A triangle-only scene whose per-triangle arrays live on the GPU (extension: the reference has no counterpart).
+    Context.upload builds its tree (the LBVH of BVHAccel(..., builder="lbvh")) and writes every scene buffer on the
+    device (trace_scene_upload_mesh_device): nothing proportional to the triangle count crosses to the host, so
+    geometry made on the GPU (simulation output, procedural meshes, a change of topology) is rebuilt without a round
+    trip through host memory.  The scene is the one BVHAccel(builder="lbvh") + Scene would give for the same triangles,
+    with the triangle index as the primitive index queries report.
+
+      vertices      [n, 3, 3] float32 world space
+      materials     list of Material; material_ids [n] integers indexing it (None: all 0)
+      normals       [n, 3, 3] float32 or None; applied to the triangles whose flags have TRI_HAS_NORMALS
+      flags         [n] uint8 TRI_FLIP | TRI_HAS_NORMALS, or None (all 0)
+
+    Arrays are contiguous CUDA tensors on one device (read in place; the context's device at upload) or numpy arrays,
+    which are moved to `device` (default: the tensors' device, else cuda:0) through torch.  Context.upload caches by
+    identity: a new DeviceMeshScene triggers a new build; to move the same triangles use Context.refit."""
+
+    def __init__(self, lights, vertices, materials, material_ids=None, normals=None, flags=None, max_node_primitives=1,
+                 device=None):
+        self.lights = list(lights)
+        self.materials = list(materials)
+        for m in self.materials:
+            if not isinstance(m, Material):
+                raise ValueError(f"materials must be Material objects, got {type(m).__name__}")
+        self.max_node_primitives = int(max_node_primitives)
+        self.has_unshaded = False             # every triangle indexes a material
+        n = self._check(vertices, "vertices", None, (3, 3), ("float32",))
+        self.n_tris = n
+        self._check(normals, "normals", n, (3, 3), ("float32",))
+        self._check(flags, "flags", n, (), ("uint8",))
+        self._check(material_ids, "material_ids", n, (), ("int8", "int16", "int32", "int64", "uint8", "uint16", "uint32"),
+                    tensor_dtypes=("int32", "int64"))
+        k = len(self.materials)
+        if n > 0 and k == 0:
+            raise ValueError("a scene with triangles needs at least one material")
+        if isinstance(material_ids, np.ndarray) and n > 0:
+            lo, hi = int(material_ids.min()), int(material_ids.max())
+            if lo < 0 or hi >= k:
+                raise ValueError(f"material_ids must be in [0, {k}), got values in [{lo}, {hi}]")
+        given = [a for a in (vertices, normals, flags, material_ids) if _is_tensor(a)]
+        devs = {a.device.index for a in given}
+        if len(devs) > 1:
+            raise ValueError(f"the CUDA tensors are on different devices {sorted(devs)}")
+        if device is not None and devs and int(device) not in devs:
+            raise ValueError(f"the CUDA tensors are on device {devs.pop()}, not device {int(device)}")
+        self.device = int(device) if device is not None else (devs.pop() if devs else 0)
+        import torch
+        dev = torch.device("cuda", self.device)
+        to_dev = lambda a: None if a is None else (a if _is_tensor(a) else torch.from_numpy(np.ascontiguousarray(a)).to(dev))
+        self.vertices, self.normals, self.flags = to_dev(vertices), to_dev(normals), to_dev(flags)
+        ids = to_dev(material_ids)
+        self.material_ids = ids if ids is None or ids.dtype == torch.int32 else ids.to(torch.int32)
+        if n == 0:
+            self.bound = Bounds3()
+        else:                                 # exact: min / max round nothing
+            v = self.vertices.view(n * 3, 3)
+            lo_hi = torch.stack([v.amin(0), v.amax(0)]).cpu().numpy()
+            self.bound = Bounds3(lo_hi[0], lo_hi[1])
+
+    @staticmethod
+    def _check(a, what, n, tail, dtypes, tensor_dtypes=None):
+        """-> the row count; ValueError on a wrong kind, shape, dtype, layout"""
+        if a is None:
+            if what == "vertices":
+                raise ValueError("vertices are required")
+            return n
+        if _is_tensor(a):
+            if not a.is_cuda:
+                raise ValueError(f"{what}: a CPU tensor; pass a CUDA tensor or a numpy array")
+            dt = str(a.dtype).replace("torch.", "")
+            if dt not in (tensor_dtypes or dtypes):
+                raise ValueError(f"{what} must have dtype {' / '.join(tensor_dtypes or dtypes)}, got {dt}")
+            if not a.is_contiguous():
+                raise ValueError(f"{what} must be contiguous")
+            shape = tuple(a.shape)
+        elif isinstance(a, np.ndarray):
+            if a.dtype.name not in dtypes:
+                raise ValueError(f"{what} must have dtype {' / '.join(dtypes) if len(dtypes) < 3 else 'integer'}, got {a.dtype.name}")
+            shape = a.shape
+        else:
+            raise ValueError(f"{what} must be a numpy array or a CUDA tensor, got {type(a).__name__}")
+        rows = shape[0] if len(shape) >= 1 else -1
+        if len(shape) != 1 + len(tail) or tuple(shape[1:]) != tuple(tail) or (n is not None and rows != n):
+            want = ("n" if n is None else str(n),) + tuple(str(t) for t in tail)
+            raise ValueError(f"{what} must have shape ({', '.join(want)}{',' if not tail else ''}), got {tuple(shape)}")
+        if rows >= 1 << 30:
+            raise ValueError(f"{what}: at most 2^30 - 1 triangles")
+        return rows
+
+    def desc(self, device):
+        """-> (MeshDeviceDesc, the host arrays it points into) for an upload to a context on `device`"""
+        if int(device) != self.device:
+            raise ValueError(f"the scene's arrays are on device {self.device}, the context is on device {int(device)}")
+        mats = np.zeros(max(1, len(self.materials)), dtype=_lib.material_dtype)
+        for i, m in enumerate(self.materials):
+            mats[i] = m.pod()
+        lights = np.zeros(len(self.lights), dtype=_lib.light_dtype)
+        for i, l in enumerate(self.lights):
+            k, m, im, I, pos, ct, cf = l.pod()
+            lights[i] = (k, m.reshape(-1), im.reshape(-1), I, pos, ct, cf)
+        ptr = lambda t: None if t is None else t.data_ptr()
+        d = _lib.MeshDeviceDesc()
+        d.n_tris = self.n_tris
+        d.tri_vertices, d.tri_normals = ptr(self.vertices), ptr(self.normals)
+        d.tri_flags, d.tri_materials = ptr(self.flags), ptr(self.material_ids)
+        d.max_node_primitives = self.max_node_primitives
+        d.n_materials, d.materials = len(self.materials), _lib.ptr(mats)
+        d.n_lights, d.lights = len(lights), _lib.ptr(lights)
+        return d, (mats, lights)
+
+
 class FlatScene:
     """The POD upload (trace_scene_desc): BVH nodes with nested BVHAccel primitives spliced in place, the BVH-ordered
     primitive list, triangle / sphere arrays, materials and lights."""
