@@ -206,11 +206,12 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
     if (d->n_prims >= (1ll << 30)) return c->fail("scene: too many primitives");
     // --- validate + pack on the host
     std::vector<float4> nodes((size_t)d->n_nodes * 2);
+    int64_t n_pairs = 0;                                   // pair records (traverse.cuh): one per interior node
     for (int64_t i = 0; i < d->n_nodes; ++i) {
         const trace_bvh_node& n = d->nodes[i];
-        const uint32_t kind = n.meta >> 30;
-        if (kind == 3) { if ((int64_t)n.offset + (int64_t)(n.meta & 0x3FFFFFFFu) > d->n_prims) return c->fail("scene: leaf %lld out of range", (long long)i); }
+        if (tr_node_leaf(n.meta)) { if ((int64_t)n.offset + (int64_t)(n.meta & ~TRACE_NODE_LEAF) > d->n_prims) return c->fail("scene: leaf %lld out of range", (long long)i); }
         else if ((int64_t)n.offset >= d->n_nodes || i + 1 >= d->n_nodes) return c->fail("scene: interior node %lld out of range", (long long)i);
+        else ++n_pairs;
         float4 a, b;
         a.x = n.bmin[0]; a.y = n.bmin[1]; a.z = n.bmin[2]; a.w = n.bmax[0];
         b.x = n.bmax[1]; b.y = n.bmax[2];
@@ -224,13 +225,13 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
         for (int64_t i = d->n_nodes - 1; i >= 0; --i) {
             const trace_bvh_node& n = d->nodes[i];
             uint8_t f = 0;
-            if ((n.meta >> 30) == 3) {
-                const uint32_t cnt = n.meta & 0x3FFFFFFFu;
-                if (cnt >= 0x20000000u) return c->fail("scene: leaf %lld holds too many primitives", (long long)i);
+            if (tr_node_leaf(n.meta)) {
+                const uint32_t cnt = n.meta & ~TRACE_NODE_LEAF;
+                if (cnt > TR_NODE_COUNT_MASK) return c->fail("scene: leaf %lld holds too many primitives", (long long)i);
                 for (uint32_t k = 0; k < cnt; ++k) if (d->prims[n.offset + k].kind == TRACE_PRIM_SPHERE) f = 1;
             } else f = below[i + 1] | below[n.offset];
             below[i] = f;
-            if (f) { uint32_t m; memcpy(&m, &nodes[2 * i + 1].w, 4); m |= 0x20000000u; memcpy(&nodes[2 * i + 1].w, &m, 4); }
+            if (f) { uint32_t m; memcpy(&m, &nodes[2 * i + 1].w, 4); m |= TR_NODE_SPHERE_BELOW; memcpy(&nodes[2 * i + 1].w, &m, 4); }
         }
     }
     std::vector<float4> prims((size_t)d->n_prims * 3), tnorm((size_t)d->n_prims * 3);
@@ -243,10 +244,7 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
             if ((int64_t)p.index >= d->n_tris || !d->tri_vertices) return c->fail("scene: triangle index out of range");
             const float* v = d->tri_vertices + 9 * (size_t)p.index;
             A.x = v[0]; A.y = v[1]; A.z = v[2]; B.x = v[3]; B.y = v[4]; B.z = v[5]; C.x = v[6]; C.y = v[7]; C.z = v[8];
-            // is_degenerate (triangle_mesh.jl:65-68) depends on the vertices only: decided once, here
-            const float3 p0 = f3(v[0], v[1], v[2]), p1 = f3(v[3], v[4], v[5]), p2 = f3(v[6], v[7], v[8]);
-            const float3 g = cross3(p2 - p0, p1 - p0);
-            if (dot3(g, g) == 0.0f) tag = TR_PRIM_DEGENERATE_BIT;
+            if (tri_degenerate(f3(v[0], v[1], v[2]), f3(v[3], v[4], v[5]), f3(v[6], v[7], v[8]))) tag = TR_PRIM_DEGENERATE_BIT;
             tri_index[i] = p.index;
             flags = d->tri_flags ? d->tri_flags[p.index] : 0;
             if (!d->tri_normals) flags &= ~(uint32_t)TRACE_TRI_HAS_NORMALS;
@@ -264,48 +262,7 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
         prims[3 * i] = A; prims[3 * i + 1] = B; prims[3 * i + 2] = C;
         tnorm[3 * i] = N0; tnorm[3 * i + 1] = N1; tnorm[3 * i + 2] = N2;
     }
-    // pair nodes (traverse.cuh): one 64-byte record per INTERIOR node holding both children's boxes and references.
-    // Preorder numbering: interior node i gets pair index = number of interior nodes before it.
-    std::vector<float4> pairs;
-    uint32_t root_ref = 0;
-    uint32_t n_pairs = 0;
-    {
-        std::vector<uint32_t> pair_of((size_t)d->n_nodes, 0);
-        for (int64_t i = 0; i < d->n_nodes; ++i) if ((d->nodes[i].meta >> 30) != 3) pair_of[i] = n_pairs++;
-        if (n_pairs >= 0x40000000u) return c->fail("scene: too many interior nodes");
-        pairs.resize((size_t)n_pairs * 4);
-        const float qnan = std::nanf("");
-        auto child_ref = [&](int64_t k) -> uint32_t {
-            const trace_bvh_node& n = d->nodes[k];
-            uint32_t m; memcpy(&m, &nodes[2 * k + 1].w, 4);
-            const uint32_t below = (m & 0x20000000u) ? 0x40000000u : 0u;
-            if ((n.meta >> 30) == 3) return 0x80000000u | below | n.offset;
-            return below | pair_of[k];
-        };
-        for (int64_t i = 0; i < d->n_nodes; ++i) {
-            const trace_bvh_node& n = d->nodes[i];
-            if ((n.meta >> 30) == 3) {
-                // mark the last primitive of the leaf (a zero-primitive leaf owns none and is never entered: its box is
-                // invalid and fails every slab test in the reference, Q16/Q17 - enforced below with a NaN box)
-                const uint32_t cnt = n.meta & 0x3FFFFFFFu;
-                if (cnt) { uint32_t t; memcpy(&t, &prims[3 * (size_t)(n.offset + cnt - 1)].w, 4); t |= 0x20000000u; memcpy(&prims[3 * (size_t)(n.offset + cnt - 1)].w, &t, 4); }
-                continue;
-            }
-            const int64_t kids[2] = {i + 1, (int64_t)n.offset};
-            float4* q = &pairs[(size_t)pair_of[i] * 4];
-            for (int k = 0; k < 2; ++k) {
-                const trace_bvh_node& ch = d->nodes[kids[k]];
-                float4 a = nodes[2 * kids[k]], b = nodes[2 * kids[k] + 1];
-                if ((ch.meta >> 30) == 3 && (ch.meta & 0x3FFFFFFFu) == 0u) { a.x = a.y = a.z = a.w = qnan; b.x = b.y = qnan; }
-                const uint32_t ref = child_ref(kids[k]);
-                const uint32_t extra = k == 0 ? (1u << (n.meta >> 30)) : 0u;  // split axis of THIS node as a bit (1 << axis), in the first half
-                memcpy(&b.z, &ref, 4); memcpy(&b.w, &extra, 4);
-                q[2 * k] = a; q[2 * k + 1] = b;
-            }
-        }
-        if (d->n_nodes > 0) root_ref = child_ref(0) & ~0x40000000u;
-        if (d->n_nodes > 0 && (d->nodes[0].meta >> 30) == 3 && (d->nodes[0].meta & 0x3FFFFFFFu) == 0u) root_ref = 0x80000000u;   // (cannot be hit: see below)
-    }
+    if (n_pairs > TR_REF_INDEX_MASK) return c->fail("scene: too many interior nodes");
     std::vector<DeviceSphere> spheres((size_t)d->n_spheres);
     for (int64_t i = 0; i < d->n_spheres; ++i) {
         static_assert(sizeof(DeviceSphere) == sizeof(trace_sphere), "sphere layout");
@@ -314,24 +271,27 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
     std::vector<DeviceMaterial> mats;
     std::vector<DeviceLight> lights;
     if (ctx_pack_materials(c, d->n_materials, d->materials, mats) || ctx_pack_lights(c, d->n_lights, d->lights, lights)) return 1;
-    // --- upload
+    const size_t scan_bytes = d->n_nodes > 0 ? pair_scan_bytes(d->n_nodes, c->stream) : 1;
+    if (!scan_bytes) return c->fail("scene: cannot size the pair scan");
+    // --- upload; then the pair records and last-of-leaf bits, on the device (upload_device.cu)
     TR_CUDA(c, cudaStreamSynchronize(c->stream));
     if (ctx_put(c, c->b_nodes, nodes.data(), nodes.size() * sizeof(float4)) ||
-        ctx_put(c, c->b_pairs, pairs.data(), pairs.size() * sizeof(float4)) ||
         ctx_put(c, c->b_prims, prims.data(), prims.size() * sizeof(float4)) ||
         ctx_put(c, c->b_tnorm, tnorm.data(), tnorm.size() * sizeof(float4)) ||
         ctx_put(c, c->b_spheres, spheres.data(), spheres.size() * sizeof(DeviceSphere)) ||
         ctx_put(c, c->b_materials, mats.data(), mats.size() * sizeof(DeviceMaterial)) ||
         ctx_put(c, c->b_lights, lights.data(), lights.size() * sizeof(DeviceLight)))
         return 1;
+    TR_CUDA(c, c->b_pairs.ensure(n_pairs ? (size_t)n_pairs * 4 * sizeof(float4) : 16));
+    if (d->n_nodes > 0) {
+        TR_CUDA(c, c->b_build.ensure(pair_scratch_bytes(d->n_nodes, scan_bytes)));
+        if (ctx_pack_pairs(c, d->n_nodes, c->b_build.as<char>(), scan_bytes)) return 1;
+    }
     TR_CUDA(c, cudaStreamSynchronize(c->stream));      // host staging vectors die at return
-    float root_box[6] = {};
-    if (d->n_nodes > 0)
-        for (int k = 0; k < 3; ++k) { root_box[k] = d->nodes[0].bmin[k]; root_box[3 + k] = d->nodes[0].bmax[k]; }
     c->refit.tri_index.swap(tri_index);
     c->refit.slot_tri_on_device = false;
     return ctx_commit_scene(c, d->n_nodes, d->n_prims, d->n_spheres, d->n_materials, d->n_lights, d->n_tris, n_pairs,
-                            root_ref, root_box, nullptr);
+                            nodes.data(), nullptr);
 }
 
 int ctx_pack_materials(trace_ctx* c, int64_t n, const trace_material* in, std::vector<DeviceMaterial>& out) {
@@ -388,20 +348,30 @@ int ctx_put(trace_ctx* c, DevBuf& b, const void* src, size_t bytes) {
     return 0;
 }
 
-// The tail of every upload, once the scene buffers hold the new scene: the DeviceScene, scene_scale from the root box
-// (min xyz, max xyz), the shadow tree, the refit state and the end of any SPPM session.  The caller sets the refit's
-// slot -> triangle map.
+// The walks' root reference (DeviceScene::root_ref) from the root node record: pair 0, or a single leaf by its first
+// primitive (a zero-primitive leaf by 0: it is never entered)
+static uint32_t root_ref_of(const float4* root) {
+    uint32_t offset, meta;
+    memcpy(&offset, &root[1].z, 4); memcpy(&meta, &root[1].w, 4);
+    if (!tr_node_leaf(meta)) return 0u;
+    return TR_REF_LEAF | (tr_node_count(meta) ? offset : 0u);
+}
+
+// The tail of every upload, once the scene buffers hold the new scene: the DeviceScene, root_ref and scene_scale from
+// the root node record, the shadow tree, the refit state and the end of any SPPM session.  The caller sets the
+// refit's slot -> triangle map.
 int ctx_commit_scene(trace_ctx* c, int64_t n_nodes, int64_t n_prims, int64_t n_spheres, int64_t n_materials,
-                     int64_t n_lights, int64_t n_tris, int64_t n_pairs, uint32_t root_ref, const float* root_box,
-                     void* shadow_scratch) {
+                     int64_t n_lights, int64_t n_tris, int64_t n_pairs, const float4* root, void* shadow_scratch) {
     DeviceScene& s = c->scene;
-    s.nodes = c->b_nodes.as<float4>(); s.pairs = c->b_pairs.as<float4>(); s.root_ref = root_ref; s.prims = c->b_prims.as<float4>(); s.tnorm = c->b_tnorm.as<float4>();
+    s.nodes = c->b_nodes.as<float4>(); s.pairs = c->b_pairs.as<float4>(); s.prims = c->b_prims.as<float4>(); s.tnorm = c->b_tnorm.as<float4>();
     s.spheres = c->b_spheres.as<DeviceSphere>(); s.materials = c->b_materials.as<DeviceMaterial>();
     s.lights = c->b_lights.as<DeviceLight>();
     s.n_nodes = (int)n_nodes; s.n_prims = (int)n_prims; s.n_spheres = (int)n_spheres;
     s.n_materials = (int)n_materials; s.n_lights = (int)n_lights;
+    s.root_ref = n_nodes > 0 ? root_ref_of(root) : 0u;
     s.scene_scale = 0.0f;
     if (n_nodes > 0) {
+        const float root_box[6] = {root[0].x, root[0].y, root[0].z, root[0].w, root[1].x, root[1].y};   // min xyz, max xyz
         for (int k = 0; k < 6; ++k) {
             const float a = fabsf(root_box[k]);
             if (std::isfinite(a)) s.scene_scale = fmaxf(s.scene_scale, a);
@@ -415,13 +385,21 @@ int ctx_commit_scene(trace_ctx* c, int64_t n_nodes, int64_t n_prims, int64_t n_s
         TR_CUDA(c, c->b_shadow.ensure((size_t)(n_prims - 1) * 4 * sizeof(float4)));
         const int rc = shadow_tree_build(c->stream, c->b_prims.p, n_prims, c->b_shadow.p, shadow_scratch);
         if (rc == 0) s.shadow_pairs = c->b_shadow.as<float4>();
-        else if (rc != 5 && rc != 6) return c->fail("scene: shadow tree build failed (CUDA error)");
+        else if (rc != LBVH_NAN_BOUND && rc != LBVH_TOO_DEEP) return c->fail("scene: shadow tree build failed (CUDA error)");
     }
     c->have_scene = true;
     c->refit.n_tris = n_tris; c->refit.n_spheres = n_spheres; c->refit.n_pairs = n_pairs;
     c->refit.topo_ready = false;
     c->refit.shadow_topo_ready = false;
     sppm_end_session(c);
+    return 0;
+}
+
+int ctx_drain(trace_ctx* c) {
+    TR_CUDA(c, cudaStreamSynchronize(c->stream));
+    for (int l = 0; l < trace_ctx::MAX_LANES; ++l) if (c->side[l]) TR_CUDA(c, cudaStreamSynchronize(c->side[l]));
+    cudaStream_t more[] = {c->chain_stream, c->coll_stream, c->copy_stream};
+    for (cudaStream_t s : more) if (s) TR_CUDA(c, cudaStreamSynchronize(s));
     return 0;
 }
 

@@ -20,7 +20,8 @@
 
 #include <cub/device/device_radix_sort.cuh>
 
-#include "../../include/trace_cuda.h"
+#include "context.hpp"
+#include "traverse.cuh"
 
 // bvh_build.cpp: an uninitialised host handle with room for the given arrays (nullptr when out of memory)
 trace_bvh* bvh_alloc(int64_t n_nodes, int64_t n_prims, trace_bvh_node** nodes, uint32_t** order);
@@ -44,10 +45,6 @@ __device__ __forceinline__ uint32_t ord_key(float f) {
 __device__ __forceinline__ float ord_float(uint32_t k) {
     return __uint_as_float((k & 0x80000000u) ? (k & 0x7FFFFFFFu) : ~k);
 }
-// Julia's min / max without NaN: exact, and -0.0 < +0.0
-__device__ __forceinline__ float jl_min(float a, float b) { return (b < a || (b == a && signbit(b))) ? b : a; }
-__device__ __forceinline__ float jl_max(float a, float b) { return (b > a || (b == a && !signbit(b))) ? b : a; }
-
 __device__ __forceinline__ float centroid(const float* pb, int64_t i, int k) {
     return __fadd_rn(__fmul_rn(0.5f, pb[6 * i + k]), __fmul_rn(0.5f, pb[6 * i + 3 + k]));
 }
@@ -212,8 +209,6 @@ __global__ void lbvh_emit(int64_t n, int m, const uint32_t* __restrict__ child, 
     out[pre] = nd;
 }
 
-inline unsigned blocks_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
-
 // The build's device buffers, carved out of one allocation: carve() with base == 0 sizes it, then again on the real one.
 // `pb` (the primitive bounds) and the node array are carved only when asked for.
 struct Buffers {
@@ -222,16 +217,12 @@ struct Buffers {
     uint32_t *child, *first, *count; int32_t* parent; uint8_t* axis;           // hierarchy (parent: every node)
     uint32_t* arrive; float* box; uint32_t *size, *depth;                      // bottom-up, every node
     trace_bvh_node* nodes = nullptr; void* sort_tmp;
-    size_t used = 0;
+    Carve k;
     char* base = nullptr;
-    template <class T> T* take(int64_t count) {
-        const size_t off = (used + 255) & ~(size_t)255;
-        used = off + (size_t)count * sizeof(T);
-        return reinterpret_cast<T*>(base + off);
-    }
+    template <class T> T* take(int64_t count) { return reinterpret_cast<T*>(base + k.take((size_t)count * sizeof(T))); }
     void carve(int64_t n, size_t sort_bytes, bool with_pb, bool with_nodes) {
         const int64_t nn = 2 * n - 1;
-        used = 0;
+        k = Carve();
         if (with_pb) pb = take<float>(6 * n);
         st = take<Status>(1);
         keys = take<uint64_t>(n); keys_sorted = take<uint64_t>(n); ids = take<uint32_t>(n); ids_sorted = take<uint32_t>(n);
@@ -244,7 +235,7 @@ struct Buffers {
     // one allocation for everything; freed by the destructor
     int alloc(int64_t n, size_t sort_bytes, bool with_pb, bool with_nodes) {
         carve(n, sort_bytes, with_pb, with_nodes);
-        if (cudaMalloc(&base, used) != cudaSuccess) { cudaGetLastError(); base = nullptr; return 7; }
+        if (cudaMalloc(&base, k.used) != cudaSuccess) { cudaGetLastError(); base = nullptr; return LBVH_CUDA; }
         owned = true;
         carve(n, sort_bytes, with_pb, with_nodes);
         return 0;
@@ -258,13 +249,6 @@ struct Buffers {
     ~Buffers() { if (owned) cudaFree(base); }
 };
 
-struct Phases {
-    bool on = false;
-    cudaEvent_t ev[8] = {};
-    int n = 0;
-    void mark(cudaStream_t s) { if (on && n < 8) cudaEventRecord(ev[n++], s); }
-};
-
 size_t sort_bytes_for(int64_t n, cudaStream_t s) {
     size_t bytes = 0;
     if (cub::DeviceRadixSort::SortPairs(nullptr, bytes, (const uint64_t*)nullptr, (uint64_t*)nullptr, (const uint32_t*)nullptr,
@@ -274,8 +258,7 @@ size_t sort_bytes_for(int64_t n, cudaStream_t s) {
 }
 
 // The device-resident core: bounds b.pb (device, [n][6]) -> keys, sorted order, hierarchy, boxes, subtree sizes and
-// depths in `b`, and the status on the host.  Returns 0, 5 (a NaN bound), 6 (deeper than the 64-entry traversal
-// stack) or 7 (CUDA error).
+// depths in `b`, and the status on the host.  Returns LBVH_OK, _NAN_BOUND, _TOO_DEEP or _CUDA.
 void core_reset(cudaStream_t s, int64_t n, Buffers& b) {
     cudaMemsetAsync(b.st, 0xFF, sizeof(b.st->cmin), s);
     cudaMemsetAsync(&b.st->cmax, 0, sizeof(Status) - sizeof(b.st->cmin), s);
@@ -284,50 +267,50 @@ void core_reset(cudaStream_t s, int64_t n, Buffers& b) {
 }
 
 // build_core without the reset: what runs after core_reset (and anything that reports into the status block)
-int core_run(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, Status& hs, Phases& ph) {
+int core_run(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, Status& hs, PhaseTimer& ph) {
     const int T = 256;
     lbvh_centroid_box<<<(unsigned)std::min<int64_t>(blocks_for(n, T), 4096), T, 0, s>>>(b.pb, n, b.st);
     lbvh_keys<<<blocks_for(n, T), T, 0, s>>>(b.pb, n, b.st, b.keys, b.ids);
-    ph.mark(s);
+    ph.mark(s, "keys");
     if (cub::DeviceRadixSort::SortPairs(b.sort_tmp, sort_bytes, b.keys, b.keys_sorted, b.ids, b.ids_sorted, (int)n, 0, 63, s)
         != cudaSuccess)
-        return 7;
-    ph.mark(s);
+        return LBVH_CUDA;
+    ph.mark(s, "sort");
     if (n > 1) lbvh_hierarchy<<<blocks_for(n - 1, T), T, 0, s>>>(b.keys_sorted, n, b.child, b.parent, b.first, b.count, b.axis);
-    ph.mark(s);
+    ph.mark(s, "hierarchy");
     lbvh_bottom_up<<<blocks_for(n, T), T, 0, s>>>(b.pb, b.ids_sorted, n, m, b.child, b.parent, b.count, b.arrive, b.box,
                                                    b.size, b.depth, b.st);
     if (cudaGetLastError() != cudaSuccess ||
         cudaMemcpyAsync(&hs, b.st, sizeof(Status), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
         cudaStreamSynchronize(s) != cudaSuccess)
-        return 7;
-    ph.mark(s);
-    if (hs.nan) return 5;
-    if (hs.root_depth > 64) return 6;                        // TR_STACK_SIZE (traverse.cuh): the walks' stacks would overflow
-    return 0;
+        return LBVH_CUDA;
+    ph.mark(s, "bottom-up");
+    if (hs.nan) return LBVH_NAN_BOUND;
+    if (hs.root_depth > TR_STACK_SIZE) return LBVH_TOO_DEEP;   // the walks' stacks would overflow
+    return LBVH_OK;
 }
 
-int build_core(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, Status& hs, Phases& ph) {
+int build_core(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, Status& hs, PhaseTimer& ph) {
     core_reset(s, n, b);
     return core_run(s, n, m, b, sort_bytes, hs, ph);
 }
 
-int build(cudaStream_t s, const float* hb, int64_t n, int m, trace_bvh** out, Phases& ph) {
+int build(cudaStream_t s, const float* hb, int64_t n, int m, trace_bvh** out, PhaseTimer& ph) {
     const int64_t nn = 2 * n - 1;
     const size_t sort_bytes = sort_bytes_for(n, s);
-    if (!sort_bytes) return 7;
+    if (!sort_bytes) return LBVH_CUDA;
     Buffers b;
-    if (b.alloc(n, sort_bytes, true, true)) return 7;
+    if (b.alloc(n, sort_bytes, true, true)) return LBVH_CUDA;
     const int T = 256;
-    ph.mark(s);
-    if (cudaMemcpyAsync(b.pb, hb, (size_t)n * 6 * sizeof(float), cudaMemcpyHostToDevice, s) != cudaSuccess) return 7;
-    ph.mark(s);
+    ph.mark(s, nullptr);
+    if (cudaMemcpyAsync(b.pb, hb, (size_t)n * 6 * sizeof(float), cudaMemcpyHostToDevice, s) != cudaSuccess) return LBVH_CUDA;
+    ph.mark(s, "upload");
     Status hs;
     if (const int rc = build_core(s, n, m, b, sort_bytes, hs, ph)) return rc;
     const int64_t n_nodes = hs.root_size;
     lbvh_emit<<<blocks_for(nn, T), T, 0, s>>>(n, m, b.child, b.parent, b.first, b.count, b.axis, b.box, b.size, b.nodes);
-    if (cudaGetLastError() != cudaSuccess) return 7;
-    ph.mark(s);
+    if (cudaGetLastError() != cudaSuccess) return LBVH_CUDA;
+    ph.mark(s, "emit");
     trace_bvh_node* hn = nullptr;
     uint32_t* ho = nullptr;
     trace_bvh* bvh = bvh_alloc(n_nodes, n, &hn, &ho);
@@ -335,12 +318,12 @@ int build(cudaStream_t s, const float* hb, int64_t n, int m, trace_bvh** out, Ph
     if (cudaMemcpyAsync(hn, b.nodes, (size_t)n_nodes * sizeof(trace_bvh_node), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
         cudaMemcpyAsync(ho, b.ids_sorted, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToHost, s) != cudaSuccess) {
         trace_bvh_free(bvh);
-        return 7;
+        return LBVH_CUDA;
     }
-    ph.mark(s);
-    if (cudaStreamSynchronize(s) != cudaSuccess) { trace_bvh_free(bvh); return 7; }
+    ph.mark(s, "download");
+    if (cudaStreamSynchronize(s) != cudaSuccess) { trace_bvh_free(bvh); return LBVH_CUDA; }
     *out = bvh;
-    return 0;
+    return LBVH_OK;
 }
 
 // ------------------------------------------------------------------ the shadow tree (traverse.cuh, traverse_shadow)
@@ -350,10 +333,8 @@ __global__ void lbvh_prim_bounds(const float4* __restrict__ prims, int64_t n, fl
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= n) return;
     const float4 A = prims[3 * i], B = prims[3 * i + 1], C = prims[3 * i + 2];
-    float lo[3] = {jl_min(jl_min(jl_min(INFINITY, A.x), B.x), C.x), jl_min(jl_min(jl_min(INFINITY, A.y), B.y), C.y),
-                   jl_min(jl_min(jl_min(INFINITY, A.z), B.z), C.z)};
-    float hi[3] = {jl_max(jl_max(jl_max(-INFINITY, A.x), B.x), C.x), jl_max(jl_max(jl_max(-INFINITY, A.y), B.y), C.y),
-                   jl_max(jl_max(jl_max(-INFINITY, A.z), B.z), C.z)};
+    float lo[3] = {TR_INF, TR_INF, TR_INF}, hi[3] = {-TR_INF, -TR_INF, -TR_INF};
+    tri_box(xyz(A), xyz(B), xyz(C), lo, hi);
     const bool nan = A.x != A.x || A.y != A.y || A.z != A.z || B.x != B.x || B.y != B.y || B.z != B.z || C.x != C.x ||
                      C.y != C.y || C.z != C.z;
     for (int c = 0; c < 3; ++c) {
@@ -363,7 +344,7 @@ __global__ void lbvh_prim_bounds(const float4* __restrict__ prims, int64_t n, fl
 }
 
 // One 64-byte pair record per internal node, in Karras numbering (the root is pair 0): both children's boxes, their
-// references (a pair index, or 0x80000000 | primitive slot for a leaf: TR_REF_LEAF, traverse.cuh) and the split axis as
+// references (a pair index, or TR_REF_LEAF | primitive slot for a leaf, traverse.cuh) and the split axis as
 // a bit in the first half - the layout of the upload's pair records (api.cu).
 __global__ void lbvh_emit_pairs(int64_t n, const uint32_t* __restrict__ child, const uint32_t* __restrict__ sorted_ids,
                                 const uint8_t* __restrict__ axis, const float* __restrict__ box, float4* __restrict__ pairs) {
@@ -372,7 +353,7 @@ __global__ void lbvh_emit_pairs(int64_t n, const uint32_t* __restrict__ child, c
     for (int k = 0; k < 2; ++k) {
         const int64_t v = child[2 * i + k];
         const float* bx = box + 6 * v;
-        const uint32_t ref = v < n - 1 ? (uint32_t)v : (0x80000000u | sorted_ids[v - (n - 1)]);
+        const uint32_t ref = v < n - 1 ? (uint32_t)v : (TR_REF_LEAF | sorted_ids[v - (n - 1)]);
         const uint32_t extra = k == 0 ? (1u << axis[i]) : 0u;
         pairs[4 * i + 2 * k] = make_float4(bx[0], bx[1], bx[2], bx[3]);
         pairs[4 * i + 2 * k + 1] = make_float4(bx[4], bx[5], __uint_as_float(ref), __uint_as_float(extra));
@@ -401,9 +382,11 @@ __global__ void lbvh_tri_bounds(const float* __restrict__ v, int64_t n, float* _
     const float* p = v + 9 * i;
     bool nan = false;
     for (int k = 0; k < 9; ++k) nan |= p[k] != p[k];
+    float lo[3] = {TR_INF, TR_INF, TR_INF}, hi[3] = {-TR_INF, -TR_INF, -TR_INF};
+    tri_box(f3(p[0], p[1], p[2]), f3(p[3], p[4], p[5]), f3(p[6], p[7], p[8]), lo, hi);
     for (int c = 0; c < 3; ++c) {
-        pb[6 * i + c] = nan ? NAN : jl_min(jl_min(jl_min(INFINITY, p[c]), p[3 + c]), p[6 + c]);
-        pb[6 * i + 3 + c] = nan ? NAN : jl_max(jl_max(jl_max(-INFINITY, p[c]), p[3 + c]), p[6 + c]);
+        pb[6 * i + c] = nan ? NAN : lo[c];
+        pb[6 * i + 3 + c] = nan ? NAN : hi[c];
     }
 }
 
@@ -416,87 +399,72 @@ size_t lbvh_scratch_bytes(int64_t n, cudaStream_t s) {
     if (!sort_bytes) return 0;
     Buffers b;
     b.carve(n, sort_bytes, true, false);
-    return b.used;
+    return b.k.used;
 }
 
 // The shadow tree of an uploaded scene (api.cu): an LBVH with one primitive per leaf over the n >= 2 uploaded primitive
 // records `prims` (device, BVH slot order, triangles only), written as n - 1 pair records to `pairs` (device).  Nothing
 // crosses to the host but the build's status.  `scratch` (lbvh_scratch_bytes(n)) or nullptr: an allocation of its own.
-// Returns 0, 5 (a NaN vertex), 6 (deeper than 64 levels) or 7 (CUDA error).
+// Returns LBVH_OK, _NAN_BOUND (a NaN vertex), _TOO_DEEP or _CUDA.
 int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs, void* scratch) {
     if (n < 2 || n >= 0x40000000ll) return 1;
     const size_t sort_bytes = sort_bytes_for(n, s);
-    if (!sort_bytes) return 7;
+    if (!sort_bytes) return LBVH_CUDA;
     Buffers b;
     if (scratch) b.borrow(scratch, n, sort_bytes);
-    else if (b.alloc(n, sort_bytes, true, false)) return 7;
+    else if (b.alloc(n, sort_bytes, true, false)) return LBVH_CUDA;
     const int T = 256;
     lbvh_prim_bounds<<<blocks_for(n, T), T, 0, s>>>(static_cast<const float4*>(prims), n, b.pb);
-    Phases ph;
+    PhaseTimer quiet;
     Status hs;
-    if (const int rc = build_core(s, n, 1, b, sort_bytes, hs, ph)) return rc;
+    if (const int rc = build_core(s, n, 1, b, sort_bytes, hs, quiet)) return rc;
     lbvh_emit_pairs<<<blocks_for(n - 1, T), T, 0, s>>>(n, b.child, b.ids_sorted, b.axis, b.box, static_cast<float4*>(pairs));
-    if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess) return 7;
-    return 0;
+    if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess) return LBVH_CUDA;
+    return LBVH_OK;
 }
 
-// The tree of trace_scene_upload_mesh_device, in steps over `scratch` (lbvh_scratch_bytes(n), n >= 1):
-//   lbvh_mesh_validate  reset the status block, check normals (NULL: none) and material indices (NULL: all 0) into it;
-//   lbvh_mesh_bounds    the triangles' boxes (no host wait so far);
-//   lbvh_mesh_build     the LBVH core and its status read back: 0, 5 a NaN vertex, 6 deeper than 64 levels, 7 CUDA
-//                       error, 8 a NaN normal, 9 a material index out of range; *n_nodes, and *order = the sorted
-//                       triangle ids (slot -> triangle, device, inside the scratch);
-//   lbvh_mesh_emit      the preorder node records (trace_bvh_node, 32 B) into `nodes` (device).
-// Nothing is written outside the scratch before lbvh_mesh_emit, so a refused input leaves the caller's buffers intact.
-int lbvh_mesh_validate(cudaStream_t s, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n, void* scratch) {
+// The tree of trace_scene_upload_mesh_device over `scratch` (lbvh_scratch_bytes(n), n >= 1): the status block reset,
+// normals (NULL: none) and material indices (NULL: all 0) checked into it, the triangles' boxes, then the LBVH core
+// and its status read back.  Returns LBVH_OK with *n_nodes and *order = the sorted triangle ids (slot -> triangle,
+// device, inside the scratch), or the first refusal in the order vertices, normals, materials, depth.  Nothing is
+// written outside the scratch before lbvh_mesh_emit (the preorder node records into `nodes`, device), so a refused
+// input leaves the caller's buffers intact.
+int lbvh_mesh_build(cudaStream_t s, const float* v, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n,
+                    int m, void* scratch, PhaseTimer& ph, int64_t* n_nodes, const uint32_t** order) {
     const size_t sort_bytes = sort_bytes_for(n, s);
-    if (!sort_bytes) return 7;
+    if (!sort_bytes) return LBVH_CUDA;
     Buffers b;
     b.borrow(scratch, n, sort_bytes);
     core_reset(s, n, b);
     const int T = 256;
     const uint32_t nm = n_materials > 0xFFFFFFFFll ? 0xFFFFFFFFu : (uint32_t)n_materials;
     lbvh_mesh_validate<<<(unsigned)std::min<int64_t>(blocks_for(n, T), 4096), T, 0, s>>>(nrm, mat, n, nm, b.st);
-    return cudaGetLastError() == cudaSuccess ? 0 : 7;
-}
-
-int lbvh_mesh_bounds(cudaStream_t s, const float* v, int64_t n, void* scratch) {
-    const size_t sort_bytes = sort_bytes_for(n, s);
-    if (!sort_bytes) return 7;
-    Buffers b;
-    b.borrow(scratch, n, sort_bytes);
-    const int T = 256;
+    ph.mark(s, "validate");
     lbvh_tri_bounds<<<blocks_for(n, T), T, 0, s>>>(v, n, b.pb);
-    return cudaGetLastError() == cudaSuccess ? 0 : 7;
-}
-
-int lbvh_mesh_build(cudaStream_t s, int64_t n, int m, void* scratch, int64_t* n_nodes, const uint32_t** order) {
-    const size_t sort_bytes = sort_bytes_for(n, s);
-    if (!sort_bytes) return 7;
-    Buffers b;
-    b.borrow(scratch, n, sort_bytes);
-    Phases ph;
+    ph.mark(s, "bounds");
+    PhaseTimer quiet;                                      // the core's own phases are not the upload's
     Status hs;
-    const int rc = core_run(s, n, m, b, sort_bytes, hs, ph);
-    if (rc == 7) return 7;
-    if (hs.nan) return 5;                  // the order of the refusals: vertices, normals, materials, depth
-    if (hs.bad & 1u) return 8;
-    if (hs.bad & 2u) return 9;
+    const int rc = core_run(s, n, m, b, sort_bytes, hs, quiet);   // (its launch check covers the two kernels above)
+    ph.mark(s, "build");
+    if (rc == LBVH_CUDA) return rc;
+    if (hs.nan) return LBVH_NAN_BOUND;
+    if (hs.bad & 1u) return LBVH_NAN_NORMAL;
+    if (hs.bad & 2u) return LBVH_BAD_MATERIAL;
     if (rc) return rc;
     *n_nodes = hs.root_size;
     *order = b.ids_sorted;
-    return 0;
+    return LBVH_OK;
 }
 
 int lbvh_mesh_emit(cudaStream_t s, int64_t n, int m, void* scratch, void* nodes) {
     const size_t sort_bytes = sort_bytes_for(n, s);
-    if (!sort_bytes) return 7;
+    if (!sort_bytes) return LBVH_CUDA;
     Buffers b;
     b.borrow(scratch, n, sort_bytes);
     const int T = 256;
     lbvh_emit<<<blocks_for(2 * n - 1, T), T, 0, s>>>(n, m, b.child, b.parent, b.first, b.count, b.axis, b.box, b.size,
                                                     static_cast<trace_bvh_node*>(nodes));
-    return cudaGetLastError() == cudaSuccess ? 0 : 7;
+    return cudaGetLastError() == cudaSuccess ? LBVH_OK : LBVH_CUDA;
 }
 
 extern "C" int trace_bvh_build_gpu(int device, const float* pb, int64_t n, int max_node_primitives, trace_bvh** out) {
@@ -507,33 +475,26 @@ extern "C" int trace_bvh_build_gpu(int device, const float* pb, int64_t n, int m
     int n_dev = 0, prev = 0;
     if (cudaGetDeviceCount(&n_dev) != cudaSuccess || device < 0 || device >= n_dev || cudaGetDevice(&prev) != cudaSuccess) {
         cudaGetLastError();
-        return 7;                                            // no CPU fallback
+        return LBVH_CUDA;                                    // no CPU fallback
     }
     if (n == 0) {
         trace_bvh_node* hn; uint32_t* ho;
         *out = bvh_alloc(0, 0, &hn, &ho);
         return *out ? 0 : 2;
     }
-    if (cudaSetDevice(device) != cudaSuccess) { cudaGetLastError(); return 7; }
+    if (cudaSetDevice(device) != cudaSuccess) { cudaGetLastError(); return LBVH_CUDA; }
     cudaStream_t s;
-    int rc = 7;
+    int rc = LBVH_CUDA;
     if (cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking) == cudaSuccess) {
-        Phases ph;
+        PhaseTimer ph;
         ph.on = getenv("TRACE_BVH_PROFILE") != nullptr;
-        for (int i = 0; ph.on && i < 8; ++i) cudaEventCreate(&ph.ev[i]);
         const auto t0 = std::chrono::steady_clock::now();
         rc = build(s, pb, n, m, out, ph);
-        if (ph.on && rc == 0) {
-            const double wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-            static const char* names[7] = {"upload", "keys", "sort", "hierarchy", "bottom-up", "emit", "download"};
-            fprintf(stderr, "bvh build gpu: n %lld, device %d, wall %.3f ms;", (long long)n, device, wall);
-            for (int i = 0; i + 1 < ph.n; ++i) {
-                float ms = 0.0f;
-                cudaEventElapsedTime(&ms, ph.ev[i], ph.ev[i + 1]);
-                fprintf(stderr, " %s %.3f ms%s", names[i], ms, i + 2 < ph.n ? "," : "\n");
-            }
+        if (ph.on && rc == LBVH_OK) {
+            char head[96];
+            snprintf(head, sizeof(head), "bvh build gpu: n %lld, device %d", (long long)n, device);
+            ph.print(head, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count());
         }
-        for (int i = 0; ph.on && i < 8; ++i) cudaEventDestroy(ph.ev[i]);
         cudaStreamDestroy(s);
     }
     cudaGetLastError();

@@ -319,29 +319,23 @@ int whitted_render_device(trace_ctx* ctx, const trace_camera* cam, const trace_f
 void sppm_free(trace_ctx* ctx);
 void sppm_end_session(trace_ctx* ctx);
 void whitted_film_range(const trace_ctx* ctx, long long npix, long long* p0, long long* p1);
-// implemented in bvh_gpu.cu: the shadow tree over uploaded primitive records (0, 5 NaN, 6 too deep, 7 CUDA error), in
-// `scratch` (lbvh_scratch_bytes(n) bytes) or, with nullptr, an allocation of its own; the device mesh build's steps
-int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs, void* scratch);
-size_t lbvh_scratch_bytes(int64_t n, cudaStream_t s);
-int lbvh_mesh_validate(cudaStream_t s, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n, void* scratch);
-int lbvh_mesh_bounds(cudaStream_t s, const float* v, int64_t n, void* scratch);
-int lbvh_mesh_build(cudaStream_t s, int64_t n, int m, void* scratch, int64_t* n_nodes, const uint32_t** order);
-int lbvh_mesh_emit(cudaStream_t s, int64_t n, int m, void* scratch, void* nodes);
-// implemented in api.cu: the parts of a scene upload that do not depend on where the tree was built
+// implemented in api.cu: the parts of a scene upload that do not depend on where the tree was built.  `root` is the
+// uploaded root node record (2 float4; unused for an empty tree).
 int ctx_pack_materials(trace_ctx* ctx, int64_t n, const trace_material* in, std::vector<DeviceMaterial>& out);
 int ctx_pack_lights(trace_ctx* ctx, int64_t n, const trace_light* in, std::vector<DeviceLight>& out);
 int ctx_put(trace_ctx* ctx, DevBuf& b, const void* src, size_t bytes);
 int ctx_commit_scene(trace_ctx* ctx, int64_t n_nodes, int64_t n_prims, int64_t n_spheres, int64_t n_materials,
-                     int64_t n_lights, int64_t n_tris, int64_t n_pairs, uint32_t root_ref, const float* root_box,
-                     void* shadow_scratch);
-// implemented in refit.cu: waits for every stream of the context (caller's, lanes, SPPM chain / collectives, copies)
+                     int64_t n_lights, int64_t n_tris, int64_t n_pairs, const float4* root, void* shadow_scratch);
+// implemented in api.cu: waits for every stream of the context (caller's, lanes, SPPM chain / collectives, copies)
 int ctx_drain(trace_ctx* ctx);
-// implemented in refit.cu: the upload's preorder pair numbering of a device node array (2 float4 per node), pair_of[i] =
-// interior nodes before node i, as an exclusive scan of "is interior" (`flag`: n words of scratch; `tmp`:
-// pair_scan_bytes(n) bytes of scan scratch)
+// implemented in upload_device.cu, the device half of both uploads: the preorder pair numbering of a device node array
+// (2 float4 per node), pair_of[i] = interior nodes before node i, as an exclusive scan of "is interior" (`flag`: n
+// words of scratch; `tmp`: pair_scan_bytes(n) bytes of scan scratch); and the scene's pair records built with it
 size_t pair_scan_bytes(int64_t n, cudaStream_t s);
 cudaError_t pair_numbering(cudaStream_t s, const float4* nodes, int64_t n, uint32_t* flag, uint32_t* pair_of, void* tmp,
                            size_t tmp_bytes);
+size_t pair_scratch_bytes(int64_t n_nodes, size_t scan_bytes);
+int ctx_pack_pairs(trace_ctx* ctx, int64_t n_nodes, char* scratch, size_t scan_bytes);
 
 // TRACE_BVH_PROFILE=1: CUDA events between the phases of an upload / refit call, printed as one stderr line
 struct PhaseTimer {
@@ -365,3 +359,22 @@ struct PhaseTimer {
     }
     ~PhaseTimer() { for (auto e : ev) if (e) cudaEventDestroy(e); }
 };
+
+// implemented in bvh_gpu.cu.  The LBVH builds' status; trace_bvh_build_gpu returns 0, 5, 6 and 7 as its public codes.
+enum LbvhStatus {
+    LBVH_OK = 0,
+    LBVH_NAN_BOUND = 5,          // a NaN primitive bound (a NaN vertex)
+    LBVH_TOO_DEEP = 6,           // deeper than the walks' 64-entry stack (TR_STACK_SIZE)
+    LBVH_CUDA = 7,               // a CUDA error
+    LBVH_NAN_NORMAL = 8,         // mesh builds: a NaN normal
+    LBVH_BAD_MATERIAL = 9,       // mesh builds: a material index out of range
+};
+// The shadow tree over uploaded primitive records, in `scratch` (lbvh_scratch_bytes(n) bytes) or, with nullptr, an
+// allocation of its own: LBVH_OK, _NAN_BOUND, _TOO_DEEP or _CUDA.
+int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs, void* scratch);
+size_t lbvh_scratch_bytes(int64_t n, cudaStream_t s);
+// The tree of trace_scene_upload_mesh_device, in `scratch`: lbvh_mesh_build validates, bounds and builds (phases
+// "validate", "bounds" and "build" of `ph`); lbvh_mesh_emit, once the input is accepted, writes the node records.
+int lbvh_mesh_build(cudaStream_t s, const float* v, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n,
+                    int m, void* scratch, PhaseTimer& ph, int64_t* n_nodes, const uint32_t** order);
+int lbvh_mesh_emit(cudaStream_t s, int64_t n, int m, void* scratch, void* nodes);

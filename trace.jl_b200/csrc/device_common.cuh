@@ -56,6 +56,19 @@ __device__ __forceinline__ float3 xform_normal(const float* __restrict__ im, flo
               (im[2] * n.x + im[6] * n.y) + im[10] * n.z);
 }
 
+// ------------------------------------------------------------------ launch and scratch sizing (host)
+inline unsigned blocks_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
+
+// Sub-buffers of one allocation: take() returns the next one's offset, 256-byte aligned; `used` is the bytes so far
+struct Carve {
+    size_t used = 0;
+    size_t take(size_t bytes) {
+        const size_t off = (used + 255) & ~(size_t)255;
+        used = off + bytes;
+        return off;
+    }
+};
+
 // ------------------------------------------------------------------ device scene (all arrays live in HBM)
 // nodes : 2 x float4 per node  {bmin.xyz, bmax.x} {bmax.y, bmax.z, offset(bits), meta(bits)}          32 B
 // prims : 3 x float4 per BVH-ordered primitive                                                          48 B

@@ -17,33 +17,19 @@
 #include <cmath>
 #include <cstring>
 
-#include <cub/device/device_scan.cuh>
-
 #include "context.hpp"
 #include "traverse.cuh"
 
 namespace {
 
-// Julia's min / max without NaN: exact, and -0.0 < +0.0 (as bvh_gpu.cu)
-__device__ __forceinline__ float jl_min(float a, float b) { return (b < a || (b == a && signbit(b))) ? b : a; }
-__device__ __forceinline__ float jl_max(float a, float b) { return (b > a || (b == a && !signbit(b))) ? b : a; }
-
-__device__ __forceinline__ uint32_t node_meta(const float4* nodes, int64_t i) { return __float_as_uint(nodes[2 * i + 1].w); }
-
-// topology 1: 1 for an interior node (scanned into the upload's preorder pair numbering)
-__global__ void refit_is_interior(const float4* __restrict__ nodes, int64_t n, uint32_t* __restrict__ flag) {
-    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (i < n) flag[i] = (node_meta(nodes, i) >> 30) != 3u ? 1u : 0u;
-}
-
-// topology 2: parents, each node's slot in its parent's pair record, the leaf list (leaf i is number i - pair_of[i])
+// topology (after the upload's pair numbering, upload_device.cu): parents, each node's slot in its parent's pair record, the leaf list (leaf i is number i - pair_of[i])
 __global__ void refit_topology(const float4* __restrict__ nodes, int64_t n, const uint32_t* __restrict__ pair_of,
                                int32_t* __restrict__ parent, uint32_t* __restrict__ up, uint32_t* __restrict__ leaves) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= n) return;
     if (i == 0) { parent[0] = -1; up[0] = 0u; }
     const float4 b = nodes[2 * i + 1];
-    if ((__float_as_uint(b.w) >> 30) == 3u) { leaves[i - pair_of[i]] = (uint32_t)i; return; }
+    if (tr_node_leaf(__float_as_uint(b.w))) { leaves[i - pair_of[i]] = (uint32_t)i; return; }
     const uint32_t q = pair_of[i], second = __float_as_uint(b.z);
     parent[i + 1] = (int32_t)i; up[i + 1] = 2u * q;
     parent[second] = (int32_t)i; up[second] = 2u * q + 1u;
@@ -69,8 +55,7 @@ __global__ void refit_scatter(const float* __restrict__ v, const float* __restri
     const size_t t = slot_tri[s];
     const float* p = v + 9 * t;
     const float3 p0 = f3(p[0], p[1], p[2]), p1 = f3(p[3], p[4], p[5]), p2 = f3(p[6], p[7], p[8]);
-    const float3 g = cross3(p2 - p0, p1 - p0);                // is_degenerate, exactly as trace_scene_upload
-    tag = dot3(g, g) == 0.0f ? (tag | TR_PRIM_DEGENERATE_BIT) : (tag & ~TR_PRIM_DEGENERATE_BIT);
+    tag = tri_degenerate(p0, p1, p2) ? (tag | TR_PRIM_DEGENERATE_BIT) : (tag & ~TR_PRIM_DEGENERATE_BIT);
     const float mat = prims[3 * s + 1].w, orig = prims[3 * s + 2].w;
     prims[3 * s] = f4(p0, __uint_as_float(tag));
     prims[3 * s + 1] = f4(p1, mat);
@@ -111,19 +96,16 @@ __global__ void refit_climb(const float4* __restrict__ prims, const float* __res
     bool e;
     {
         const float4 b = nodes[2 * v + 1];
-        const uint32_t first = __float_as_uint(b.z), cnt = __float_as_uint(b.w) & 0x1FFFFFFFu;
+        const uint32_t first = __float_as_uint(b.z), cnt = tr_node_count(__float_as_uint(b.w));
         for (uint32_t j = 0; j < cnt; ++j) {
             const int64_t s = first + j;
             const float4 A = prims[3 * s];
             const uint32_t tag = __float_as_uint(A.w);
             if (tag & TR_PRIM_SPHERE_BIT) {
-                const float* sb = sphere_bounds + 6 * (size_t)(tag & 0x1FFFFFFFu);
+                const float* sb = sphere_bounds + 6 * (size_t)(tag & TR_PRIM_INDEX_MASK);
                 for (int c = 0; c < 3; ++c) { lo[c] = jl_min(lo[c], sb[c]); hi[c] = jl_max(hi[c], sb[3 + c]); }
             } else {
-                const float4 B = prims[3 * s + 1], C = prims[3 * s + 2];
-                lo[0] = jl_min(jl_min(jl_min(lo[0], A.x), B.x), C.x); hi[0] = jl_max(jl_max(jl_max(hi[0], A.x), B.x), C.x);
-                lo[1] = jl_min(jl_min(jl_min(lo[1], A.y), B.y), C.y); hi[1] = jl_max(jl_max(jl_max(hi[1], A.y), B.y), C.y);
-                lo[2] = jl_min(jl_min(jl_min(lo[2], A.z), B.z), C.z); hi[2] = jl_max(jl_max(jl_max(hi[2], A.z), B.z), C.z);
+                tri_box(xyz(A), xyz(prims[3 * s + 1]), xyz(prims[3 * s + 2]), lo, hi);
             }
         }
         // (+inf, -inf) is the identity of the union, so an empty subtree's registers never change a sibling's box
@@ -182,11 +164,8 @@ __global__ void shadow_climb(const float4* __restrict__ prims, int64_t n_prims, 
                              float4* pairs) {
     const int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (s >= n_prims || *status) return;
-    const float4 A = prims[3 * s], B = prims[3 * s + 1], C = prims[3 * s + 2];
-    float lo[3] = {jl_min(jl_min(jl_min(TR_INF, A.x), B.x), C.x), jl_min(jl_min(jl_min(TR_INF, A.y), B.y), C.y),
-                   jl_min(jl_min(jl_min(TR_INF, A.z), B.z), C.z)};
-    float hi[3] = {jl_max(jl_max(jl_max(-TR_INF, A.x), B.x), C.x), jl_max(jl_max(jl_max(-TR_INF, A.y), B.y), C.y),
-                   jl_max(jl_max(jl_max(-TR_INF, A.z), B.z), C.z)};
+    float lo[3] = {TR_INF, TR_INF, TR_INF}, hi[3] = {-TR_INF, -TR_INF, -TR_INF};
+    tri_box(xyz(prims[3 * s]), xyz(prims[3 * s + 1]), xyz(prims[3 * s + 2]), lo, hi);
     uint32_t u = up_prim[s];
     put_half(pairs, u, lo, hi);
     for (;;) {
@@ -204,8 +183,6 @@ __global__ void shadow_climb(const float4* __restrict__ prims, int64_t n_prims, 
     }
 }
 
-inline unsigned blocks_for(int64_t n, int threads) { return (unsigned)((n + threads - 1) / threads); }
-
 // first refit after an upload: parents, pair slots and leaves from b_nodes, the slot -> triangle map from the host (or,
 // after a device mesh upload, the one it left on the device)
 int derive_topology(trace_ctx* c) {
@@ -213,13 +190,11 @@ int derive_topology(trace_ctx* c) {
     const int64_t n = c->scene.n_nodes, n_prims = c->scene.n_prims, n_leaves = n - R.n_pairs;
     const size_t scan_bytes = pair_scan_bytes(n, c->stream);
     if (!scan_bytes) return c->fail("scene refit: cannot size the pair scan");
-    size_t used = 0;
-    auto take = [&](size_t bytes) { const size_t off = (used + 255) & ~(size_t)255; used = off + bytes; return off; };
-    const size_t o_parent = take(n * 4), o_up = take(n * 4), o_pair = take(n * 4), o_leaves = take(n_leaves * 4),
-                 o_empty = take(n), o_arrive = take(R.n_pairs * 4), o_tri = take(R.slot_tri_on_device ? 0 : n_prims * 4),
-                 o_status = take(16),
-                 o_scan = take(scan_bytes);
-    TR_CUDA(c, R.topo.ensure(used));
+    Carve k;
+    const size_t o_parent = k.take(n * 4), o_up = k.take(n * 4), o_pair = k.take(n * 4), o_leaves = k.take(n_leaves * 4),
+                 o_empty = k.take(n), o_arrive = k.take(R.n_pairs * 4), o_tri = k.take(R.slot_tri_on_device ? 0 : n_prims * 4),
+                 o_status = k.take(16), o_scan = k.take(scan_bytes);
+    TR_CUDA(c, R.topo.ensure(k.used));
     char* base = R.topo.as<char>();
     R.parent = (int32_t*)(base + o_parent); R.up = (uint32_t*)(base + o_up); R.pair_of = (uint32_t*)(base + o_pair);
     R.leaves = (uint32_t*)(base + o_leaves); R.empty = (uint8_t*)(base + o_empty); R.arrive = (uint32_t*)(base + o_arrive);
@@ -240,10 +215,9 @@ int derive_topology(trace_ctx* c) {
 int derive_shadow_topology(trace_ctx* c) {
     auto& R = c->refit;
     const int64_t n_prims = c->scene.n_prims, n_pairs = n_prims - 1;
-    size_t used = 0;
-    auto take = [&](size_t bytes) { const size_t off = (used + 255) & ~(size_t)255; used = off + bytes; return off; };
-    const size_t o_up_pair = take(n_pairs * 4), o_up_prim = take(n_prims * 4), o_arrive = take(n_pairs * 4);
-    TR_CUDA(c, R.shadow_topo.ensure(used));
+    Carve k;
+    const size_t o_up_pair = k.take(n_pairs * 4), o_up_prim = k.take(n_prims * 4), o_arrive = k.take(n_pairs * 4);
+    TR_CUDA(c, R.shadow_topo.ensure(k.used));
     char* base = R.shadow_topo.as<char>();
     R.shadow_up_pair = (uint32_t*)(base + o_up_pair); R.shadow_up_prim = (uint32_t*)(base + o_up_prim);
     R.shadow_arrive = (uint32_t*)(base + o_arrive);
@@ -354,28 +328,6 @@ int refit_run(trace_ctx* c, int64_t n_tris, const float* v, const float* nrm, bo
 
 }  // namespace
 
-size_t pair_scan_bytes(int64_t n, cudaStream_t s) {
-    size_t bytes = 0;
-    if (cub::DeviceScan::ExclusiveSum(nullptr, bytes, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)n, s) != cudaSuccess)
-        return 0;
-    return bytes ? bytes : 1;
-}
-
-cudaError_t pair_numbering(cudaStream_t s, const float4* nodes, int64_t n, uint32_t* flag, uint32_t* pair_of, void* tmp,
-                           size_t tmp_bytes) {
-    refit_is_interior<<<blocks_for(n, 256), 256, 0, s>>>(nodes, n, flag);
-    const cudaError_t e = cudaGetLastError();
-    return e != cudaSuccess ? e : cub::DeviceScan::ExclusiveSum(tmp, tmp_bytes, flag, pair_of, (int)n, s);
-}
-
-int ctx_drain(trace_ctx* c) {
-    TR_CUDA(c, cudaStreamSynchronize(c->stream));
-    for (int l = 0; l < trace_ctx::MAX_LANES; ++l) if (c->side[l]) TR_CUDA(c, cudaStreamSynchronize(c->side[l]));
-    cudaStream_t more[] = {c->chain_stream, c->coll_stream, c->copy_stream};
-    for (cudaStream_t s : more) if (s) TR_CUDA(c, cudaStreamSynchronize(s));
-    return 0;
-}
-
 extern "C" int trace_scene_refit(trace_ctx* c, int64_t n_tris, const float* tri_vertices, const float* tri_normals,
                                  int64_t n_spheres, const float* sphere_bounds) {
     if (!c) return 1;
@@ -405,7 +357,7 @@ extern "C" int trace_scene_copy_nodes(trace_ctx* c, trace_bvh_node* out) {
         trace_bvh_node& o = out[i];
         o.bmin[0] = a.x; o.bmin[1] = a.y; o.bmin[2] = a.z; o.bmax[0] = a.w; o.bmax[1] = b.x; o.bmax[2] = b.y;
         memcpy(&o.offset, &b.z, 4); memcpy(&o.meta, &b.w, 4);
-        o.meta &= ~0x20000000u;                            // the device-only "sphere below" bit (api.cu)
+        o.meta &= ~TR_NODE_SPHERE_BELOW;                   // the device-only "sphere below" bit (api.cu)
     }
     return 0;
 }

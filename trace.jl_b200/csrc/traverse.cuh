@@ -31,6 +31,21 @@ struct RayPrep {            // quantities that depend on the ray only
 #define TR_GUARD_REL 7.62939453125e-6f
 #define TR_NODE_SPHERE_BELOW 0x20000000u   // device-side node meta bit 29, set at upload
 #define TR_NODE_COUNT_MASK 0x1FFFFFFFu
+// node meta: bits 31-30 are 3 for a leaf (TRACE_NODE_LEAF), else the split axis; a leaf's primitive count below bit 29
+__host__ __device__ __forceinline__ bool tr_node_leaf(uint32_t meta) { return (meta >> 30) == 3u; }
+__host__ __device__ __forceinline__ uint32_t tr_node_count(uint32_t meta) { return meta & TR_NODE_COUNT_MASK; }
+__host__ __device__ __forceinline__ uint32_t tr_node_axis(uint32_t meta) { return meta >> 30; }
+
+// Julia's min / max without NaN: exact, and -0.0 < +0.0.  Every box the GPU builds or refits is a union under these,
+// so it does not depend on the order in which threads combine it.
+__device__ __forceinline__ float jl_min(float a, float b) { return (b < a || (b == a && signbit(b))) ? b : a; }
+__device__ __forceinline__ float jl_max(float a, float b) { return (b > a || (b == a && !signbit(b))) ? b : a; }
+// a triangle's vertex box folded into (lo, hi); from (+inf, -inf) it is the triangle's own box
+__device__ __forceinline__ void tri_box(float3 a, float3 b, float3 c, float lo[3], float hi[3]) {
+    lo[0] = jl_min(jl_min(jl_min(lo[0], a.x), b.x), c.x); hi[0] = jl_max(jl_max(jl_max(hi[0], a.x), b.x), c.x);
+    lo[1] = jl_min(jl_min(jl_min(lo[1], a.y), b.y), c.y); hi[1] = jl_max(jl_max(jl_max(hi[1], a.y), b.y), c.y);
+    lo[2] = jl_min(jl_min(jl_min(lo[2], a.z), b.z), c.z); hi[2] = jl_max(jl_max(jl_max(hi[2], a.z), b.z), c.z);
+}
 
 __device__ __forceinline__ RayPrep prepare_ray(float3 o, float3 d, float scene_scale = 0.0f) {
     RayPrep r;
@@ -191,6 +206,11 @@ static __device__ __noinline__ bool sphere_test(const DeviceSphere& s, float3 ro
 #define TR_PRIM_DEGENERATE_BIT 0x40000000u
 #define TR_PRIM_LAST_BIT 0x20000000u        // last primitive of its BVH leaf (set at upload; used by the pair-node walk)
 #define TR_PRIM_INDEX_MASK 0x1FFFFFFFu
+// is_degenerate (triangle_mesh.jl:65-68), the TR_PRIM_DEGENERATE_BIT of a triangle: decided from its vertices alone
+__host__ __device__ __forceinline__ bool tri_degenerate(float3 p0, float3 p1, float3 p2) {
+    const float3 g = cross3(p2 - p0, p1 - p0);
+    return dot3(g, g) == 0.0f;
+}
 #define TR_STACK_SIZE 64
 #define TR_WALK_PAIR (-1)     // "walk" selector of the kernels: 0 reference loop, -1 pair nodes, 4..32 batched leaves
 #ifndef TR_PARK_MAX
