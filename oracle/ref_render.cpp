@@ -628,6 +628,17 @@ extern "C" int ref_bsdf_sample(const trace_material* m, int mode, const float wo
     out[6] = s.pdf; out[7] = (float)s.type;
     return b.n;
 }
+// batched forms: q[i] = {material index, mode, flags (bsdf_f) or type (bsdf_sample)}; n_lobes[i] = the lobe count
+extern "C" int ref_bsdf_f_batch(const trace_material* mats, int64_t n, const int32_t* q, const float* wo, const float* wi,
+                                float* f, int32_t* n_lobes) {
+    for (int64_t i = 0; i < n; ++i) n_lobes[i] = ref_bsdf_f(&mats[q[3 * i]], q[3 * i + 1], wo + 3 * i, wi + 3 * i, q[3 * i + 2], f + 3 * i);
+    return 0;
+}
+extern "C" int ref_bsdf_sample_batch(const trace_material* mats, int64_t n, const int32_t* q, const float* wo, const float* u,
+                                     float* out, int32_t* n_lobes) {
+    for (int64_t i = 0; i < n; ++i) n_lobes[i] = ref_bsdf_sample(&mats[q[3 * i]], q[3 * i + 1], wo + 3 * i, u + 2 * i, q[3 * i + 2], out + 8 * i);
+    return 0;
+}
 extern "C" int ref_film_tile_add_sample(const trace_film_desc* f, const int tbv[4], float px, float py, const float rgb[3],
                                         float* contrib, float* wsum) {
     TileBounds tb = {tbv[0], tbv[1], tbv[2], tbv[3]};

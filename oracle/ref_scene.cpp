@@ -404,6 +404,15 @@ extern "C" int ref_prim_hit_record(const ref_scene* rs, int64_t prim_index, cons
     return 1;
 }
 
+// ref_hit_record over n rays (out: 24 floats per ray, a miss is all zeros)
+extern "C" int ref_hit_record_batch(const ref_scene* rs, int64_t n, const float* o, const float* d, const float* tmax, float* out,
+                                    int n_threads) {
+    parallel_for(n, n_threads, [&](int64_t a, int64_t b, int) {
+        for (int64_t i = a; i < b; ++i) ref_prim_hit_record(rs, -1, o + 3 * i, d + 3 * i, tmax ? tmax[i] : INF_F, out + 24 * i);
+    });
+    return 0;
+}
+
 extern "C" int ref_bounds_intersect(const float bmin[3], const float bmax[3], const float o[3], const float d[3],
                                     float tmax, float* t0o, float* t1o) {        // bounds.jl:151-167
     float t0 = 0.0f, t1 = tmax;

@@ -76,6 +76,14 @@ float ref_roughness_to_alpha(float r);                                          
 int   ref_bsdf_f(const trace_material*, int mode, const float wo[3], const float wi[3], int flags, float f_out[3]);
 int   ref_bsdf_sample(const trace_material*, int mode, const float wo[3], const float u[2], int type,
                       float out[8] /* wi(3), f(3), pdf, sampled_type */);
+/* the same over n inputs: q[i] = {material index into mats, mode, flags / type}; n_lobes[i] = the BSDF's lobe count */
+int   ref_bsdf_f_batch(const trace_material* mats, int64_t n, const int32_t* q, const float* wo, const float* wi,
+                       float* f_out /* n x 3 */, int32_t* n_lobes);
+int   ref_bsdf_sample_batch(const trace_material* mats, int64_t n, const int32_t* q, const float* wo, const float* u,
+                            float* out /* n x 8 */, int32_t* n_lobes);
+/* ref_hit_record over n rays (tmax may be NULL: Inf); out is n x 24, all zeros for a miss */
+int   ref_hit_record_batch(const ref_scene*, int64_t n, const float* o, const float* d, const float* tmax, float* out,
+                           int n_threads);
 /* add_sample! on a FilmTile (film.jl:134-164): splats into tile pixel arrays of size (ty1-ty0+1) x (tx1-tx0+1) */
 int   ref_film_tile_add_sample(const trace_film_desc*, const int tile_bounds[4] /* x0,y0,x1,y1 */,
                                float px, float py, const float rgb[3], float* contrib_rgb, float* weight_sum);

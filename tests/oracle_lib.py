@@ -53,6 +53,9 @@ def lib():
         L.ref_roughness_to_alpha.argtypes = [C.c_float]
         L.ref_bsdf_f.argtypes = [P, C.c_int, P, P, C.c_int, P]
         L.ref_bsdf_sample.argtypes = [P, C.c_int, P, P, C.c_int, P]
+        L.ref_bsdf_f_batch.argtypes = [P, C.c_int64, P, P, P, P, P]
+        L.ref_bsdf_sample_batch.argtypes = [P, C.c_int64, P, P, P, P, P]
+        L.ref_hit_record_batch.argtypes = [P, C.c_int64, P, P, P, P, C.c_int]
         L.ref_film_tile_add_sample.argtypes = [P, P, C.c_float, C.c_float, P, P, P]
         L.ref_rng.restype = C.c_float
         L.ref_rng.argtypes = [C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32]
@@ -82,6 +85,26 @@ def bvh_build(bounds, max_node_prims=1):
     depth = L.ref_bvh_max_depth(h)
     L.ref_bvh_free(h)
     return nodes, order, depth
+
+
+def bsdf_f_batch(mats, q, wo, wi):
+    """ref_bsdf_f over n inputs; q: [n, 3] (material index, mode, flags) -> f [n, 3], lobe count [n]"""
+    mats = np.ascontiguousarray(mats)
+    q = np.ascontiguousarray(q, dtype=np.int32)
+    wo, wi = f3(wo), f3(wi)
+    f, nl = np.zeros((len(q), 3), np.float32), np.zeros(len(q), np.int32)
+    lib().ref_bsdf_f_batch(p(mats), len(q), p(q), p(wo), p(wi), p(f), p(nl))
+    return f, nl
+
+
+def bsdf_sample_batch(mats, q, wo, u):
+    """ref_bsdf_sample over n inputs; q: [n, 3] (material index, mode, type) -> [n, 8] (wi, f, pdf, type), lobe count [n]"""
+    mats = np.ascontiguousarray(mats)
+    q = np.ascontiguousarray(q, dtype=np.int32)
+    wo, u = f3(wo), f3(u)
+    out, nl = np.zeros((len(q), 8), np.float32), np.zeros(len(q), np.int32)
+    lib().ref_bsdf_sample_batch(p(mats), len(q), p(q), p(wo), p(u), p(out), p(nl))
+    return out, nl
 
 
 class OracleScene:
@@ -128,6 +151,14 @@ class OracleScene:
             return None
         return dict(t=out[1], p=out[2:5], ng=out[5:8], ns=out[8:11], ss=out[11:14], ts=out[14:17], wo=out[17:20],
                     uv=out[20:22], prim=int(out[22]), material=int(out[23]))
+
+    def hit_records(self, o, d, t_max=None):
+        """ref_hit_record over n rays -> float32 [n, 24] (hit, t, p, ng, ns, ss, ts, wo, uv, original, material)"""
+        o, d = f3(o).reshape(-1, 3), f3(d).reshape(-1, 3)
+        t = None if t_max is None else f3(t_max)
+        out = np.zeros((len(o), 24), np.float32)
+        lib().ref_hit_record_batch(self.h, len(o), p(o), p(d), p(t), p(out), self.threads)
+        return out
 
     def render_whitted(self, cam, fd, spp, max_depth, seed, film_xyzw, max_tiles=0, threads=None):
         cnt = np.zeros(2, np.uint64)

@@ -163,9 +163,14 @@ __device__ __forceinline__ int num_components(const LobeSet& s, uint32_t flags) 
     return n;
 }
 
+// Julia's max(0f0, x) and min(x, 1f0): a NaN x stays NaN (fmaxf / fminf would return the other operand) and
+// max(0f0, -0f0) is +0, as the reference computes them (the oracle's jl_max / jl_min)
+__device__ __forceinline__ float jl_max0(float x) { return !(x <= 0.0f) ? x : 0.0f; }
+__device__ __forceinline__ float jl_min1(float x) { return !(x >= 1.0f) ? x : 1.0f; }
+
 // ------------------------------------------------------------------ local-frame helpers, Trace.jl:109-121
 __device__ __forceinline__ float cos_th(float3 w) { return w.z; }
-__device__ __forceinline__ float sin_th(float3 w) { return sqrtf(fmaxf(0.0f, 1.0f - w.z * w.z)); }
+__device__ __forceinline__ float sin_th(float3 w) { return sqrtf(jl_max0(1.0f - w.z * w.z)); }
 __device__ __forceinline__ float tan_th(float3 w) { return sin_th(w) / w.z; }
 __device__ __forceinline__ float cos_ph(float3 w) { float s = sin_th(w); return s == 0.0f ? 1.0f : clampf(w.x / s, -1.0f, 1.0f); }
 __device__ __forceinline__ float sin_ph(float3 w) { float s = sin_th(w); return s == 0.0f ? 1.0f : clampf(w.y / s, -1.0f, 1.0f); }
@@ -184,11 +189,11 @@ __device__ __forceinline__ float2 concentric_disk(float u0, float u1) {
 }
 __device__ __forceinline__ float3 cosine_hemisphere(float u0, float u1) {
     float2 d = concentric_disk(u0, u1);
-    return f3(d.x, d.y, sqrtf(fmaxf(0.0f, 1.0f - d.x * d.x - d.y * d.y)));
+    return f3(d.x, d.y, sqrtf(jl_max0(1.0f - d.x * d.x - d.y * d.y)));
 }
 __device__ __forceinline__ float3 uniform_sphere(float u0, float u1) {
     float z = 1.0f - 2.0f * u0;
-    float r = sqrtf(fmaxf(0.0f, 1.0f - z * z));
+    float r = sqrtf(jl_max0(1.0f - z * z));
     float phi = 2.0f * TR_PI * u1;
     return f3(r * cosf(phi), r * sinf(phi), z);
 }
@@ -202,7 +207,7 @@ __device__ __forceinline__ float3 uniform_cone(float u0, float u1, float cmax) {
 // ------------------------------------------------------------------ Fresnel / refraction, reflection/bxdf.jl:52-95
 __device__ __forceinline__ bool refract(float3 wi, float3 n, float eta, float3& wt) {
     float ci = dot3(n, wi);
-    float s2i = fmaxf(0.0f, 1.0f - ci * ci);
+    float s2i = jl_max0(1.0f - ci * ci);
     float s2t = (eta * eta) * s2i;
     if (s2t >= 1.0f) { wt = f3s(0.0f); return false; }
     float ct = sqrtf(1.0f - s2t);
@@ -212,10 +217,10 @@ __device__ __forceinline__ bool refract(float3 wi, float3 n, float eta, float3& 
 __device__ __forceinline__ float fresnel_dielectric(float ci, float ei, float et) {
     ci = clampf(ci, -1.0f, 1.0f);
     if (ci <= 0.0f) { float t = ei; ei = et; et = t; ci = fabsf(ci); }
-    float si = sqrtf(fmaxf(0.0f, 1.0f - ci * ci));
+    float si = sqrtf(jl_max0(1.0f - ci * ci));
     float st = si * ei / et;
     if (st >= 1.0f) return 1.0f;
-    float ct = sqrtf(fmaxf(0.0f, 1.0f - st * st));
+    float ct = sqrtf(jl_max0(1.0f - st * st));
     float rpar = (et * ci - ei * ct) / (et * ci + ei * ct);
     float rper = (ei * ci - et * ct) / (ei * ci + et * ct);
     return 0.5f * (rpar * rpar + rper * rper);
@@ -245,7 +250,7 @@ __device__ __forceinline__ float2 tr_sample11(float cth, float u1, float u2) {
         double phi = 6.28318530718 * (double)u2;
         return make_float2((float)((double)r * cos(phi)), (float)((double)r * sin(phi)));
     }
-    float sth = sqrtf(fmaxf(0.0f, 1.0f - cth * cth));
+    float sth = sqrtf(jl_max0(1.0f - cth * cth));
     float tth = sth / cth;
     float a = 1.0f / tth;
     float g1 = 2.0f / (1.0f + sqrtf(1.0f + 1.0f / (a * a)));
@@ -253,7 +258,7 @@ __device__ __forceinline__ float2 tr_sample11(float cth, float u1, float u2) {
     float tmp = 1.0f / (a * a - 1.0f);
     if (tmp > 1e10f) tmp = 1e10f;
     float b = tth, b2 = b * b;
-    float d = sqrtf(fmaxf(0.0f, b2 * (tmp * tmp) - (a * a - b2) * tmp));
+    float d = sqrtf(jl_max0(b2 * (tmp * tmp) - (a * a - b2) * tmp));
     float x1 = b * tmp - d, x2 = b * tmp + d;
     float sx = (a < 0.0f || x2 > 1.0f / tth) ? x1 : x2;
     float s;
@@ -306,7 +311,7 @@ __device__ __forceinline__ float3 lobe_f(const Lobe& l, float3 wo, float3 wi) {
     if (l.kind == LK_OREN_NAYAR) {                     // microfacet.jl:21-42
         const float si = sin_th(wi), so = sin_th(wo);
         float max_cos = 0.0f;
-        if (si > 1e-4f && so > 1e-4f) max_cos = fmaxf(0.0f, cos_ph(wi) * cos_ph(wo) + sin_ph(wi) * sin_ph(wo));
+        if (si > 1e-4f && so > 1e-4f) max_cos = jl_max0(cos_ph(wi) * cos_ph(wo) + sin_ph(wi) * sin_ph(wo));
         float sa, tb;
         if (wi.z > fabsf(wo.z)) { sa = so; tb = si / fabsf(wi.z); }        // abs(Bool) quirk, Q18
         else { sa = si; tb = so / fabsf(wo.z); }
@@ -415,7 +420,7 @@ __device__ __forceinline__ BSDFSample bsdf_sample(const LobeSet& s, const Frame&
         }
     }
     const Lobe& bx = s.l[chosen];
-    float ur0 = fminf(u0 * (float)mc - (float)comp, 1.0f);
+    float ur0 = jl_min1(u0 * (float)mc - (float)comp);
     float3 wo = to_local(fr, wo_w);
     if (wo.z == 0.0f) return none;
     LobeSample ls = lobe_sample(bx, wo, ur0, u1);
