@@ -7,6 +7,7 @@
  *   trace_bvh_build            <- BVHAccel(primitives, max_node_primitives)   src/accel/bvh.jl:55-80 (+ _init :87-185, _unroll :187-206)
  *   trace_scene_upload         <- Scene(lights, aggregate)                    src/Trace.jl:176-187
  *   trace_scene_upload_mesh_device  (extension: a triangle scene built and packed on the GPU from device arrays)
+ *   trace_scene_attach_mesh_device  (extension: such a mesh attached to the uploaded scene, rebuilt alone per frame)
  *   trace_intersect            <- intersect!(bvh|scene, ray)                  src/accel/bvh.jl:212-258, src/Trace.jl:189-191
  *   trace_occluded             <- intersect_p(bvh|scene, ray)                 src/accel/bvh.jl:260-299, src/Trace.jl:192-194
  *   trace_render_whitted       <- (i::SamplerIntegrator)(scene)               src/integrators/sampler.jl:12-56
@@ -260,6 +261,38 @@ typedef struct trace_mesh_device_desc {
     int64_t n_lights;     const trace_light* lights;         /* host */
 } trace_mesh_device_desc;
 int trace_scene_upload_mesh_device(trace_ctx* ctx, const trace_mesh_device_desc* mesh, int64_t* n_nodes_out);
+
+/* ---- attach a device mesh to the uploaded scene (extension: the reference has no counterpart).  The base is the scene
+ * of the last trace_scene_upload or trace_scene_upload_mesh_device; each attach composes it with `mesh` (the same
+ * descriptor and checks as trace_scene_upload_mesh_device), and a later attach replaces the mesh attached before it
+ * while the base stays resident.  The composed device scene is bit for bit the one trace_scene_upload builds from D:
+ * with the base's Nb nodes, Qb interior nodes, Pb primitives, Tb triangles, Mb materials and Lb lights and the mesh's
+ * n triangles,
+ *   node 0          interior, box = Julia min / max union of the base's and the mesh's root boxes, first child the
+ *                   base, second child the mesh (offset 1 + Nb); split axis = the k maximising (mesh.min[k] +
+ *                   mesh.max[k]) - (base.min[k] + base.max[k]) in float32, ties to the lowest k, non-finite values lose;
+ *   nodes 1 .. Nb   the base's nodes in order, interior offsets + 1 (leaf offsets unchanged);
+ *   the rest        the mesh's LBVH as trace_scene_upload_mesh_device builds it, interior offsets + 1 + Nb, leaf
+ *                   offsets + Pb;
+ *   primitives      the base's, then {TRIANGLE, Tb + order[k], Mb + tri_materials[order[k]], Pb + order[k]}: queries
+ *                   report mesh triangle i as Pb + i;
+ *   arrays          triangles base ++ mesh, the base's spheres, materials base ++ mesh, lights base ++ mesh
+ * - nodes, pair records, primitive and normal records, spheres, materials, lights, root reference, scene_scale and
+ * counts alike.  The shadow tree is composed, not rebuilt: the scene has one only when both parts have one (or are a
+ * single primitive), it has no spheres and 1 + max(base depth, mesh depth) <= 64.  Its pair 0 holds the two parts'
+ * root boxes and references with the root's split-axis bit, then come the base's pairs (pair references + 1), then
+ * the mesh's (pair references + Pb, leaf references + Pb): n_prims - 1 pairs.  Answers do not depend on the shadow
+ * tree.
+ * The first attach after an upload moves the base's node, pair and shadow-pair records up one slot (a cost
+ * proportional to the base, with a transient peak of about twice those buffers); later attaches write node 0, pair 0
+ * and the mesh's part only.  Refused before anything is written (the previous scene stays uploaded and usable): the
+ * refusals of trace_scene_upload_mesh_device, n_tris == 0, no scene uploaded, a base without primitives, 2^30 or more
+ * primitives or too many interior nodes in the composed scene.  trace_scene_refit[_device] applies as after
+ * trace_scene_upload(D): its input is all Tb + n triangles in D's order.  A refit moves base triangles until the next
+ * upload; the next attach reads the base's boxes from the device.  Like the uploads the call waits for all of the
+ * context's work, ends any SPPM session and is synchronous; it is local to the context (every rank attaches the same
+ * mesh).  *n_nodes_out (may be NULL) receives the composed node count.  TRACE_BVH_PROFILE=1 prints per-phase times. */
+int trace_scene_attach_mesh_device(trace_ctx* ctx, const trace_mesh_device_desc* mesh, int64_t* n_nodes_out);
 
 /* ---- refit (extension: the reference has no counterpart; it rebuilds BVHAccel).  New positions for the triangles of
  * the last upload, with the tree's topology kept (node structure, primitive order, materials, spheres, lights) and every

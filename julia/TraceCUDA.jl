@@ -308,6 +308,24 @@ function upload_mesh_device!(ctx::Context, n_tris, vertices, normals, flags, mat
     n_nodes[]
 end
 
+# A moving device mesh inside a static environment: upload!(ctx, env) once, then attach_mesh_device!(ctx, ...) each
+# frame (trace_scene_attach_mesh_device).  Each attach rebuilds only the mesh's tree and composes it with the environment
+# under a new root (environment first), replacing the mesh attached before; the environment keeps its own tree
+# (spheres, nested BVHAccels, any builder).  Same arguments as upload_mesh_device!; the mesh's materials and lights come
+# after the environment's, and queries report mesh triangle i as (the environment's primitive count) + i.  The functors
+# called with `env` render the composed scene; refit! does not apply (trace_scene_refit_device with all triangles does).
+function attach_mesh_device!(ctx::Context, n_tris, vertices, normals, flags, material_ids, materials::Vector, lights::Vector;
+                             max_node_primitives = 1)
+    GC.@preserve materials lights begin
+        d = MeshDeviceDesc(n_tris, UInt(vertices), UInt(normals), UInt(flags), UInt(material_ids), Int32(max_node_primitives),
+                           Int32(0), length(materials), pointer(materials), length(lights), pointer(lights))
+        n_nodes = Ref{Int64}(0)
+        check(ctx, ccall((:trace_scene_attach_mesh_device, LIB), Cint, (Ptr{Cvoid}, Ref{MeshDeviceDesc}, Ref{Int64}),
+                         ctx.h, d, n_nodes))
+    end
+    n_nodes[]
+end
+
 # ---- the two functors ------------------------------------------------------------------------------------------------
 struct GPU{I<:Trace.Integrator,C}
     integrator::I

@@ -12,7 +12,7 @@ through the C ABI in include/trace_cuda.h.  There is no CPU fallback.
 """
 from .geometry import (Bounds2, Bounds3, Normal3f, Point2f, Point3f, Transformation, Vec3f, coordinate_system, cross, dot,
                        look_at, norm, normalize, perspective, rotate_x, rotate_y, rotate_z, scale, translate)
-from .scene import (BVHAccel, ConstantTexture, MixTexture, ScaleTexture, DeviceMeshScene, DirectionalLight, FlatScene, GeometricPrimitive, GlassMaterial, MatteMaterial, MirrorMaterial,
+from .scene import (BVHAccel, ConstantTexture, MixTexture, ScaleTexture, CompositeScene, DeviceMeshScene, DirectionalLight, FlatScene, GeometricPrimitive, GlassMaterial, MatteMaterial, MirrorMaterial,
                     PlasticMaterial, PointLight, PrimitiveBatch, RGBSpectrum, Scene, ShapeCore, Sphere, SpotLight, Triangle,
                     TriangleMesh, TriangleSet, create_triangle_mesh, load_triangle_mesh)
 from .render import (Context, comm_unique_id, Film, LanczosSincFilter, PerspectiveCamera, SPPMIntegrator, UniformSampler, WhittedIntegrator,

@@ -290,8 +290,7 @@ extern "C" int trace_scene_upload(trace_ctx* c, const trace_scene_desc* d) {
     TR_CUDA(c, cudaStreamSynchronize(c->stream));      // host staging vectors die at return
     c->refit.tri_index.swap(tri_index);
     c->refit.slot_tri_on_device = false;
-    return ctx_commit_scene(c, d->n_nodes, d->n_prims, d->n_spheres, d->n_materials, d->n_lights, d->n_tris, n_pairs,
-                            nodes.data(), nullptr);
+    return ctx_commit_scene(c, d->n_nodes, d->n_prims, d->n_spheres, mats, lights, d->n_tris, n_pairs, nodes.data(), nullptr);
 }
 
 int ctx_pack_materials(trace_ctx* c, int64_t n, const trace_material* in, std::vector<DeviceMaterial>& out) {
@@ -357,11 +356,38 @@ static uint32_t root_ref_of(const float4* root) {
     return TR_REF_LEAF | (tr_node_count(meta) ? offset : 0u);
 }
 
-// The tail of every upload, once the scene buffers hold the new scene: the DeviceScene, root_ref and scene_scale from
-// the root node record, the shadow tree, the refit state and the end of any SPPM session.  The caller sets the
-// refit's slot -> triangle map.
-int ctx_commit_scene(trace_ctx* c, int64_t n_nodes, int64_t n_prims, int64_t n_spheres, int64_t n_materials,
-                     int64_t n_lights, int64_t n_tris, int64_t n_pairs, const float4* root, void* shadow_scratch) {
+// The tail of every upload, once the scene buffers hold the new scene: the shadow tree, the scene as the base of
+// later attaches (trace_scene_attach_mesh_device, upload_device.cu; `mats` and `lights` are taken), then
+// ctx_publish_scene.  The caller sets the refit's slot -> triangle map.
+int ctx_commit_scene(trace_ctx* c, int64_t n_nodes, int64_t n_prims, int64_t n_spheres, std::vector<DeviceMaterial>& mats,
+                     std::vector<DeviceLight>& lights, int64_t n_tris, int64_t n_pairs, const float4* root,
+                     void* shadow_scratch) {
+    // the shadow tree (traverse.cuh, traverse_shadow): built on the device from the uploaded primitive records.  Scenes
+    // with analytic spheres have none (the guard its walk admits nodes with is off below spheres); neither has a scene
+    // uploaded with option shadow_tree 0
+    int depth = 0;
+    bool shadow = false;
+    if (c->shadow_tree && n_spheres == 0 && n_prims >= 2) {
+        TR_CUDA(c, c->b_shadow.ensure((size_t)(n_prims - 1) * 4 * sizeof(float4)));
+        const int rc = shadow_tree_build(c->stream, c->b_prims.p, n_prims, c->b_shadow.p, shadow_scratch, &depth);
+        if (rc == 0) shadow = true;
+        else if (rc != LBVH_NAN_BOUND && rc != LBVH_TOO_DEEP) return c->fail("scene: shadow tree build failed (CUDA error)");
+    }
+    auto& B = c->base;
+    B.n_nodes = n_nodes; B.n_pairs = n_pairs; B.n_prims = n_prims; B.n_tris = n_tris; B.n_spheres = n_spheres;
+    B.shadow_depth = shadow ? depth : (n_prims == 1 ? 1 : 0);
+    B.moved = false;
+    B.materials.swap(mats);
+    B.lights.swap(lights);
+    ctx_publish_scene(c, n_nodes, n_prims, n_spheres, (int64_t)B.materials.size(), (int64_t)B.lights.size(), n_tris, n_pairs,
+                      root, shadow);
+    return 0;
+}
+
+// The DeviceScene over the scene buffers, root_ref and scene_scale from the root node record, the shadow tree in
+// b_shadow when `shadow`, the refit state and the end of any SPPM session
+void ctx_publish_scene(trace_ctx* c, int64_t n_nodes, int64_t n_prims, int64_t n_spheres, int64_t n_materials,
+                       int64_t n_lights, int64_t n_tris, int64_t n_pairs, const float4* root, bool shadow) {
     DeviceScene& s = c->scene;
     s.nodes = c->b_nodes.as<float4>(); s.pairs = c->b_pairs.as<float4>(); s.prims = c->b_prims.as<float4>(); s.tnorm = c->b_tnorm.as<float4>();
     s.spheres = c->b_spheres.as<DeviceSphere>(); s.materials = c->b_materials.as<DeviceMaterial>();
@@ -377,22 +403,12 @@ int ctx_commit_scene(trace_ctx* c, int64_t n_nodes, int64_t n_prims, int64_t n_s
             if (std::isfinite(a)) s.scene_scale = fmaxf(s.scene_scale, a);
         }
     }
-    // the shadow tree (traverse.cuh, traverse_shadow): built on the device from the uploaded primitive records.  Scenes
-    // with analytic spheres have none (the guard its walk admits nodes with is off below spheres); neither has a scene
-    // uploaded with option shadow_tree 0
-    s.shadow_pairs = nullptr;
-    if (c->shadow_tree && n_spheres == 0 && n_prims >= 2) {
-        TR_CUDA(c, c->b_shadow.ensure((size_t)(n_prims - 1) * 4 * sizeof(float4)));
-        const int rc = shadow_tree_build(c->stream, c->b_prims.p, n_prims, c->b_shadow.p, shadow_scratch);
-        if (rc == 0) s.shadow_pairs = c->b_shadow.as<float4>();
-        else if (rc != LBVH_NAN_BOUND && rc != LBVH_TOO_DEEP) return c->fail("scene: shadow tree build failed (CUDA error)");
-    }
+    s.shadow_pairs = shadow ? c->b_shadow.as<float4>() : nullptr;
     c->have_scene = true;
     c->refit.n_tris = n_tris; c->refit.n_spheres = n_spheres; c->refit.n_pairs = n_pairs;
     c->refit.topo_ready = false;
     c->refit.shadow_topo_ready = false;
     sppm_end_session(c);
-    return 0;
 }
 
 int ctx_drain(trace_ctx* c) {

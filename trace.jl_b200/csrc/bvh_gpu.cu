@@ -179,11 +179,12 @@ __global__ void lbvh_bottom_up(const float* __restrict__ pb, const uint32_t* __r
 }
 
 // 5. emit: every emitted node finds its preorder slot by climbing to the root (left child = parent + 1, right child =
-// parent + 1 + size(left); depth <= TR_STACK_SIZE is checked before this runs) and writes its record
+// parent + 1 + size(left); depth <= TR_STACK_SIZE is checked before this runs) and writes its record, interior offsets
+// shifted by node_shift and leaf offsets by prim_shift (an attached mesh's place in the composed scene; else 0)
 __global__ void lbvh_emit(int64_t n, int m, const uint32_t* __restrict__ child, const int32_t* __restrict__ parent,
                           const uint32_t* __restrict__ first, const uint32_t* __restrict__ count,
                           const uint8_t* __restrict__ axis, const float* __restrict__ box, const uint32_t* __restrict__ size,
-                          trace_bvh_node* __restrict__ out) {
+                          uint32_t node_shift, uint32_t prim_shift, trace_bvh_node* __restrict__ out) {
     const int64_t v = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (v >= 2 * n - 1) return;
     const bool internal = v < n - 1;
@@ -200,10 +201,10 @@ __global__ void lbvh_emit(int64_t n, int m, const uint32_t* __restrict__ child, 
     for (int c = 0; c < 3; ++c) { nd.bmin[c] = box[6 * v + c]; nd.bmax[c] = box[6 * v + 3 + c]; }
     const uint32_t cnt = internal ? count[v] : 1u;
     if (cnt <= (uint32_t)m) {
-        nd.offset = internal ? first[v] : (uint32_t)(v - (n - 1));
+        nd.offset = prim_shift + (internal ? first[v] : (uint32_t)(v - (n - 1)));
         nd.meta = TRACE_NODE_LEAF | cnt;
     } else {
-        nd.offset = pre + 1u + size[child[2 * v]];
+        nd.offset = node_shift + pre + 1u + size[child[2 * v]];
         nd.meta = (uint32_t)axis[v] << 30;
     }
     out[pre] = nd;
@@ -308,7 +309,7 @@ int build(cudaStream_t s, const float* hb, int64_t n, int m, trace_bvh** out, Ph
     Status hs;
     if (const int rc = build_core(s, n, m, b, sort_bytes, hs, ph)) return rc;
     const int64_t n_nodes = hs.root_size;
-    lbvh_emit<<<blocks_for(nn, T), T, 0, s>>>(n, m, b.child, b.parent, b.first, b.count, b.axis, b.box, b.size, b.nodes);
+    lbvh_emit<<<blocks_for(nn, T), T, 0, s>>>(n, m, b.child, b.parent, b.first, b.count, b.axis, b.box, b.size, 0u, 0u, b.nodes);
     if (cudaGetLastError() != cudaSuccess) return LBVH_CUDA;
     ph.mark(s, "emit");
     trace_bvh_node* hn = nullptr;
@@ -345,15 +346,16 @@ __global__ void lbvh_prim_bounds(const float4* __restrict__ prims, int64_t n, fl
 
 // One 64-byte pair record per internal node, in Karras numbering (the root is pair 0): both children's boxes, their
 // references (a pair index, or TR_REF_LEAF | primitive slot for a leaf, traverse.cuh) and the split axis as
-// a bit in the first half - the layout of the upload's pair records (api.cu).
+// a bit in the first half - the layout of the upload's pair records (api.cu).  Every reference is shifted by `shift`.
 __global__ void lbvh_emit_pairs(int64_t n, const uint32_t* __restrict__ child, const uint32_t* __restrict__ sorted_ids,
-                                const uint8_t* __restrict__ axis, const float* __restrict__ box, float4* __restrict__ pairs) {
+                                const uint8_t* __restrict__ axis, const float* __restrict__ box, uint32_t shift,
+                                float4* __restrict__ pairs) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= n - 1) return;
     for (int k = 0; k < 2; ++k) {
         const int64_t v = child[2 * i + k];
         const float* bx = box + 6 * v;
-        const uint32_t ref = v < n - 1 ? (uint32_t)v : (TR_REF_LEAF | sorted_ids[v - (n - 1)]);
+        const uint32_t ref = v < n - 1 ? shift + (uint32_t)v : (TR_REF_LEAF | (shift + sorted_ids[v - (n - 1)]));
         const uint32_t extra = k == 0 ? (1u << axis[i]) : 0u;
         pairs[4 * i + 2 * k] = make_float4(bx[0], bx[1], bx[2], bx[3]);
         pairs[4 * i + 2 * k + 1] = make_float4(bx[4], bx[5], __uint_as_float(ref), __uint_as_float(extra));
@@ -405,8 +407,10 @@ size_t lbvh_scratch_bytes(int64_t n, cudaStream_t s) {
 // The shadow tree of an uploaded scene (api.cu): an LBVH with one primitive per leaf over the n >= 2 uploaded primitive
 // records `prims` (device, BVH slot order, triangles only), written as n - 1 pair records to `pairs` (device).  Nothing
 // crosses to the host but the build's status.  `scratch` (lbvh_scratch_bytes(n)) or nullptr: an allocation of its own.
-// Returns LBVH_OK, _NAN_BOUND (a NaN vertex), _TOO_DEEP or _CUDA.
-int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs, void* scratch) {
+// Returns LBVH_OK, _NAN_BOUND (a NaN vertex), _TOO_DEEP or _CUDA; *depth (may be NULL): the tree's levels, root = 1.
+// ref_shift moves every reference: pairs and slots of a tree that starts at pair and slot ref_shift of a larger one.
+int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs, void* scratch, int* depth,
+                      uint32_t ref_shift) {
     if (n < 2 || n >= 0x40000000ll) return 1;
     const size_t sort_bytes = sort_bytes_for(n, s);
     if (!sort_bytes) return LBVH_CUDA;
@@ -418,8 +422,10 @@ int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs,
     PhaseTimer quiet;
     Status hs;
     if (const int rc = build_core(s, n, 1, b, sort_bytes, hs, quiet)) return rc;
-    lbvh_emit_pairs<<<blocks_for(n - 1, T), T, 0, s>>>(n, b.child, b.ids_sorted, b.axis, b.box, static_cast<float4*>(pairs));
+    lbvh_emit_pairs<<<blocks_for(n - 1, T), T, 0, s>>>(n, b.child, b.ids_sorted, b.axis, b.box, ref_shift,
+                                                       static_cast<float4*>(pairs));
     if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess) return LBVH_CUDA;
+    if (depth) *depth = (int)hs.root_depth;
     return LBVH_OK;
 }
 
@@ -456,14 +462,14 @@ int lbvh_mesh_build(cudaStream_t s, const float* v, const float* nrm, const uint
     return LBVH_OK;
 }
 
-int lbvh_mesh_emit(cudaStream_t s, int64_t n, int m, void* scratch, void* nodes) {
+int lbvh_mesh_emit(cudaStream_t s, int64_t n, int m, void* scratch, void* nodes, uint32_t node_shift, uint32_t prim_shift) {
     const size_t sort_bytes = sort_bytes_for(n, s);
     if (!sort_bytes) return LBVH_CUDA;
     Buffers b;
     b.borrow(scratch, n, sort_bytes);
     const int T = 256;
     lbvh_emit<<<blocks_for(2 * n - 1, T), T, 0, s>>>(n, m, b.child, b.parent, b.first, b.count, b.axis, b.box, b.size,
-                                                    static_cast<trace_bvh_node*>(nodes));
+                                                    node_shift, prim_shift, static_cast<trace_bvh_node*>(nodes));
     return cudaGetLastError() == cudaSuccess ? LBVH_OK : LBVH_CUDA;
 }
 

@@ -42,6 +42,18 @@ struct DevBuf {
         if (e == cudaSuccess) bytes = want;
         return e;
     }
+    // grow-only, keeping the first `keep` bytes (copied on `s`, which is synchronised before the old block is freed)
+    cudaError_t ensure_keep(size_t need, size_t keep, cudaStream_t s) {
+        if (need <= bytes) return cudaSuccess;
+        DevBuf n;
+        cudaError_t e = n.ensure(need);
+        if (e == cudaSuccess && keep && p) e = cudaMemcpyAsync(n.p, p, keep, cudaMemcpyDeviceToDevice, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) { n.release(); return e; }
+        release();
+        p = n.p; bytes = n.bytes;
+        return cudaSuccess;
+    }
     void release() { if (p) cudaFree(p); p = nullptr; bytes = 0; }
     template <class T> T* as() const { return reinterpret_cast<T*>(p); }
 };
@@ -120,6 +132,15 @@ struct trace_ctx {
     // trace_scene_upload_mesh_device (upload_device.cu): the LBVH build's scratch, then the pair numbering's and the
     // shadow tree build's (grow-only, so a per-frame rebuild of the same size allocates nothing)
     DevBuf b_build;
+    // trace_scene_attach_mesh_device (upload_device.cu): the base, the scene of the last upload, stays resident while
+    // meshes are attached to it.  After the first attach its node, pair and shadow-pair records sit one slot up.
+    struct Base {
+        int64_t n_nodes = 0, n_pairs = 0, n_prims = 0, n_tris = 0, n_spheres = 0;
+        std::vector<DeviceMaterial> materials;   // packed at upload: each attach puts base ++ mesh again
+        std::vector<DeviceLight> lights;
+        int shadow_depth = 0;     // levels of its shadow tree (1: a single primitive, no pair); 0: none usable
+        bool moved = false;       // its records sit one slot up (an attach ran since the upload)
+    } base;
 
     // refit (refit.cu): what trace_scene_refit needs of the last upload.  The host keeps only the BVH-slot -> triangle
     // map; the device topology (parents, pair slots, leaf list) is derived from b_nodes at the first refit after an
@@ -320,22 +341,28 @@ void sppm_free(trace_ctx* ctx);
 void sppm_end_session(trace_ctx* ctx);
 void whitted_film_range(const trace_ctx* ctx, long long npix, long long* p0, long long* p1);
 // implemented in api.cu: the parts of a scene upload that do not depend on where the tree was built.  `root` is the
-// uploaded root node record (2 float4; unused for an empty tree).
+// uploaded root node record (2 float4; unused for an empty tree).  ctx_commit_scene, the tail of both uploads, builds
+// the shadow tree, makes the scene the attach base (taking the packed materials and lights) and publishes it;
+// ctx_publish_scene alone is the tail of an attach, whose shadow tree (or none) is already in b_shadow.
 int ctx_pack_materials(trace_ctx* ctx, int64_t n, const trace_material* in, std::vector<DeviceMaterial>& out);
 int ctx_pack_lights(trace_ctx* ctx, int64_t n, const trace_light* in, std::vector<DeviceLight>& out);
 int ctx_put(trace_ctx* ctx, DevBuf& b, const void* src, size_t bytes);
-int ctx_commit_scene(trace_ctx* ctx, int64_t n_nodes, int64_t n_prims, int64_t n_spheres, int64_t n_materials,
-                     int64_t n_lights, int64_t n_tris, int64_t n_pairs, const float4* root, void* shadow_scratch);
+int ctx_commit_scene(trace_ctx* ctx, int64_t n_nodes, int64_t n_prims, int64_t n_spheres, std::vector<DeviceMaterial>& mats,
+                     std::vector<DeviceLight>& lights, int64_t n_tris, int64_t n_pairs, const float4* root,
+                     void* shadow_scratch);
+void ctx_publish_scene(trace_ctx* ctx, int64_t n_nodes, int64_t n_prims, int64_t n_spheres, int64_t n_materials,
+                       int64_t n_lights, int64_t n_tris, int64_t n_pairs, const float4* root, bool shadow);
 // implemented in api.cu: waits for every stream of the context (caller's, lanes, SPPM chain / collectives, copies)
 int ctx_drain(trace_ctx* ctx);
 // implemented in upload_device.cu, the device half of both uploads: the preorder pair numbering of a device node array
 // (2 float4 per node), pair_of[i] = interior nodes before node i, as an exclusive scan of "is interior" (`flag`: n
-// words of scratch; `tmp`: pair_scan_bytes(n) bytes of scan scratch); and the scene's pair records built with it
+// words of scratch; `tmp`: pair_scan_bytes(n) bytes of scan scratch); and the scene's pair records built with it, for
+// the n_nodes nodes from node0 on, numbered from pair0 on (both 0 for an upload; an attach's mesh part otherwise)
 size_t pair_scan_bytes(int64_t n, cudaStream_t s);
 cudaError_t pair_numbering(cudaStream_t s, const float4* nodes, int64_t n, uint32_t* flag, uint32_t* pair_of, void* tmp,
                            size_t tmp_bytes);
 size_t pair_scratch_bytes(int64_t n_nodes, size_t scan_bytes);
-int ctx_pack_pairs(trace_ctx* ctx, int64_t n_nodes, char* scratch, size_t scan_bytes);
+int ctx_pack_pairs(trace_ctx* ctx, int64_t n_nodes, char* scratch, size_t scan_bytes, int64_t node0 = 0, int64_t pair0 = 0);
 
 // TRACE_BVH_PROFILE=1: CUDA events between the phases of an upload / refit call, printed as one stderr line
 struct PhaseTimer {
@@ -370,11 +397,15 @@ enum LbvhStatus {
     LBVH_BAD_MATERIAL = 9,       // mesh builds: a material index out of range
 };
 // The shadow tree over uploaded primitive records, in `scratch` (lbvh_scratch_bytes(n) bytes) or, with nullptr, an
-// allocation of its own: LBVH_OK, _NAN_BOUND, _TOO_DEEP or _CUDA.
-int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs, void* scratch);
+// allocation of its own: LBVH_OK, _NAN_BOUND, _TOO_DEEP or _CUDA; *depth (may be NULL) its levels.  Every reference
+// it writes is shifted by ref_shift (an attach's mesh part: its pairs and primitive slots start there).
+int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs, void* scratch, int* depth = nullptr,
+                      uint32_t ref_shift = 0);
 size_t lbvh_scratch_bytes(int64_t n, cudaStream_t s);
 // The tree of trace_scene_upload_mesh_device, in `scratch`: lbvh_mesh_build validates, bounds and builds (phases
 // "validate", "bounds" and "build" of `ph`); lbvh_mesh_emit, once the input is accepted, writes the node records.
 int lbvh_mesh_build(cudaStream_t s, const float* v, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n,
                     int m, void* scratch, PhaseTimer& ph, int64_t* n_nodes, const uint32_t** order);
-int lbvh_mesh_emit(cudaStream_t s, int64_t n, int m, void* scratch, void* nodes);
+// Interior offsets are shifted by node_shift and leaf offsets by prim_shift (both 0 for an upload).
+int lbvh_mesh_emit(cudaStream_t s, int64_t n, int m, void* scratch, void* nodes, uint32_t node_shift = 0,
+                   uint32_t prim_shift = 0);

@@ -11,7 +11,7 @@ import numpy as np
 
 from . import _lib
 from .geometry import Bounds2, Point2f, Transformation, _v3, f32, perspective, scale, translate
-from .scene import DeviceMeshScene
+from .scene import CompositeScene, DeviceMeshScene
 
 
 class LanczosSincFilter:
@@ -173,6 +173,8 @@ class Context:
             raise RuntimeError(f"trace_create failed ({rc}): no usable CUDA device; there is no CPU fallback")
         self._scene = None
         self._n_nodes = 0
+        self._base = None         # the FlatScene of the last trace_scene_upload (the attach base), or None
+        self._mesh = None         # the DeviceMeshScene attached to it, or None
 
     def check(self, rc):
         if rc != 0:
@@ -201,27 +203,42 @@ class Context:
     def upload(self, scene):
         if isinstance(scene, DeviceMeshScene):
             if self._scene is not scene:
-                self._upload_mesh(scene)
+                self._scene, self._n_nodes = scene, self._mesh_call(self.lib.trace_scene_upload_mesh_device, scene)
+                self._base, self._mesh = None, None
+            return scene
+        if isinstance(scene, CompositeScene):
+            flat = scene.scene.flatten()
+            if self._base is not flat:
+                self._upload_flat(flat)
+            if self._mesh is not scene.mesh:
+                self._n_nodes = self._mesh_call(self.lib.trace_scene_attach_mesh_device, scene.mesh)
+                self._mesh = scene.mesh
+            self._scene = scene
             return scene
         flat = scene.flatten()
         if self._scene is not flat:
-            if flat.stale:
-                raise RuntimeError("this scene was refit on a context and its host nodes / vertices are stale: upload it "
-                                   "before refitting and refit every context with the same vertices, or build a new "
-                                   "BVHAccel for the moved geometry")
-            d = flat.desc()
-            self.check(self.lib.trace_scene_upload(self.h, C.byref(d)))
-            self._scene, self._n_nodes = flat, len(flat.nodes)
+            self._upload_flat(flat)
         return flat
 
-    def _upload_mesh(self, scene):
-        """trace_scene_upload_mesh_device: tree and scene buffers built on the GPU from the scene's device arrays"""
+    def _upload_flat(self, flat):
+        if flat.stale:
+            raise RuntimeError("this scene was refit on a context and its host nodes / vertices are stale: upload it "
+                               "before refitting and refit every context with the same vertices, or build a new "
+                               "BVHAccel for the moved geometry")
+        d = flat.desc()
+        self.check(self.lib.trace_scene_upload(self.h, C.byref(d)))
+        self._scene, self._n_nodes = flat, len(flat.nodes)
+        self._base, self._mesh = flat, None
+
+    def _mesh_call(self, fn, scene):
+        """trace_scene_upload_mesh_device / trace_scene_attach_mesh_device of a DeviceMeshScene's device arrays: -> the
+        scene's node count"""
         d, keep = scene.desc(self.device)
         import torch
         torch.cuda.current_stream(self.device).synchronize()       # the work that wrote the arrays is done
         n_nodes = C.c_int64()
-        self.check(self.lib.trace_scene_upload_mesh_device(self.h, C.byref(d), C.byref(n_nodes)))
-        self._scene, self._n_nodes = scene, n_nodes.value
+        self.check(fn(self.h, C.byref(d), C.byref(n_nodes)))
+        return n_nodes.value
 
     def refit(self, scene, vertices=None, normals=None):
         """Move the triangles of the scene uploaded to this context and refit its tree on the GPU (trace_scene_refit):
@@ -233,8 +250,18 @@ class Context:
         `normals` (same layout and kind as `vertices`, or None to keep the current ones) apply to triangles uploaded
         with normals.  Afterwards the host FlatScene's nodes are stale: it cannot be uploaded to another context.
         A DeviceMeshScene: `vertices` in its triangle order; None re-reads the scene's own tensors (vertices, and
-        normals if it has them) after the caller changed them in place."""
-        if isinstance(scene, DeviceMeshScene):
+        normals if it has them) after the caller changed them in place.
+        A CompositeScene: `vertices` (required) of all triangles, the environment's (in the order of its flattening)
+        followed by the mesh's; afterwards the environment's FlatScene is stale as above."""
+        if isinstance(scene, CompositeScene):
+            flat = scene.scene.flatten() if scene.scene._flat is not None else None
+            if flat is None or flat is not self._base or scene.mesh is not self._mesh:
+                raise ValueError("refit: this scene is not the one uploaded to this context")
+            if vertices is None:
+                raise ValueError("refit: a CompositeScene needs the vertices of all its triangles")
+            n = len(flat.tri_vertices) + scene.mesh.n_tris
+            sb = np.ascontiguousarray(flat.sphere_bounds, dtype=np.float32)
+        elif isinstance(scene, DeviceMeshScene):
             if scene is not self._scene:
                 raise ValueError("refit: this scene is not the one uploaded to this context")
             flat, n, sb = None, scene.n_tris, np.zeros((0, 6), np.float32)

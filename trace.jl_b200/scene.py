@@ -579,6 +579,34 @@ class DeviceMeshScene:
         return d, (mats, lights)
 
 
+class CompositeScene:
+    """A Scene (the environment) with a DeviceMeshScene attached to it (extension: the reference has no counterpart).
+    Context.upload uploads `scene` once and attaches `mesh` on the GPU (trace_scene_attach_mesh_device): each new mesh
+    rebuilds only the mesh's tree, whatever the environment holds (analytic spheres, nested BVHAccels, a reference or
+    sah tree).  The device scene is the one Scene(lights, BVHAccel) uploads when its root has the environment's tree as
+    first child and the mesh's as second: the mesh's triangles come after the environment's (queries report mesh
+    triangle i as the environment's primitive count + i), its materials and lights after the environment's.
+
+    Context.upload caches by identity: the environment is uploaded again only when its flattening changed, the mesh is
+    attached again only when `mesh` is a new object.  To move triangles use Context.refit with the vertices of all
+    triangles, the environment's first."""
+
+    def __init__(self, scene, mesh):
+        if not isinstance(scene, Scene):
+            raise ValueError(f"scene must be a Scene, got {type(scene).__name__}")
+        if not isinstance(mesh, DeviceMeshScene):
+            raise ValueError(f"mesh must be a DeviceMeshScene, got {type(mesh).__name__}")
+        if mesh.n_tris == 0:
+            raise ValueError("mesh must hold at least one triangle")
+        self.scene, self.mesh = scene, mesh
+        self.lights = scene.lights + mesh.lights
+        self.bound = scene.bound.union(mesh.bound)
+
+    @property
+    def has_unshaded(self):
+        return self.scene.flatten().has_unshaded
+
+
 class FlatScene:
     """The POD upload (trace_scene_desc): BVH nodes with nested BVHAccel primitives spliced in place, the BVH-ordered
     primitive list, triangle / sphere arrays, materials and lights."""
