@@ -127,7 +127,7 @@ enum { TRACE_K_EXTEND = 0, TRACE_K_SHADOW = 1, TRACE_K_GENERATE = 2, TRACE_K_SHA
 typedef struct trace_stats {
     uint64_t rays_extend;        /* rays through closest-hit traversal */
     uint64_t rays_shadow;        /* rays through any-hit traversal */
-    uint64_t nodes_visited;      /* only counted when option "count_nodes" is 1 */
+    uint64_t nodes_visited;      /* only counted when option "count_nodes" is 1 or 2 */
     uint64_t prims_tested;
     uint64_t kernel_launches;    /* launches of this library's kernels since the last reset */
     double   ms_extend;          /* CUDA-event time in closest-hit kernels (option "time_kernels") */
@@ -196,12 +196,17 @@ const char* trace_last_error(const trace_ctx* ctx);
  *          pushed with its entry distance; same hits bit for bit), 0 = one node per step exactly as
  *          src/accel/bvh.jl:221-257; "leaf_wait" 0/4/8/16/32 warp-synchronous variant of loop 0 with batched leaf
  *          tests (measured slower, kept for the record); "film_mode" see trace_comm_init; "persist" 0/1
- *          persistent-warp traversal kernels (default 0); "count_nodes" 0/1; "time_kernels" 0/1 (per-launch CUDA
+ *          persistent-warp traversal kernels (default 0); "count_nodes" 0/1/2 (2: closest hits count the
+ *          "hit_tree" walk the default path runs, 1: the reference tree's walk); "time_kernels" 0/1 (per-launch CUDA
  *          events; with TRACE_CUDA_TIMELINE=<file> they are also dumped); "shadow_tree" 0/1 (default 1): any-hit queries
  *          (trace_occluded*, Whitted and SPPM shadow rays) walk the scene's shadow tree, an LBVH built on the device at
  *          upload, and check every occluder they find against the reference tree: the same answers bit for bit, 0 =
  *          walk the reference tree only (it applies with "slab" 2 and "walk" 1; a scene uploaded with 0 gets no shadow
- *          tree, which saves its 64 B per primitive); "rank"/"world" shard selection (Whitted: tiles
+ *          tree, which saves its 64 B per primitive); "hit_tree" 0/1 (default 1): closest-hit queries
+ *          (trace_intersect*, Whitted and SPPM camera and photon rays) walk the shadow tree too and answer only when an
+ *          exact check proves the reference walk returns the same primitive, else they run that walk: the same hits,
+ *          t and barycentrics bit for bit, 0 = walk the reference tree only (it applies where "shadow_tree" does, and
+ *          "shadow_tree" 0 turns it off as well); "rank"/"world" shard selection (Whitted: tiles
  *          k % world; SPPM: image rows and, through the photon range arguments, photons). */
 int         trace_set_option(trace_ctx* ctx, const char* key, int64_t value);
 int         trace_get_stats(trace_ctx* ctx, trace_stats* out);
@@ -333,6 +338,9 @@ int trace_scene_shadow_tree(trace_ctx* ctx, int64_t* n_pairs, void* pairs_out);
  * check could not confirm (or had a zero, tiny or non-finite direction component), and so were answered by the
  * reference tree's walk */
 int trace_get_shadow_fallbacks(trace_ctx* ctx, uint64_t* out);
+/* closest-hit rays since the last trace_reset_stats that the shadow-tree walk ("hit_tree") did not answer itself
+ * (near tie of the two closest candidates, a check that failed, an irregular ray) and handed to the reference walk */
+int trace_get_hit_fallbacks(trace_ctx* ctx, uint64_t* out);
 
 /* ---- ray queries, host buffers. o,d: [n][3]; tmax_inout: [n] (t of the hit on return, unchanged on a miss);
  * prim_out: [n] original index + 1, 0 = miss; b0b1_out: [n][2] barycentrics (triangles) or 0; may be NULL. ---- */

@@ -106,6 +106,7 @@ SIGNATURES = {
     "trace_scene_copy_nodes": (C.c_int, [_P, _P]),
     "trace_scene_shadow_tree": (C.c_int, [_P, C.POINTER(C.c_int64), _P]),
     "trace_get_shadow_fallbacks": (C.c_int, [_P, C.POINTER(C.c_uint64)]),
+    "trace_get_hit_fallbacks": (C.c_int, [_P, C.POINTER(C.c_uint64)]),
     "trace_intersect": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P]),
     "trace_occluded": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P]),
     "trace_intersect_device": (C.c_int, [_P, _P, _P, C.c_int64, _P]),

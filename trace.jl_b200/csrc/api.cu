@@ -8,7 +8,7 @@
 // ------------------------------------------------------------------ kernels: batch closest-hit / any-hit queries
 // One thread per ray, persistent grid-stride loop (grid = multiple of the SM count).  Rays come as two float4 arrays
 // {o.xyz, t_max} and {d.xyz, -}; the closest-hit result is one float4 {t, original+1 (bits), b0, b1}.
-template <int SLAB, bool COUNT, int WAIT>
+template <int SLAB, bool COUNT, int WAIT, bool TREE>       // TREE: walk the shadow tree (traverse_closest)
 __global__ void __launch_bounds__(128, 8) k_intersect(DeviceScene sc, const float4* __restrict__ ro, const float4* __restrict__ rd,
                                                    long long n, float4* __restrict__ hits, unsigned long long* counters,
                                                    int* error_flag) {
@@ -18,7 +18,7 @@ __global__ void __launch_bounds__(128, 8) k_intersect(DeviceScene sc, const floa
         const bool valid = i < n;
         const float4 o = valid ? ro[i] : make_float4(0.0f, 0.0f, 0.0f, 0.0f), d = valid ? rd[i] : make_float4(1.0f, 1.0f, 1.0f, 0.0f);
         HitRecord h;
-        traverse_any<SLAB, false, COUNT, WAIT>(sc, valid, xyz(o), xyz(d), o.w, h, counters, error_flag);
+        traverse_closest<SLAB, COUNT, WAIT, TREE>(sc, valid, xyz(o), xyz(d), o.w, h, counters, error_flag);
         if (!valid) continue;
         uint32_t orig = 0;
         if (h.prim) orig = __float_as_uint(__ldg(&sc.prims[3 * (h.prim - 1) + 2]).w) + 1u;
@@ -125,7 +125,7 @@ extern "C" int trace_set_option(trace_ctx* c, const char* key, int64_t v) {
     if (!c || !key) return 1;
     if (!strcmp(key, "slab")) { if (v < 0 || v > 2) return c->fail("slab must be 0 (literal), 1 (textbook) or 2 (guarded)"); c->slab = (int)v; }
     else if (!strcmp(key, "batch")) { if (v < 1024) return c->fail("batch too small"); c->batch = v; }
-    else if (!strcmp(key, "count_nodes")) c->count_nodes = v != 0;
+    else if (!strcmp(key, "count_nodes")) { if (v < 0 || v > 2) return c->fail("count_nodes must be 0, 1 (closest hits on the reference tree) or 2 (the walks the default path runs)"); c->count_nodes = (int)v; }
     else if (!strcmp(key, "persist")) { if (v != 0) return c->fail("persist: the dynamic-ray-fetch kernels were measured slower in both rounds and removed (profiles/r2_experiments.md)"); }
     else if (!strcmp(key, "film_mode")) { if (v != 0 && v != 1) return c->fail("film_mode must be 0 (whole film on rank 0) or 1 (one band per rank)"); c->film_mode = (int)v; }
     else if (!strcmp(key, "film_p2p")) { c->film_p2p = v != 0; }
@@ -138,6 +138,7 @@ extern "C" int trace_set_option(trace_ctx* c, const char* key, int64_t v) {
     else if (!strcmp(key, "cap_percent")) { if (v < 100 || v > 1600) return c->fail("cap_percent must be in [100, 1600]"); c->cap_percent = (int)v; }
     else if (!strcmp(key, "time_kernels")) c->time_kernels = v != 0;
     else if (!strcmp(key, "shadow_tree")) c->shadow_tree = v != 0;
+    else if (!strcmp(key, "hit_tree")) c->hit_tree = v != 0;
     else if (!strcmp(key, "graph")) c->graph = v != 0;
     else if (!strcmp(key, "sppm_lanes")) { if (v < 0 || v > trace_ctx::MAX_LANES / 2) return c->fail("sppm_lanes must be in [0, 8]"); c->sppm_lanes = (int)v; }
     else if (!strcmp(key, "sppm_chain_priority")) c->sppm_chain_priority = v != 0;
@@ -165,6 +166,7 @@ int ctx_pull_stats(trace_ctx* c) {
     c->stats.primary_rays = h[ST_PRIMARY_RAYS];
     c->stats.primary_hits = h[ST_PRIMARY_HITS];
     c->shadow_fallbacks = h[ST_SHADOW_FALLBACKS];
+    c->hit_fallbacks = h[ST_HIT_FALLBACKS];
     return 0;
 }
 
@@ -439,6 +441,14 @@ extern "C" int trace_get_shadow_fallbacks(trace_ctx* c, uint64_t* out) {
     return 0;
 }
 
+extern "C" int trace_get_hit_fallbacks(trace_ctx* c, uint64_t* out) {
+    if (!c || !out) return 1;
+    cudaSetDevice(c->device);
+    if (ctx_pull_stats(c)) return 1;
+    *out = c->hit_fallbacks;
+    return 0;
+}
+
 // ------------------------------------------------------------------ film / camera helpers shared with the integrators
 void ctx_device_camera(const trace_camera* cam, DeviceCamera* out) {
     memcpy(out->r2c, cam->raster_to_camera, sizeof(out->r2c));
@@ -473,9 +483,13 @@ static int launch_intersect(trace_ctx* c, const float4* ro, const float4* rd, in
     unsigned long long* cnt = ctx_stats64(c) + ST_NODES;
     const int grid = (int)std::min<int64_t>((n + 127) / 128, (int64_t)persistent_grid(c, 16));
     if (c->time_kernels) cudaEventRecord(c->evk0, c->stream);
+    const DeviceScene sc = hit_launch_scene(c, c->scene);
     trav_dispatch(c, [&](auto S, auto C_, auto W) {
-        auto k = k_intersect<decltype(S)::value, decltype(C_)::value, decltype(W)::value>;
-        k<<<std::min(grid, occupancy_grid(c, k, 128)), 128, 0, c->stream>>>(c->scene, ro, rd, n, hits, cnt, err);
+        constexpr int s = decltype(S)::value, w = decltype(W)::value;
+        constexpr bool cn = decltype(C_)::value;
+        auto k = k_intersect<s, cn, w, false>;
+        if constexpr (shadow_walk_capable<s, cn, w>) if (sc.shadow_pairs) k = k_intersect<s, cn, w, true>;
+        k<<<std::min(grid, occupancy_grid(c, k, 128)), 128, 0, c->stream>>>(sc, ro, rd, n, hits, cnt, err);
     });
     if (c->time_kernels) cudaEventRecord(c->evk1, c->stream);
     TR_CUDA(c, cudaGetLastError());

@@ -87,7 +87,7 @@ struct trace_ctx {
     // options
     int slab = 2;                 // 0 literal reference slab test, 1 textbook (not hit-equivalent), 2 guarded (default)
     int64_t batch = 1 << 26;      // camera samples per wavefront batch (queues: ~350 B per sample, allocated for min(batch, work))
-    int count_nodes = 0;
+    int count_nodes = 0;          // counting pass: 1 counts closest hits on the reference tree (a tree's quality), 2 the hit_tree walk
     int cap_percent = 200;        // ray-queue capacity per bounce level, in % of the batch size
     int persist = 0;              // dynamic ray fetch in the traversal kernels: 0 off, 1 bounce levels >= 2 and shadow rays, 2 all
     int sppm_path = 0;            // SPPM: bounce levels the fused path kernel carries before handing over to the wavefront queues (0: none)
@@ -97,6 +97,7 @@ struct trace_ctx {
     int leaf_wait = -1;           // walk selector: -1 pair nodes (default, option "walk" 1), 0 the reference loop ("walk" 0), 4/8/16/32 batched leaves
     int time_kernels = 0;
     int shadow_tree = 1;          // any-hit queries walk the scene's shadow tree (traverse_shadow) when it has one; 0 = the reference tree only
+    int hit_tree = 1;             // closest-hit queries walk the shadow tree too (traverse_closest_tree); 0 = the reference tree only
     int rank = 0, world = 1;
     void* comm = nullptr;         // ncclComm_t of this rank (comm.cpp), null until trace_comm_init
     int nccl_version = 0;
@@ -178,6 +179,7 @@ struct trace_ctx {
 
     trace_stats stats{};
     unsigned long long shadow_fallbacks = 0;   // any-hit rays the shadow walk handed to the reference walk (trace_get_shadow_fallbacks)
+    unsigned long long hit_fallbacks = 0;      // closest-hit rays the shadow-tree walk handed to the reference walk (trace_get_hit_fallbacks)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, evk0 = nullptr, evk1 = nullptr;
     // per-launch CUDA-event timing of the traversal kernels (option "time_kernels"), resolved after a stream sync
     struct KernelEvent { cudaEvent_t a, b; int kind, lane; };
@@ -241,9 +243,10 @@ struct trace_ctx {
     } while (0)
 
 // u64 device stats block layout (ctx->b_counters, after the int counters)
-enum { ST_RAYS_EXTEND = 0, ST_RAYS_SHADOW = 1, ST_NODES = 2, ST_PRIMS = 3, ST_DEPOSITS = 4, ST_CANDIDATES = 5, ST_REQUESTS = 6, ST_GRID_ITEMS = 7, ST_PRIMARY_RAYS = 8, ST_PRIMARY_HITS = 9, ST_SHADOW_FALLBACKS = 10, ST_COUNT = 12 };
-// the traversal kernels get `counters` = stats + ST_NODES; the shadow walk counts its fallbacks at this offset from it
+enum { ST_RAYS_EXTEND = 0, ST_RAYS_SHADOW = 1, ST_NODES = 2, ST_PRIMS = 3, ST_DEPOSITS = 4, ST_CANDIDATES = 5, ST_REQUESTS = 6, ST_GRID_ITEMS = 7, ST_PRIMARY_RAYS = 8, ST_PRIMARY_HITS = 9, ST_SHADOW_FALLBACKS = 10, ST_HIT_FALLBACKS = 11, ST_COUNT = 12 };
+// the traversal kernels get `counters` = stats + ST_NODES; the shadow-tree walks count their fallbacks at these offsets from it
 static_assert(ST_SHADOW_FALLBACKS - ST_NODES == 8, "TR_COUNTER_SHADOW_FALLBACKS (traverse.cuh)");
+static_assert(ST_HIT_FALLBACKS - ST_NODES == 9, "TR_COUNTER_HIT_FALLBACKS (traverse.cuh)");
 static const int TR_INT_COUNTERS = 128;    // ints at the start of b_counters (64..127: work counters of persistent launches)
 // int counter slots: [1 .. TR_MAX_DEPTH] ray-queue length per bounce level, [32] shadow / deposit-request queue
 enum { IC_OVERFLOW = 60, IC_ERROR = 61, IC_OVERFLOW_SHADOW = 62, IC_OVERFLOW_DEPOSIT = 63 };
@@ -316,6 +319,13 @@ static void trav_dispatch(const trace_ctx* c, F f) {
 // (the walk it falls back to, and the guard its admission test relies on)
 inline DeviceScene shadow_launch_scene(const trace_ctx* c, DeviceScene sc) {
     if (!(c->shadow_tree && c->slab == 2 && c->leaf_wait == -1 /* TR_WALK_PAIR */)) sc.shadow_pairs = nullptr;
+    return sc;
+}
+// ... and as a closest-hit launch sees it (traverse_closest_tree): the same, with option hit_tree on and not in a
+// count_nodes 1 pass, which counts the reference tree's walk
+inline DeviceScene hit_launch_scene(const trace_ctx* c, DeviceScene sc) {
+    sc = shadow_launch_scene(c, sc);
+    if (!c->hit_tree || c->count_nodes == 1) sc.shadow_pairs = nullptr;
     return sc;
 }
 

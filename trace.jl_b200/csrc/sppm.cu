@@ -207,7 +207,7 @@ static __device__ __noinline__ bool cam_vertex(const SppmLaunch& L, int level, f
 static __device__ __noinline__ bool cam_first_ray(const SppmLaunch& L, int st, int& pix, float3& o, float3& d) {
     return cam_generate_ray(L, st, pix, o, d);
 }
-template <int SLAB, bool COUNT, int WAIT>
+template <int SLAB, bool COUNT, int WAIT, bool TREE>       // TREE: walk the shadow tree (traverse_closest)
 __global__ void __launch_bounds__(128, TR_PATH_MIN_BLOCKS) k_sppm_cam_path(const __grid_constant__ SppmLaunch L, int path_levels, int* error_flag) {
     const unsigned full = 0xffffffffu;
     const int lane = threadIdx.x & 31;
@@ -222,7 +222,7 @@ __global__ void __launch_bounds__(128, TR_PATH_MIN_BLOCKS) k_sppm_cam_path(const
             __syncwarp();                                         // reconverge before the walk (see k_wh_primary)
             if (!__any_sync(full, alive)) break;
             HitRecord h;
-            traverse_any<SLAB, false, COUNT, WAIT>(L.sc, alive, o, d, TR_INF, h, L.stats + ST_NODES, error_flag);
+            traverse_closest<SLAB, COUNT, WAIT, TREE>(L.sc, alive, o, d, TR_INF, h, L.stats + ST_NODES, error_flag);
             if (alive) {
                 n_rays++;
                 alive = h.prim != 0u && cam_vertex(L, level, make_float4(h.t, __uint_as_float(h.prim), h.b0, h.b1), o, d, beta, st, pix);
@@ -504,7 +504,7 @@ static __device__ __noinline__ bool photon_vertex(const SppmLaunch& L, int level
 static __device__ __noinline__ bool photon_first_ray(const SppmLaunch& L, int j, float3& o, float3& d, float3& beta) {
     return photon_generate_ray(L, j, o, d, beta);
 }
-template <int SLAB, bool COUNT, int WAIT>
+template <int SLAB, bool COUNT, int WAIT, bool TREE>       // TREE: walk the shadow tree (traverse_closest)
 __global__ void __launch_bounds__(128, TR_PATH_MIN_BLOCKS) k_photon_path(const __grid_constant__ SppmLaunch L, int path_levels, int* error_flag) {
     const unsigned full = 0xffffffffu;
     const int lane = threadIdx.x & 31;
@@ -519,7 +519,7 @@ __global__ void __launch_bounds__(128, TR_PATH_MIN_BLOCKS) k_photon_path(const _
             __syncwarp();
             if (!__any_sync(full, alive)) break;
             HitRecord h;
-            traverse_any<SLAB, false, COUNT, WAIT>(L.sc, alive, o, d, TR_INF, h, L.stats + ST_NODES, error_flag);
+            traverse_closest<SLAB, COUNT, WAIT, TREE>(L.sc, alive, o, d, TR_INF, h, L.stats + ST_NODES, error_flag);
             if (alive) {
                 n_rays++;
                 alive = h.prim != 0u && photon_vertex(L, level, make_float4(h.t, __uint_as_float(h.prim), h.b0, h.b1), o, d, beta, lum0, j);
@@ -896,8 +896,13 @@ static int sppm_camera_lane(trace_ctx* c, SppmState* s, int l, int iteration) {
         // all bounce levels of the camera paths in ONE launch (k_sppm_cam_path); rays are counted by the kernel itself
         c->kev_begin(TRACE_K_EXTEND);
         trav_dispatch(c, [&](auto S, auto C_, auto Wk) {
-            auto k = k_sppm_cam_path<decltype(S)::value, decltype(C_)::value, decltype(Wk)::value>;
-            k<<<occupancy_grid(c, k, 128), 128, 0, st>>>(W, c->sppm_path, W.flags + IC_ERROR);
+            constexpr int s_ = decltype(S)::value, w_ = decltype(Wk)::value;
+            constexpr bool cn = decltype(C_)::value;
+            SppmLaunch P = W;
+            P.sc = hit_launch_scene(c, W.sc);
+            auto k = k_sppm_cam_path<s_, cn, w_, false>;
+            if constexpr (shadow_walk_capable<s_, cn, w_>) if (P.sc.shadow_pairs) k = k_sppm_cam_path<s_, cn, w_, true>;
+            k<<<occupancy_grid(c, k, 128), 128, 0, st>>>(P, c->sppm_path, W.flags + IC_ERROR);
         });
         c->kev_end();
         c->stats.kernel_launches++;
@@ -1022,8 +1027,13 @@ static int sppm_trace_lane(trace_ctx* c, SppmState* s, int j, int iteration, int
     if (c->sppm_path && c->slab != 1) {
         c->kev_begin(TRACE_K_EXTEND);
         trav_dispatch(c, [&](auto S, auto C_, auto Wk) {
-            auto k = k_photon_path<decltype(S)::value, decltype(C_)::value, decltype(Wk)::value>;
-            k<<<occupancy_grid(c, k, 128), 128, 0, st>>>(W, c->sppm_path, W.flags + IC_ERROR);
+            constexpr int s_ = decltype(S)::value, w_ = decltype(Wk)::value;
+            constexpr bool cn = decltype(C_)::value;
+            SppmLaunch P = W;
+            P.sc = hit_launch_scene(c, W.sc);
+            auto k = k_photon_path<s_, cn, w_, false>;
+            if constexpr (shadow_walk_capable<s_, cn, w_>) if (P.sc.shadow_pairs) k = k_photon_path<s_, cn, w_, true>;
+            k<<<occupancy_grid(c, k, 128), 128, 0, st>>>(P, c->sppm_path, W.flags + IC_ERROR);
         });
         c->kev_end();
         c->stats.kernel_launches++;

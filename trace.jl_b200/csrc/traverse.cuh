@@ -117,9 +117,10 @@ __device__ __forceinline__ bool slab_test(const float4 n0, const float4 n1, cons
     return tx_min < tmax && tx_max > 0.0f;
 }
 
-// Watertight triangle test. a, b, c are the primitive record's float4s (xyz = vertices).
+// Watertight triangle test. a, b, c are the primitive record's float4s (xyz = vertices).  ts_out: the scaled distance
+// ts (t_hit = ts * (1 / det)), which traverse_closest_tree needs for its ulp argument.
 __device__ __forceinline__ bool triangle_test(const float4 a, const float4 b, const float4 c, const RayPrep& r, float tmax,
-                                              float& t_hit, float& b0, float& b1, float& b2) {
+                                              float& t_hit, float& b0, float& b1, float& b2, float& ts_out) {
     float X0, Y0, Z0, X1, Y1, Z1, X2, Y2, Z2;
     {
         float qx = a.x - r.o.x, qy = a.y - r.o.y, qz = a.z - r.o.z;     // (v - o), then permuted
@@ -156,7 +157,13 @@ __device__ __forceinline__ bool triangle_test(const float4 a, const float4 b, co
     float inv_det = 1.0f / det;
     b0 = e0 * inv_det; b1 = e1 * inv_det; b2 = e2 * inv_det;
     t_hit = ts * inv_det;
+    ts_out = ts;
     return true;
+}
+__device__ __forceinline__ bool triangle_test(const float4 a, const float4 b, const float4 c, const RayPrep& r, float tmax,
+                                              float& t_hit, float& b0, float& b1, float& b2) {
+    float ts;
+    return triangle_test(a, b, c, r, tmax, t_hit, b0, b1, b2, ts);
 }
 
 struct SphereHitInfo { float t; float3 p; float phi; };
@@ -603,6 +610,137 @@ __device__ __forceinline__ bool traverse_shadow(const DeviceScene& sc, float3 o,
     return shadow_fallback<COUNT>(sc, o, d, tmax, counters, error_flag);
 }
 
+// ------------------------------------------------------------------ closest-hit walk on the shadow tree
+// The reference's closest hit depends on its visit order only when two candidates lie within rounding of each other
+// (ties, t_max updates that round up).  traverse_closest_tree finds the closest hit on the shadow tree, which costs
+// about half the box tests of the reference tree, and answers only when it can prove that the reference walk
+// (traverse_pair<2, false>) returns the same primitive; every other ray gets that walk's own answer.
+// With band = 2^-18 (TR_HIT_BAND_UP = 1 + band) and t_max0 the ray's t_max:
+//   walk       bound B = min(t_max0, rn(t1 * (1 + band))), t1 the smallest candidate t so far (B never grows).  Every pair
+//              fetch tests both children with traverse_shadow's guard, its t_max term taken at B; the nearer admitted
+//              child (guard entry) is entered, the farther pushed as {ref, entry} and dropped on pop if its entry is
+//              past B + |B| TR_GUARD_REL.  No early exit.
+//   candidate  a primitive passing triangle_test(r, B).  P is the candidate of smallest t (t1), t2 the smallest t of
+//              any other.  A candidate with a non-finite t, or with |ts| <= FLT_MIN, sets t2 = -inf (see step 3).
+//   confirm    answer P (t, b0, b1 recomputed: they do not depend on t_max) iff the ray is regular (below), t1 >= 2^-100,
+//              B < t_max0 (so B = rn(t1 (1 + band))), t2 > B, and with L = rn(B (1 - 2^-22)): triangle_test(P, L) passes
+//              and P's vertex box textbook-accepts with t_enter < L.
+//   end        no candidate: a miss; otherwise hit_fallback (the reference walk, counted).
+// Why this is the reference's answer (u = 2^-24; det > 0 shown, det < 0 is the mirror image):
+//   0. triangle_test passes at t_max iff some conditions independent of t_max hold and ts <= rn(t_max det): monotone
+//      in t_max.  If ts > rn(x) for floats, then ts > x exactly (ts is at least the float after rn(x)).  Regular: a
+//      finite origin, finite non-zero 1/d, and the origin and the reference root box within 2^56 - then every |det|
+//      is < 2^120, so rn(1 / det) is a normal number (error <= u) or +inf.
+//   1. Every primitive Q passing triangle_test(Q, B_final) is a candidate.  It passes at every B the walk held, and
+//      the guarded reference walk already relies on the guard (at the same t_max) never rejecting a box that holds
+//      the vertices of a triangle passing triangle_test; shadow-tree boxes are unions of vertex boxes.  So all its
+//      ancestors are admitted and not dropped on pop.  Likewise with no candidate the reference accepts nothing.
+//   2. The reference reaches and accepts P.  Every t_max it holds before it tests P is >= L: t_max0 > B; a candidate
+//      Q != P has t >= t2 > B; any other accepted Q fails at B (step 1), so ts > B det exactly (step 0) and
+//      t = rn(ts rn(1/det)) >= B (1 - u)^2 >= L, or t = +inf.  P's vertex box textbook-accepts with entry < L, so, as
+//      in traverse_shadow, every reference ancestor box accepts with tx_min < L <= t_max (neither the far-child cull
+//      nor the pop test drops it), and triangle_test(P, L) passing means it passes at every t_max >= L.
+//   3. After P (t_max = t1) nothing is accepted.  A Q != P passing at t1 passes at B >= t1, so it is a candidate with
+//      t > B >= t1 (1 + band)(1 - u), finite and |ts| > FLT_MIN.  Then ts rn(1/det) > B, so ts > B det / (1 + u) >
+//      t1 det (1 + 60 u), while passing needs ts <= rn(t1 det) <= t1 det (1 + u) - unless t1 det is subnormal, where
+//      |ts| <= FLT_MIN.  Contradiction: the reference's last accepted primitive is P, with P's t, b0, b1.
+// Deviation, as traverse_shadow's: a reference-tree stack overflow is reported only when the fallback runs.
+#define TR_COUNTER_HIT_FALLBACKS 9         // offset of ST_HIT_FALLBACKS from `counters` (context.hpp)
+#define TR_HIT_BAND_UP 0x1.00004p0f        // 1 + 2^-18
+#define TR_HIT_LOWER 0x1.fffff8p-1f        // 1 - 2^-22
+#define TR_HIT_T_MIN 0x1p-100f
+#define TR_HIT_REACH 0x1p56f
+
+// kept out of line, as shadow_fallback
+template <bool COUNT>
+static __device__ __noinline__ HitRecord hit_fallback(const DeviceScene sc, float3 o, float3 d, float tmax,
+                                                      unsigned long long* counters, int* error_flag) {
+    if (counters) atomicAdd(&counters[TR_COUNTER_HIT_FALLBACKS], 1ull);
+    HitRecord h;
+    traverse_pair<2, false, COUNT>(sc, o, d, tmax, h, counters, error_flag);
+    return h;
+}
+
+template <bool COUNT>
+__device__ __forceinline__ bool traverse_closest_tree(const DeviceScene& sc, float3 o, float3 d, float tmax, HitRecord& out,
+                                                      unsigned long long* counters, int* error_flag) {
+    const RayPrep r = prepare_ray(o, d, sc.scene_scale);
+    bool regular = (fabsf(o.x) <= TR_HIT_REACH) & (fabsf(o.y) <= TR_HIT_REACH) & (fabsf(o.z) <= TR_HIT_REACH) &
+                   isfinite(r.inv.x) & isfinite(r.inv.y) & isfinite(r.inv.z) &
+                   (r.inv.x != 0.0f) & (r.inv.y != 0.0f) & (r.inv.z != 0.0f);
+    {   // the reference root box holds every vertex the reference can test
+        const float4 n0 = __ldg(&sc.nodes[0]), n1 = __ldg(&sc.nodes[1]);
+        regular &= (fabsf(n0.x) <= TR_HIT_REACH) & (fabsf(n0.y) <= TR_HIT_REACH) & (fabsf(n0.z) <= TR_HIT_REACH) &
+                   (fabsf(n0.w) <= TR_HIT_REACH) & (fabsf(n1.x) <= TR_HIT_REACH) & (fabsf(n1.y) <= TR_HIT_REACH);
+    }
+    if (regular) {
+        uint2 stack[TR_STACK_SIZE];
+        int sp = 0;
+        uint32_t item = 0;                  // the root: pair 0
+        unsigned n_nodes = 0, n_prims = 0;
+        float bound = tmax, t1 = TR_INF, t2 = TR_INF;
+        uint32_t best = 0;
+        for (;;) {
+            if (item & TR_REF_LEAF) {
+                const uint32_t pi = item & TR_REF_INDEX_MASK;
+                const float4 a = __ldg(&sc.prims[3 * pi]);
+                if (COUNT) n_prims++;
+                if ((__float_as_uint(a.w) & ~TR_PRIM_LAST_BIT) == 0u) {        // degenerate triangles never hit
+                    const float4 b = __ldg(&sc.prims[3 * pi + 1]), c = __ldg(&sc.prims[3 * pi + 2]);
+                    float t, b0, b1, b2, ts;
+                    if (triangle_test(a, b, c, r, bound, t, b0, b1, b2, ts)) {
+                        if (!(fabsf(t) < TR_INF) | !(fabsf(ts) > 0x1p-126f)) t2 = -TR_INF;
+                        else if (t < t1) { t2 = fminf(t2, t1); t1 = t; best = pi + 1; bound = fminf(tmax, t * TR_HIT_BAND_UP); }
+                        else t2 = fminf(t2, t);
+                    }
+                }
+            } else {
+                const float4* np = sc.shadow_pairs + 4u * item;
+                const float4 q0 = __ldg(np), q1 = __ldg(np + 1), q2 = __ldg(np + 2), q3 = __ldg(np + 3);
+                if (COUNT) n_nodes += 2;
+                float e0, x0, e1, x1;
+                slab_interval(q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, r, r.mx, r.my, r.mz, e0, x0);
+                slab_interval(q2.x, q2.y, q2.z, q2.w, q3.x, q3.y, r, r.mx, r.my, r.mz, e1, x1);
+                const float bound_guard = bound + fabsf(bound) * TR_GUARD_REL;     // slab_test<2>'s t_max term at B
+                const bool in0 = !((e0 > x0) | (x0 < 0.0f) | (e0 > bound_guard));
+                const bool in1 = !((e1 > x1) | (x1 < 0.0f) | (e1 > bound_guard));
+                const uint32_t ref0 = __float_as_uint(q1.z), ref1 = __float_as_uint(q3.z);
+                if (in0 & in1) {
+                    const bool second_first = e1 < e0;
+                    stack[sp++] = second_first ? make_uint2(ref0, __float_as_uint(e0)) : make_uint2(ref1, __float_as_uint(e1));
+                    item = second_first ? ref1 : ref0;
+                    continue;
+                }
+                if (in0 | in1) { item = in0 ? ref0 : ref1; continue; }
+            }
+            for (;;) {                      // pop the next pending child that B still admits
+                if (sp == 0) goto walked;
+                const uint2 e = stack[--sp];
+                item = e.x;
+                if (!(__uint_as_float(e.y) > bound + fabsf(bound) * TR_GUARD_REL)) break;
+            }
+        }
+    walked:
+        if (COUNT && counters) { atomicAdd(&counters[0], (unsigned long long)n_nodes); atomicAdd(&counters[1], (unsigned long long)n_prims); }
+        if (best == 0 && t2 > 0.0f) { out.prim = 0; out.t = tmax; out.b0 = 0.0f; out.b1 = 0.0f; return false; }
+        if ((best != 0) & (t1 >= TR_HIT_T_MIN) & (bound < tmax) & (t2 > bound)) {
+            const float lower = bound * TR_HIT_LOWER;
+            const uint32_t pi = best - 1;
+            const float4 a = __ldg(&sc.prims[3 * pi]), b = __ldg(&sc.prims[3 * pi + 1]), c = __ldg(&sc.prims[3 * pi + 2]);
+            float t, b0, b1, b2, t_enter, t_exit;
+            slab_interval(fminf(fminf(a.x, b.x), c.x), fminf(fminf(a.y, b.y), c.y), fminf(fminf(a.z, b.z), c.z),
+                          fmaxf(fmaxf(a.x, b.x), c.x), fmaxf(fmaxf(a.y, b.y), c.y), fmaxf(fmaxf(a.z, b.z), c.z), r,
+                          0.0f, 0.0f, 0.0f, t_enter, t_exit);
+            if (triangle_test(a, b, c, r, lower, t, b0, b1, b2) & (t_enter <= t_exit) & (t_exit > 0.0f) & (t_enter < lower)) {
+                out.prim = best; out.t = t; out.b0 = b0; out.b1 = b1;
+                return true;
+            }
+        }
+    }
+    out = hit_fallback<COUNT>(sc, o, d, tmax, counters, error_flag);
+    return out.prim != 0u;
+}
+
 // ------------------------------------------------------------------ warp-synchronous traversal with batched leaves
 // Same walk, same order, same tests as traverse<>() per ray - only WHEN a lane runs the primitive tests of a leaf changes.
 // In the plain loop a warp executes the ~120-instruction triangle test whenever ANY of its lanes stands on a leaf;
@@ -698,5 +836,17 @@ __device__ __forceinline__ bool traverse_any(const DeviceScene& sc, bool valid, 
         if (WAIT == TR_WALK_PAIR) return traverse_pair<SLAB == 1 ? 0 : SLAB, ANY, COUNT>(sc, o, d, tmax, out, counters, error_flag);
         return traverse<SLAB, ANY, COUNT>(sc, o, d, tmax, out, counters, error_flag);
     } else return traverse_lb<SLAB, ANY, COUNT, (WAIT > 0 ? WAIT : 1), TR_PARK_MAX>(sc, valid, o, d, tmax, out, counters, error_flag);
+}
+
+// closest hit of the kernels: TREE walks the shadow tree (traverse_closest_tree; the launch passes a scene that has one,
+// hit_launch_scene in context.hpp, and instantiates TREE only where shadow_walk_capable), else the dispatch above
+template <int SLAB, bool COUNT, int WAIT, bool TREE>
+__device__ __forceinline__ bool traverse_closest(const DeviceScene& sc, bool valid, float3 o, float3 d, float tmax, HitRecord& out,
+                                                 unsigned long long* counters, int* error_flag) {
+    if (TREE) {
+        if (!valid) { out.prim = 0; out.t = tmax; out.b0 = 0.0f; out.b1 = 0.0f; return false; }
+        return traverse_closest_tree<COUNT>(sc, o, d, tmax, out, counters, error_flag);
+    }
+    return traverse_any<SLAB, false, COUNT, WAIT>(sc, valid, o, d, tmax, out, counters, error_flag);
 }
 

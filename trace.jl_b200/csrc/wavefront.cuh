@@ -26,7 +26,7 @@ __device__ __forceinline__ void queue_extent(const int* count, const int* count_
     n = nf + (count_back ? min(*count_back, cap - nf) : 0);
 }
 
-template <int SLAB, bool COUNT, int WAIT>
+template <int SLAB, bool COUNT, int WAIT, bool TREE>       // TREE: walk the shadow tree (traverse_closest)
 __global__ void __launch_bounds__(128, TR_TRAV_MIN_BLOCKS) k_wh_extend(DeviceScene sc, const float4* __restrict__ ro, const float4* __restrict__ rd,
                                                    const int* __restrict__ count, const int* __restrict__ count_back, int cap,
                                                    float4* __restrict__ hits, unsigned long long* counters, int* error_flag) {
@@ -40,7 +40,7 @@ __global__ void __launch_bounds__(128, TR_TRAV_MIN_BLOCKS) k_wh_extend(DeviceSce
         const float4 o = valid ? q_load(&ro[i]) : make_float4(0.0f, 0.0f, 0.0f, 0.0f), d = valid ? q_load(&rd[i]) : make_float4(1.0f, 1.0f, 1.0f, 0.0f);
         HitRecord h;
         // closest hit; the third barycentric is rebuilt exactly in the shade stage from the winning triangle
-        traverse_any<SLAB, false, COUNT, WAIT>(sc, valid, xyz(o), xyz(d), o.w, h, counters, error_flag);
+        traverse_closest<SLAB, COUNT, WAIT, TREE>(sc, valid, xyz(o), xyz(d), o.w, h, counters, error_flag);
         if (valid) q_store(&hits[i], make_float4(h.t, __uint_as_float(h.prim), h.b0, h.b1));
     }
 }
@@ -80,11 +80,15 @@ __device__ __forceinline__ float third_barycentric(const DeviceScene& sc, uint32
     return b2;
 }
 
-template <class... Args>
-static void launch_extend_plain(trace_ctx* c, int grid, Args... args) {
+static void launch_extend_plain(trace_ctx* c, DeviceScene sc, const float4* ro, const float4* rd, const int* count,
+                                const int* count_back, int cap, float4* hits, unsigned long long* counters, int* err) {
     c->kev_begin(0);
     trav_dispatch(c, [&](auto S, auto C_, auto W) {
-        k_wh_extend<decltype(S)::value, decltype(C_)::value, decltype(W)::value><<<persistent_grid(c, 16), 128, 0, c->cur_stream>>>(args...);
+        constexpr int s = decltype(S)::value, w = decltype(W)::value;
+        constexpr bool cn = decltype(C_)::value;
+        auto k = k_wh_extend<s, cn, w, false>;
+        if constexpr (shadow_walk_capable<s, cn, w>) if (sc.shadow_pairs) k = k_wh_extend<s, cn, w, true>;
+        k<<<persistent_grid(c, 16), 128, 0, c->cur_stream>>>(sc, ro, rd, count, count_back, cap, hits, counters, err);
     });
     c->stats.kernel_launches++;
     c->kev_end();
@@ -105,7 +109,7 @@ static void launch_shadow_plain(trace_ctx* c, DeviceScene sc, const float4* so, 
 
 static void launch_extend(trace_ctx* c, int grid, DeviceScene sc, const float4* ro, const float4* rd, const int* count, int cap,
                           float4* hits, unsigned long long* counters, int* err, const int* count_back = nullptr) {
-    launch_extend_plain(c, grid, sc, ro, rd, count, count_back, cap, hits, counters, err);
+    launch_extend_plain(c, hit_launch_scene(c, sc), ro, rd, count, count_back, cap, hits, counters, err);
 }
 static void launch_shadow(trace_ctx* c, int grid, DeviceScene sc, const float4* so, const float4* sd, const float4* contrib,
                           const int* count, int cap, float4* accum, unsigned long long* counters, int* err) {

@@ -118,7 +118,8 @@ static __device__ __noinline__ bool primary_ray(const WhittedLaunch& L, int i, f
     return true;
 }
 
-template <int SLAB, int WAIT>
+// TREE: walk the shadow tree (traverse_closest); L.sc is then the launch's hit_launch_scene
+template <int SLAB, int WAIT, bool TREE>
 __global__ void __launch_bounds__(128, TR_TRAV_MIN_BLOCKS) k_wh_primary(const __grid_constant__ WhittedLaunch L, int* error_flag) {
     const int lane = threadIdx.x & 31;
     int n_active = 0;
@@ -131,7 +132,8 @@ __global__ void __launch_bounds__(128, TR_TRAV_MIN_BLOCKS) k_wh_primary(const __
         // instruction and 3x the run time without this barrier
         __syncwarp();
         HitRecord h;
-        traverse_any<SLAB, false, false, WAIT>(L.sc, valid, o, d, TR_INF, h, nullptr, error_flag);
+        // counters: only the shadow-tree walk's fallback count (COUNT is off)
+        traverse_closest<SLAB, false, WAIT, TREE>(L.sc, valid, o, d, TR_INF, h, L.stats + ST_NODES, error_flag);
         if (i < L.n_slots) {
             L.accum[i] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
             q_store(&L.hits[i], make_float4(h.t, __uint_as_float(valid ? h.prim : 0u), h.b0, h.b1));
@@ -448,8 +450,13 @@ static int run_batch(trace_ctx* c, WhittedLaunch& L, long long begin, long long 
     int* d_err = ctx_icounters_lane(c, 0) + IC_ERROR;
     if (L.fused) {
         c->kev_begin(0);
+        WhittedLaunch P = L;
+        P.sc = hit_launch_scene(c, L.sc);
         trav_dispatch(c, [&](auto S, auto C_, auto W) {
-            k_wh_primary<decltype(S)::value, decltype(W)::value><<<g_trav, 128, 0, c->cur_stream>>>(L, d_err);
+            constexpr int s = decltype(S)::value, w = decltype(W)::value;
+            auto k = k_wh_primary<s, w, false>;
+            if constexpr (shadow_walk_capable<s, false, w>) if (P.sc.shadow_pairs) k = k_wh_primary<s, w, true>;
+            k<<<g_trav, 128, 0, c->cur_stream>>>(P, d_err);
         });
         c->kev_end();
     } else { c->kev_begin(TRACE_K_GENERATE); k_wh_generate<<<g_stream, 256, 0, c->cur_stream>>>(L); c->kev_end(); }
@@ -647,7 +654,7 @@ int whitted_render_device(trace_ctx* c, const trace_camera* cam, const trace_fil
     if (c->graph && !c->time_kernels && (size_t)c->stream > 2) {       // (legacy / per-thread default streams cannot be captured)
         std::string key((const char*)lane.data(), lane.size() * sizeof(WhittedLaunch));
         key.append((const char*)b_count.data(), b_count.size() * sizeof(long long));
-        const long long extra[] = {nb, batch, K, total_slots, (long long)(size_t)d_flags, c->slab, c->persist, c->count_nodes, c->leaf_wait, c->fuse_primary, c->shadow_tree,
+        const long long extra[] = {nb, batch, K, total_slots, (long long)(size_t)d_flags, c->slab, c->persist, c->count_nodes, c->leaf_wait, c->fuse_primary, c->shadow_tree, c->hit_tree,
                                    (long long)(size_t)c->stream};
         key.append((const char*)extra, sizeof(extra));
         if (!c->wh_graph || key != c->wh_graph_key) {

@@ -330,6 +330,8 @@ class Context:
         fb = C.c_uint64()
         self.check(self.lib.trace_get_shadow_fallbacks(self.h, C.byref(fb)))
         out["shadow_fallbacks"] = fb.value
+        self.check(self.lib.trace_get_hit_fallbacks(self.h, C.byref(fb)))
+        out["hit_fallbacks"] = fb.value
         return out
 
     def reset_stats(self):
