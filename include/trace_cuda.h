@@ -8,6 +8,7 @@
  *   trace_scene_upload         <- Scene(lights, aggregate)                    src/Trace.jl:176-187
  *   trace_scene_upload_mesh_device  (extension: a triangle scene built and packed on the GPU from device arrays)
  *   trace_scene_attach_mesh_device  (extension: such a mesh attached to the uploaded scene, rebuilt alone per frame)
+ *   trace_scene_attach_meshes_device (extension: several such meshes, each rebuilt only when it changes)
  *   trace_intersect            <- intersect!(bvh|scene, ray)                  src/accel/bvh.jl:212-258, src/Trace.jl:189-191
  *   trace_occluded             <- intersect_p(bvh|scene, ray)                 src/accel/bvh.jl:260-299, src/Trace.jl:192-194
  *   trace_render_whitted       <- (i::SamplerIntegrator)(scene)               src/integrators/sampler.jl:12-56
@@ -267,36 +268,52 @@ typedef struct trace_mesh_device_desc {
 } trace_mesh_device_desc;
 int trace_scene_upload_mesh_device(trace_ctx* ctx, const trace_mesh_device_desc* mesh, int64_t* n_nodes_out);
 
-/* ---- attach a device mesh to the uploaded scene (extension: the reference has no counterpart).  The base is the scene
- * of the last trace_scene_upload or trace_scene_upload_mesh_device; each attach composes it with `mesh` (the same
- * descriptor and checks as trace_scene_upload_mesh_device), and a later attach replaces the mesh attached before it
- * while the base stays resident.  The composed device scene is bit for bit the one trace_scene_upload builds from D:
- * with the base's Nb nodes, Qb interior nodes, Pb primitives, Tb triangles, Mb materials and Lb lights and the mesh's
- * n triangles,
- *   node 0          interior, box = Julia min / max union of the base's and the mesh's root boxes, first child the
- *                   base, second child the mesh (offset 1 + Nb); split axis = the k maximising (mesh.min[k] +
- *                   mesh.max[k]) - (base.min[k] + base.max[k]) in float32, ties to the lowest k, non-finite values lose;
- *   nodes 1 .. Nb   the base's nodes in order, interior offsets + 1 (leaf offsets unchanged);
- *   the rest        the mesh's LBVH as trace_scene_upload_mesh_device builds it, interior offsets + 1 + Nb, leaf
- *                   offsets + Pb;
- *   primitives      the base's, then {TRIANGLE, Tb + order[k], Mb + tri_materials[order[k]], Pb + order[k]}: queries
- *                   report mesh triangle i as Pb + i;
- *   arrays          triangles base ++ mesh, the base's spheres, materials base ++ mesh, lights base ++ mesh
+/* ---- attach device meshes to the uploaded scene (extension: the reference has no counterpart).  The base is the scene
+ * of the last trace_scene_upload or trace_scene_upload_mesh_device; a call composes it with the meshes of k slots,
+ * each built from a descriptor (the same descriptor and checks as trace_scene_upload_mesh_device) or kept, while the
+ * base stays resident.  The composed device scene is bit for bit the one trace_scene_upload builds from D:
+ *   C(A, B)         the composition of two parts: a new root, interior, box = Julia min / max union of A's and B's
+ *                   root boxes, first child A (node 1), second child B (offset 1 + NA); split axis = the k maximising
+ *                   (B.min[k] + B.max[k]) - (A.min[k] + A.max[k]) in float32, ties to the lowest k, non-finite values
+ *                   lose; then A's nodes (interior offsets + 1), then B's (interior offsets + 1 + NA, leaf offsets +
+ *                   PA); primitives, triangles, materials and lights A's then B's, B's triangle, material and
+ *                   `original` indices shifted by A's counts;
+ *   G(lo, hi)       mesh lo when hi - lo == 1, else C(G(lo, mid), G(mid, hi)) with mid = lo + ceil((hi - lo) / 2): a
+ *                   balanced tree over the meshes in slot order, each mesh the LBVH trace_scene_upload_mesh_device
+ *                   builds (prims[k] = {TRIANGLE, order[k], tri_materials[order[k]], order[k]});
+ *   D               C(base, G(0, k)): the meshes' triangles, materials and lights follow the base's in slot order, and
+ *                   queries report triangle i of mesh j as Pb + n_0 + ... + n_{j-1} + i (Pb: the base's primitives)
  * - nodes, pair records, primitive and normal records, spheres, materials, lights, root reference, scene_scale and
- * counts alike.  The shadow tree is composed, not rebuilt: the scene has one only when both parts have one (or are a
- * single primitive), it has no spheres and 1 + max(base depth, mesh depth) <= 64.  Its pair 0 holds the two parts'
- * root boxes and references with the root's split-axis bit, then come the base's pairs (pair references + 1), then
- * the mesh's (pair references + Pb, leaf references + Pb): n_prims - 1 pairs.  Answers do not depend on the shadow
- * tree.
+ * counts alike.  A kept mesh enters D as the device holds it (with a refit's boxes and vertices).  The shadow tree is
+ * composed, not rebuilt: C composes the parts' shadow trees the same way - pair 0 holds the two parts' root boxes and
+ * references with C's split-axis bit, then A's pairs (pair references + 1), then B's (pair references + PA, leaf
+ * references + PA): n_prims - 1 pairs, applied recursively through G.  The scene has one only when every part has one
+ * (or is a single primitive), it has no spheres and the composed depth (1 + the deeper part's, per level) is at most
+ * 64.  Answers do not depend on the shadow tree.
+ * meshes[j] != NULL builds slot j from that descriptor (replacing or appending it); meshes[j] == NULL keeps the mesh
+ * in slot j, which is not rebuilt: it costs a device copy with its references rebased when its place or its shifts
+ * change, and nothing otherwise; nothing proportional to it crosses to the host.  Its shadow tree moves with it only
+ * while option shadow_tree is on; a kept mesh moved with the option off has none until it is rebuilt (the scene then
+ * has no shadow tree).  Slots from n_meshes on are dropped.  The call waits for the device a fixed number of times
+ * whatever n_meshes is (the new meshes' build statuses are read back together).
  * The first attach after an upload moves the base's node, pair and shadow-pair records up one slot (a cost
- * proportional to the base, with a transient peak of about twice those buffers); later attaches write node 0, pair 0
- * and the mesh's part only.  Refused before anything is written (the previous scene stays uploaded and usable): the
- * refusals of trace_scene_upload_mesh_device, n_tris == 0, no scene uploaded, a base without primitives, 2^30 or more
- * primitives or too many interior nodes in the composed scene.  trace_scene_refit[_device] applies as after
- * trace_scene_upload(D): its input is all Tb + n triangles in D's order.  A refit moves base triangles until the next
- * upload; the next attach reads the base's boxes from the device.  Like the uploads the call waits for all of the
- * context's work, ends any SPPM session and is synchronous; it is local to the context (every rank attaches the same
- * mesh).  *n_nodes_out (may be NULL) receives the composed node count.  TRACE_BVH_PROFILE=1 prints per-phase times. */
+ * proportional to the base, with a transient peak of about twice those buffers); later calls do not touch the base.
+ * Memory: the build scratch holds every new mesh's LBVH build at once (each as trace_scene_upload_mesh_device's) and a
+ * staging copy of the kept meshes that move; buffers only grow, so a repeated call with the same sizes allocates
+ * nothing.  Refused before anything outside the build scratch is written (the previous scene and every slot stay as
+ * they were, even when an earlier descriptor of the call was valid): the refusals of trace_scene_upload_mesh_device
+ * for each new mesh, n_tris == 0, a new or kept mesh's tree deeper than 64 - ceil(log2 n_meshes) levels, n_meshes outside
+ * [1, 64], a NULL descriptor for a slot that holds no mesh (every upload clears the slots), no scene uploaded, a base
+ * without primitives, 2^30 or more primitives or too many interior nodes in the composed scene.
+ * trace_scene_refit[_device] applies as after trace_scene_upload(D): its input is all triangles in D's order.  A
+ * refit moves base and kept-mesh triangles until the next upload or replacement; a refit of a scene without a shadow
+ * tree leaves the parts' shadow trees stale, so later calls compose none while such a part remains.  Like the uploads
+ * the call drains all of the context's work, ends any SPPM session and is synchronous; it is local to the context
+ * (every rank attaches the same meshes).  *n_nodes_out (may be NULL) receives the composed node count.
+ * TRACE_BVH_PROFILE=1 prints per-phase times and the bytes staged for kept meshes. */
+int trace_scene_attach_meshes_device(trace_ctx* ctx, int64_t n_meshes, const trace_mesh_device_desc* const* meshes,
+                                     int64_t* n_nodes_out);
+/* trace_scene_attach_meshes_device(ctx, 1, &mesh, n_nodes_out): the base with this one mesh. */
 int trace_scene_attach_mesh_device(trace_ctx* ctx, const trace_mesh_device_desc* mesh, int64_t* n_nodes_out);
 
 /* ---- refit (extension: the reference has no counterpart; it rebuilds BVHAccel).  New positions for the triangles of

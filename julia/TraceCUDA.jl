@@ -326,6 +326,26 @@ function attach_mesh_device!(ctx::Context, n_tris, vertices, normals, flags, mat
     n_nodes[]
 end
 
+# Several moving device meshes inside a static environment (trace_scene_attach_meshes_device): slot j of `meshes` is
+# `nothing` (keep the mesh in slot j, which is not rebuilt) or a NamedTuple with the arguments of upload_mesh_device!
+# (n_tris, vertices, normals, flags, material_ids, materials, lights and optionally max_node_primitives).  Afterwards
+# the environment holds exactly length(meshes) meshes (1 to 64); slots past the end are dropped.  The meshes' triangles,
+# materials and lights come after the environment's in slot order; queries report triangle i of mesh j as (the
+# environment's primitive count) + (the triangles of meshes 1 .. j - 1) + i.  Returns the composed node count.
+function attach_meshes_device!(ctx::Context, meshes::AbstractVector)
+    descs = [m === nothing ? nothing :
+             Ref(MeshDeviceDesc(m.n_tris, UInt(m.vertices), UInt(m.normals), UInt(m.flags), UInt(m.material_ids),
+                                Int32(get(m, :max_node_primitives, 1)), Int32(0), length(m.materials), pointer(m.materials),
+                                length(m.lights), pointer(m.lights))) for m in meshes]
+    n_nodes = Ref{Int64}(0)
+    GC.@preserve meshes descs begin
+        ptrs = Ptr{MeshDeviceDesc}[d === nothing ? C_NULL : Base.unsafe_convert(Ptr{MeshDeviceDesc}, d) for d in descs]
+        check(ctx, ccall((:trace_scene_attach_meshes_device, LIB), Cint, (Ptr{Cvoid}, Int64, Ptr{Ptr{MeshDeviceDesc}}, Ref{Int64}),
+                         ctx.h, length(meshes), ptrs, n_nodes))
+    end
+    n_nodes[]
+end
+
 # ---- the two functors ------------------------------------------------------------------------------------------------
 struct GPU{I<:Trace.Integrator,C}
     integrator::I

@@ -101,6 +101,7 @@ SIGNATURES = {
     "trace_scene_upload": (C.c_int, [_P, C.POINTER(SceneDesc)]),
     "trace_scene_upload_mesh_device": (C.c_int, [_P, C.POINTER(MeshDeviceDesc), C.POINTER(C.c_int64)]),
     "trace_scene_attach_mesh_device": (C.c_int, [_P, C.POINTER(MeshDeviceDesc), C.POINTER(C.c_int64)]),
+    "trace_scene_attach_meshes_device": (C.c_int, [_P, C.c_int64, C.POINTER(C.POINTER(MeshDeviceDesc)), C.POINTER(C.c_int64)]),
     "trace_scene_refit": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int64, _P]),
     "trace_scene_refit_device": (C.c_int, [_P, C.c_int64, _P, _P, C.c_int64, _P]),
     "trace_scene_copy_nodes": (C.c_int, [_P, _P]),

@@ -379,6 +379,7 @@ int ctx_commit_scene(trace_ctx* c, int64_t n_nodes, int64_t n_prims, int64_t n_s
     B.n_nodes = n_nodes; B.n_pairs = n_pairs; B.n_prims = n_prims; B.n_tris = n_tris; B.n_spheres = n_spheres;
     B.shadow_depth = shadow ? depth : (n_prims == 1 ? 1 : 0);
     B.moved = false;
+    c->slots.clear();
     B.materials.swap(mats);
     B.lights.swap(lights);
     ctx_publish_scene(c, n_nodes, n_prims, n_spheres, (int64_t)B.materials.size(), (int64_t)B.lights.size(), n_tris, n_pairs,

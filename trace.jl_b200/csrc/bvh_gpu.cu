@@ -17,6 +17,8 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
+#include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
 
@@ -267,8 +269,9 @@ void core_reset(cudaStream_t s, int64_t n, Buffers& b) {
     if (n > 1) cudaMemsetAsync(b.arrive, 0, (size_t)(n - 1) * sizeof(uint32_t), s);
 }
 
-// build_core without the reset: what runs after core_reset (and anything that reports into the status block)
-int core_run(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, Status& hs, PhaseTimer& ph) {
+// build_core without the reset and the read-back: the kernels that run after core_reset (and anything that reports
+// into the status block).  LBVH_OK or LBVH_CUDA.
+int core_enqueue(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, PhaseTimer& ph) {
     const int T = 256;
     lbvh_centroid_box<<<(unsigned)std::min<int64_t>(blocks_for(n, T), 4096), T, 0, s>>>(b.pb, n, b.st);
     lbvh_keys<<<blocks_for(n, T), T, 0, s>>>(b.pb, n, b.st, b.keys, b.ids);
@@ -281,14 +284,24 @@ int core_run(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, St
     ph.mark(s, "hierarchy");
     lbvh_bottom_up<<<blocks_for(n, T), T, 0, s>>>(b.pb, b.ids_sorted, n, m, b.child, b.parent, b.count, b.arrive, b.box,
                                                    b.size, b.depth, b.st);
-    if (cudaGetLastError() != cudaSuccess ||
+    return cudaGetLastError() == cudaSuccess ? LBVH_OK : LBVH_CUDA;
+}
+
+// the core's verdict from its status block on the host
+int core_verdict(const Status& hs) {
+    if (hs.nan) return LBVH_NAN_BOUND;
+    if (hs.root_depth > TR_STACK_SIZE) return LBVH_TOO_DEEP;   // the walks' stacks would overflow
+    return LBVH_OK;
+}
+
+// core_enqueue, the status read back, its verdict
+int core_run(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, Status& hs, PhaseTimer& ph) {
+    if (core_enqueue(s, n, m, b, sort_bytes, ph) != LBVH_OK ||
         cudaMemcpyAsync(&hs, b.st, sizeof(Status), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
         cudaStreamSynchronize(s) != cudaSuccess)
         return LBVH_CUDA;
     ph.mark(s, "bottom-up");
-    if (hs.nan) return LBVH_NAN_BOUND;
-    if (hs.root_depth > TR_STACK_SIZE) return LBVH_TOO_DEEP;   // the walks' stacks would overflow
-    return LBVH_OK;
+    return core_verdict(hs);
 }
 
 int build_core(cudaStream_t s, int64_t n, int m, Buffers& b, size_t sort_bytes, Status& hs, PhaseTimer& ph) {
@@ -346,16 +359,17 @@ __global__ void lbvh_prim_bounds(const float4* __restrict__ prims, int64_t n, fl
 
 // One 64-byte pair record per internal node, in Karras numbering (the root is pair 0): both children's boxes, their
 // references (a pair index, or TR_REF_LEAF | primitive slot for a leaf, traverse.cuh) and the split axis as
-// a bit in the first half - the layout of the upload's pair records (api.cu).  Every reference is shifted by `shift`.
+// a bit in the first half - the layout of the upload's pair records (api.cu).  Pair references are shifted by
+// pair_shift, primitive slots by leaf_shift.
 __global__ void lbvh_emit_pairs(int64_t n, const uint32_t* __restrict__ child, const uint32_t* __restrict__ sorted_ids,
-                                const uint8_t* __restrict__ axis, const float* __restrict__ box, uint32_t shift,
-                                float4* __restrict__ pairs) {
+                                const uint8_t* __restrict__ axis, const float* __restrict__ box, uint32_t pair_shift,
+                                uint32_t leaf_shift, float4* __restrict__ pairs) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= n - 1) return;
     for (int k = 0; k < 2; ++k) {
         const int64_t v = child[2 * i + k];
         const float* bx = box + 6 * v;
-        const uint32_t ref = v < n - 1 ? shift + (uint32_t)v : (TR_REF_LEAF | (shift + sorted_ids[v - (n - 1)]));
+        const uint32_t ref = v < n - 1 ? pair_shift + (uint32_t)v : (TR_REF_LEAF | (leaf_shift + sorted_ids[v - (n - 1)]));
         const uint32_t extra = k == 0 ? (1u << axis[i]) : 0u;
         pairs[4 * i + 2 * k] = make_float4(bx[0], bx[1], bx[2], bx[3]);
         pairs[4 * i + 2 * k + 1] = make_float4(bx[4], bx[5], __uint_as_float(ref), __uint_as_float(extra));
@@ -408,35 +422,78 @@ size_t lbvh_scratch_bytes(int64_t n, cudaStream_t s) {
 // records `prims` (device, BVH slot order, triangles only), written as n - 1 pair records to `pairs` (device).  Nothing
 // crosses to the host but the build's status.  `scratch` (lbvh_scratch_bytes(n)) or nullptr: an allocation of its own.
 // Returns LBVH_OK, _NAN_BOUND (a NaN vertex), _TOO_DEEP or _CUDA; *depth (may be NULL): the tree's levels, root = 1.
-// ref_shift moves every reference: pairs and slots of a tree that starts at pair and slot ref_shift of a larger one.
+// pair_shift and leaf_shift move the references: a tree whose pairs start at pair pair_shift and whose primitives
+// start at slot leaf_shift of a larger one.
+namespace {
+// the shadow tree's bounds and core over `b`, no read-back
+int shadow_enqueue(cudaStream_t s, const void* prims, int64_t n, Buffers& b, size_t sort_bytes) {
+    lbvh_prim_bounds<<<blocks_for(n, 256), 256, 0, s>>>(static_cast<const float4*>(prims), n, b.pb);
+    core_reset(s, n, b);
+    PhaseTimer quiet;
+    return core_enqueue(s, n, 1, b, sort_bytes, quiet);
+}
+// after the status `hs` is on the host: its verdict, and the pair records when it is LBVH_OK
+int shadow_emit(cudaStream_t s, const Status& hs, int64_t n, Buffers& b, void* pairs, int* depth, uint32_t pair_shift,
+                uint32_t leaf_shift) {
+    if (const int rc = core_verdict(hs)) return rc;
+    lbvh_emit_pairs<<<blocks_for(n - 1, 256), 256, 0, s>>>(n, b.child, b.ids_sorted, b.axis, b.box, pair_shift, leaf_shift,
+                                                           static_cast<float4*>(pairs));
+    if (cudaGetLastError() != cudaSuccess) return LBVH_CUDA;
+    if (depth) *depth = (int)hs.root_depth;
+    return LBVH_OK;
+}
+}  // namespace
+
 int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs, void* scratch, int* depth,
-                      uint32_t ref_shift) {
+                      uint32_t pair_shift, uint32_t leaf_shift) {
     if (n < 2 || n >= 0x40000000ll) return 1;
     const size_t sort_bytes = sort_bytes_for(n, s);
     if (!sort_bytes) return LBVH_CUDA;
     Buffers b;
     if (scratch) b.borrow(scratch, n, sort_bytes);
     else if (b.alloc(n, sort_bytes, true, false)) return LBVH_CUDA;
-    const int T = 256;
-    lbvh_prim_bounds<<<blocks_for(n, T), T, 0, s>>>(static_cast<const float4*>(prims), n, b.pb);
-    PhaseTimer quiet;
     Status hs;
-    if (const int rc = build_core(s, n, 1, b, sort_bytes, hs, quiet)) return rc;
-    lbvh_emit_pairs<<<blocks_for(n - 1, T), T, 0, s>>>(n, b.child, b.ids_sorted, b.axis, b.box, ref_shift,
-                                                       static_cast<float4*>(pairs));
-    if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(s) != cudaSuccess) return LBVH_CUDA;
-    if (depth) *depth = (int)hs.root_depth;
-    return LBVH_OK;
+    if (shadow_enqueue(s, prims, n, b, sort_bytes) != LBVH_OK ||
+        cudaMemcpyAsync(&hs, b.st, sizeof(Status), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+        cudaStreamSynchronize(s) != cudaSuccess)
+        return LBVH_CUDA;
+    if (const int rc = shadow_emit(s, hs, n, b, pairs, depth, pair_shift, leaf_shift)) return rc;
+    return cudaStreamSynchronize(s) == cudaSuccess ? LBVH_OK : LBVH_CUDA;
+}
+
+size_t lbvh_status_bytes() { return sizeof(Status); }
+
+const void* lbvh_status(void* scratch, int64_t n) {
+    Buffers b;
+    b.borrow(scratch, n, 0);                               // (the status block sits before anything sized by the sort)
+    return b.st;
+}
+
+int shadow_tree_enqueue(cudaStream_t s, const void* prims, int64_t n, void* scratch) {
+    const size_t sort_bytes = sort_bytes_for(n, s);
+    if (n < 2 || !sort_bytes) return LBVH_CUDA;
+    Buffers b;
+    b.borrow(scratch, n, sort_bytes);
+    return shadow_enqueue(s, prims, n, b, sort_bytes);
+}
+
+int shadow_tree_emit(cudaStream_t s, const void* status, int64_t n, void* scratch, void* pairs, int* depth,
+                     uint32_t pair_shift, uint32_t leaf_shift) {
+    Status hs;
+    memcpy(&hs, status, sizeof(hs));
+    Buffers b;
+    b.borrow(scratch, n, sort_bytes_for(n, s));
+    return shadow_emit(s, hs, n, b, pairs, depth, pair_shift, leaf_shift);
 }
 
 // The tree of trace_scene_upload_mesh_device over `scratch` (lbvh_scratch_bytes(n), n >= 1): the status block reset,
 // normals (NULL: none) and material indices (NULL: all 0) checked into it, the triangles' boxes, then the LBVH core
-// and its status read back.  Returns LBVH_OK with *n_nodes and *order = the sorted triangle ids (slot -> triangle,
-// device, inside the scratch), or the first refusal in the order vertices, normals, materials, depth.  Nothing is
-// written outside the scratch before lbvh_mesh_emit (the preorder node records into `nodes`, device), so a refused
-// input leaves the caller's buffers intact.
-int lbvh_mesh_build(cudaStream_t s, const float* v, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n,
-                    int m, void* scratch, PhaseTimer& ph, int64_t* n_nodes, const uint32_t** order) {
+// and its status read back.  Returns LBVH_OK with *n_nodes, *depth (may be NULL: the tree's levels) and *order = the
+// sorted triangle ids (slot -> triangle, device, inside the scratch), or the first refusal in the order vertices,
+// normals, materials, depth.  Nothing is written outside the scratch before lbvh_mesh_emit (the preorder node records
+// into `nodes`, device), so a refused input leaves the caller's buffers intact.
+int lbvh_mesh_enqueue(cudaStream_t s, const float* v, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n,
+                      int m, void* scratch, PhaseTimer& ph) {
     const size_t sort_bytes = sort_bytes_for(n, s);
     if (!sort_bytes) return LBVH_CUDA;
     Buffers b;
@@ -449,17 +506,34 @@ int lbvh_mesh_build(cudaStream_t s, const float* v, const float* nrm, const uint
     lbvh_tri_bounds<<<blocks_for(n, T), T, 0, s>>>(v, n, b.pb);
     ph.mark(s, "bounds");
     PhaseTimer quiet;                                      // the core's own phases are not the upload's
-    Status hs;
-    const int rc = core_run(s, n, m, b, sort_bytes, hs, quiet);   // (its launch check covers the two kernels above)
+    const int rc = core_enqueue(s, n, m, b, sort_bytes, quiet);   // (its launch check covers the two kernels above)
     ph.mark(s, "build");
-    if (rc == LBVH_CUDA) return rc;
+    return rc;
+}
+
+int lbvh_mesh_result(const void* status, void* scratch, int64_t n, int64_t* n_nodes, const uint32_t** order, int* depth) {
+    Status hs;
+    memcpy(&hs, status, sizeof(hs));
     if (hs.nan) return LBVH_NAN_BOUND;
     if (hs.bad & 1u) return LBVH_NAN_NORMAL;
     if (hs.bad & 2u) return LBVH_BAD_MATERIAL;
-    if (rc) return rc;
+    if (const int rc = core_verdict(hs)) return rc;
+    Buffers b;
+    b.borrow(scratch, n, 0);                               // (ids_sorted sits before the sort's temp)
     *n_nodes = hs.root_size;
     *order = b.ids_sorted;
+    if (depth) *depth = (int)hs.root_depth;
     return LBVH_OK;
+}
+
+int lbvh_mesh_build(cudaStream_t s, const float* v, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n,
+                    int m, void* scratch, PhaseTimer& ph, int64_t* n_nodes, const uint32_t** order, int* depth) {
+    if (lbvh_mesh_enqueue(s, v, nrm, mat, n_materials, n, m, scratch, ph) != LBVH_OK) return LBVH_CUDA;
+    std::vector<char> hs(lbvh_status_bytes());
+    if (cudaMemcpyAsync(hs.data(), lbvh_status(scratch, n), hs.size(), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+        cudaStreamSynchronize(s) != cudaSuccess)
+        return LBVH_CUDA;
+    return lbvh_mesh_result(hs.data(), scratch, n, n_nodes, order, depth);
 }
 
 int lbvh_mesh_emit(cudaStream_t s, int64_t n, int m, void* scratch, void* nodes, uint32_t node_shift, uint32_t prim_shift) {

@@ -133,15 +133,26 @@ struct trace_ctx {
     // trace_scene_upload_mesh_device (upload_device.cu): the LBVH build's scratch, then the pair numbering's and the
     // shadow tree build's (grow-only, so a per-frame rebuild of the same size allocates nothing)
     DevBuf b_build;
-    // trace_scene_attach_mesh_device (upload_device.cu): the base, the scene of the last upload, stays resident while
+    // trace_scene_attach_meshes_device (upload_device.cu): the base, the scene of the last upload, stays resident while
     // meshes are attached to it.  After the first attach its node, pair and shadow-pair records sit one slot up.
     struct Base {
         int64_t n_nodes = 0, n_pairs = 0, n_prims = 0, n_tris = 0, n_spheres = 0;
-        std::vector<DeviceMaterial> materials;   // packed at upload: each attach puts base ++ mesh again
+        std::vector<DeviceMaterial> materials;   // packed at upload: each attach puts base ++ meshes again
         std::vector<DeviceLight> lights;
         int shadow_depth = 0;     // levels of its shadow tree (1: a single primitive, no pair); 0: none usable
         bool moved = false;       // its records sit one slot up (an attach ran since the upload)
     } base;
+    // the meshes attached to the base, in slot order (cleared by every upload): their sizes, packed materials and
+    // lights, and where the composed scene holds their records
+    struct Slot {
+        int64_t n_tris = 0, n_nodes = 0, n_pairs = 0;
+        int node_depth = 0;       // levels of its LBVH (a kept mesh must still fit the stack under a larger top tree)
+        std::vector<DeviceMaterial> materials;
+        std::vector<DeviceLight> lights;
+        int shadow_depth = 0;     // as Base::shadow_depth (0 also: not built, left behind by a move, or stale after a refit)
+        int64_t node = 0, pair = 0, prim = 0, shadow = 0, tri = 0, material = 0;   // first node, pair, primitive slot, shadow pair, triangle, material
+    };
+    std::vector<Slot> slots;
 
     // refit (refit.cu): what trace_scene_refit needs of the last upload.  The host keeps only the BVH-slot -> triangle
     // map; the device topology (parents, pair slots, leaf list) is derived from b_nodes at the first refit after an
@@ -407,15 +418,28 @@ enum LbvhStatus {
     LBVH_BAD_MATERIAL = 9,       // mesh builds: a material index out of range
 };
 // The shadow tree over uploaded primitive records, in `scratch` (lbvh_scratch_bytes(n) bytes) or, with nullptr, an
-// allocation of its own: LBVH_OK, _NAN_BOUND, _TOO_DEEP or _CUDA; *depth (may be NULL) its levels.  Every reference
-// it writes is shifted by ref_shift (an attach's mesh part: its pairs and primitive slots start there).
+// allocation of its own: LBVH_OK, _NAN_BOUND, _TOO_DEEP or _CUDA; *depth (may be NULL) its levels.  Pair references
+// are shifted by pair_shift and primitive slots by leaf_shift (an attached mesh's part: where its shadow pairs and its
+// primitives start).
 int shadow_tree_build(cudaStream_t s, const void* prims, int64_t n, void* pairs, void* scratch, int* depth = nullptr,
-                      uint32_t ref_shift = 0);
+                      uint32_t pair_shift = 0, uint32_t leaf_shift = 0);
 size_t lbvh_scratch_bytes(int64_t n, cudaStream_t s);
+// The same builds in two halves, so that a caller with several builds reads their status blocks back once: the
+// *_enqueue half runs every kernel (LBVH_OK or LBVH_CUDA); lbvh_status is the device address of the build's status
+// block in `scratch` (lbvh_status_bytes bytes); the second half takes that block once it is on the host and returns
+// what the one-call function returns (shadow_tree_emit then writes the pair records).
+size_t lbvh_status_bytes();
+const void* lbvh_status(void* scratch, int64_t n);
+int shadow_tree_enqueue(cudaStream_t s, const void* prims, int64_t n, void* scratch);
+int shadow_tree_emit(cudaStream_t s, const void* status, int64_t n, void* scratch, void* pairs, int* depth,
+                     uint32_t pair_shift, uint32_t leaf_shift);
 // The tree of trace_scene_upload_mesh_device, in `scratch`: lbvh_mesh_build validates, bounds and builds (phases
 // "validate", "bounds" and "build" of `ph`); lbvh_mesh_emit, once the input is accepted, writes the node records.
 int lbvh_mesh_build(cudaStream_t s, const float* v, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n,
-                    int m, void* scratch, PhaseTimer& ph, int64_t* n_nodes, const uint32_t** order);
+                    int m, void* scratch, PhaseTimer& ph, int64_t* n_nodes, const uint32_t** order, int* depth = nullptr);
+int lbvh_mesh_enqueue(cudaStream_t s, const float* v, const float* nrm, const uint32_t* mat, int64_t n_materials, int64_t n,
+                      int m, void* scratch, PhaseTimer& ph);
+int lbvh_mesh_result(const void* status, void* scratch, int64_t n, int64_t* n_nodes, const uint32_t** order, int* depth);
 // Interior offsets are shifted by node_shift and leaf offsets by prim_shift (both 0 for an upload).
 int lbvh_mesh_emit(cudaStream_t s, int64_t n, int m, void* scratch, void* nodes, uint32_t node_shift = 0,
                    uint32_t prim_shift = 0);

@@ -310,8 +310,12 @@ int refit_run(trace_ctx* c, int64_t n_tris, const float* v, const float* nrm, bo
     TR_CUDA(c, cudaStreamSynchronize(c->stream));
     ph.mark(c->stream, "readback");
     if (nan) return c->fail("scene refit: NaN in the new vertices or normals (the scene is unchanged)");
-    // a composed scene without a shadow tree left the base's shadow pairs with the old boxes: later attaches get none
-    if (c->base.moved && !c->scene.shadow_pairs && c->base.shadow_depth > 1) c->base.shadow_depth = 0;
+    // a composed scene without a shadow tree left the base's and the meshes' shadow pairs with the old boxes: later
+    // attaches get none while one of those parts is in the scene
+    if (c->base.moved && !c->scene.shadow_pairs) {
+        if (c->base.shadow_depth > 1) c->base.shadow_depth = 0;
+        for (auto& sl : c->slots) if (sl.shadow_depth > 1) sl.shadow_depth = 0;
+    }
     if (n_nodes > 0) {                                     // the upload's rule (api.cu)
         const float b[6] = {root[0].x, root[0].y, root[0].z, root[0].w, root[1].x, root[1].y};
         float scale = 0.0f;

@@ -174,7 +174,16 @@ class Context:
         self._scene = None
         self._n_nodes = 0
         self._base = None         # the FlatScene of the last trace_scene_upload (the attach base), or None
-        self._mesh = None         # the DeviceMeshScene attached to it, or None
+        self._meshes = []         # the DeviceMeshScenes attached to it, slot by slot
+
+    @property
+    def _mesh(self):
+        """the DeviceMeshScene attached to the base when there is exactly one, else None"""
+        return self._meshes[0] if len(self._meshes) == 1 else None
+
+    @_mesh.setter
+    def _mesh(self, mesh):
+        self._meshes = [] if mesh is None else [mesh]
 
     def check(self, rc):
         if rc != 0:
@@ -204,15 +213,16 @@ class Context:
         if isinstance(scene, DeviceMeshScene):
             if self._scene is not scene:
                 self._scene, self._n_nodes = scene, self._mesh_call(self.lib.trace_scene_upload_mesh_device, scene)
-                self._base, self._mesh = None, None
+                self._base, self._meshes = None, []
             return scene
         if isinstance(scene, CompositeScene):
             flat = scene.scene.flatten()
             if self._base is not flat:
                 self._upload_flat(flat)
-            if self._mesh is not scene.mesh:
-                self._n_nodes = self._mesh_call(self.lib.trace_scene_attach_mesh_device, scene.mesh)
-                self._mesh = scene.mesh
+            keep = [j < len(self._meshes) and self._meshes[j] is m for j, m in enumerate(scene.meshes)]
+            if not all(keep) or len(scene.meshes) != len(self._meshes):
+                self._n_nodes = self._attach([None if k else m for k, m in zip(keep, scene.meshes)])
+                self._meshes = list(scene.meshes)
             self._scene = scene
             return scene
         flat = scene.flatten()
@@ -228,16 +238,26 @@ class Context:
         d = flat.desc()
         self.check(self.lib.trace_scene_upload(self.h, C.byref(d)))
         self._scene, self._n_nodes = flat, len(flat.nodes)
-        self._base, self._mesh = flat, None
+        self._base, self._meshes = flat, []
 
     def _mesh_call(self, fn, scene):
-        """trace_scene_upload_mesh_device / trace_scene_attach_mesh_device of a DeviceMeshScene's device arrays: -> the
-        scene's node count"""
+        """trace_scene_upload_mesh_device of a DeviceMeshScene's device arrays: -> the scene's node count"""
         d, keep = scene.desc(self.device)
         import torch
         torch.cuda.current_stream(self.device).synchronize()       # the work that wrote the arrays is done
         n_nodes = C.c_int64()
         self.check(fn(self.h, C.byref(d), C.byref(n_nodes)))
+        return n_nodes.value
+
+    def _attach(self, meshes):
+        """trace_scene_attach_meshes_device with a descriptor for each DeviceMeshScene of `meshes` and NULL (keep the
+        slot) for each None: -> the composed scene's node count"""
+        descs = [None if m is None else m.desc(self.device) for m in meshes]
+        arr = (C.POINTER(_lib.MeshDeviceDesc) * len(meshes))(*[C.pointer(d[0]) if d else None for d in descs])
+        import torch
+        torch.cuda.current_stream(self.device).synchronize()       # the work that wrote the arrays is done
+        n_nodes = C.c_int64()
+        self.check(self.lib.trace_scene_attach_meshes_device(self.h, len(meshes), arr, C.byref(n_nodes)))
         return n_nodes.value
 
     def refit(self, scene, vertices=None, normals=None):
@@ -252,14 +272,15 @@ class Context:
         A DeviceMeshScene: `vertices` in its triangle order; None re-reads the scene's own tensors (vertices, and
         normals if it has them) after the caller changed them in place.
         A CompositeScene: `vertices` (required) of all triangles, the environment's (in the order of its flattening)
-        followed by the mesh's; afterwards the environment's FlatScene is stale as above."""
+        followed by the meshes' in slot order; afterwards the environment's FlatScene is stale as above."""
         if isinstance(scene, CompositeScene):
             flat = scene.scene.flatten() if scene.scene._flat is not None else None
-            if flat is None or flat is not self._base or scene.mesh is not self._mesh:
+            if (flat is None or flat is not self._base or len(scene.meshes) != len(self._meshes) or
+                    any(a is not b for a, b in zip(scene.meshes, self._meshes))):
                 raise ValueError("refit: this scene is not the one uploaded to this context")
             if vertices is None:
                 raise ValueError("refit: a CompositeScene needs the vertices of all its triangles")
-            n = len(flat.tri_vertices) + scene.mesh.n_tris
+            n = len(flat.tri_vertices) + sum(m.n_tris for m in scene.meshes)
             sb = np.ascontiguousarray(flat.sphere_bounds, dtype=np.float32)
         elif isinstance(scene, DeviceMeshScene):
             if scene is not self._scene:

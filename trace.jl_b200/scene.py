@@ -580,27 +580,42 @@ class DeviceMeshScene:
 
 
 class CompositeScene:
-    """A Scene (the environment) with a DeviceMeshScene attached to it (extension: the reference has no counterpart).
-    Context.upload uploads `scene` once and attaches `mesh` on the GPU (trace_scene_attach_mesh_device): each new mesh
-    rebuilds only the mesh's tree, whatever the environment holds (analytic spheres, nested BVHAccels, a reference or
-    sah tree).  The device scene is the one Scene(lights, BVHAccel) uploads when its root has the environment's tree as
-    first child and the mesh's as second: the mesh's triangles come after the environment's (queries report mesh
-    triangle i as the environment's primitive count + i), its materials and lights after the environment's.
+    """A Scene (the environment) with DeviceMeshScenes attached to it (extension: the reference has no counterpart).
+    `mesh` is one DeviceMeshScene or an iterable of 1 to 64 of them, the slots in order.  Context.upload uploads
+    `scene` once and attaches the meshes on the GPU (trace_scene_attach_meshes_device): each new mesh object rebuilds
+    only that mesh's tree, whatever the environment holds (analytic spheres, nested BVHAccels, a reference or sah tree).
+    The device scene is the one Scene(lights, BVHAccel) uploads when its root has the environment's tree as first child
+    and a balanced tree over the meshes' trees, in slot order, as second: the meshes' triangles come after the
+    environment's in slot order (queries report triangle i of mesh j as the environment's primitive count + the
+    triangles of meshes 0 .. j - 1 + i), their materials and lights after the environment's.
 
-    Context.upload caches by identity: the environment is uploaded again only when its flattening changed, the mesh is
-    attached again only when `mesh` is a new object.  To move triangles use Context.refit with the vertices of all
-    triangles, the environment's first."""
+    Context.upload caches by identity: the environment is uploaded again only when its flattening changed, a slot is
+    rebuilt only when it holds a new object.  To move triangles use Context.refit with the vertices of all triangles,
+    the environment's first, then the meshes' in slot order.  `mesh` is the mesh when there is exactly one, else None."""
+
+    MAX_MESHES = 64
 
     def __init__(self, scene, mesh):
         if not isinstance(scene, Scene):
             raise ValueError(f"scene must be a Scene, got {type(scene).__name__}")
-        if not isinstance(mesh, DeviceMeshScene):
-            raise ValueError(f"mesh must be a DeviceMeshScene, got {type(mesh).__name__}")
-        if mesh.n_tris == 0:
-            raise ValueError("mesh must hold at least one triangle")
-        self.scene, self.mesh = scene, mesh
-        self.lights = scene.lights + mesh.lights
-        self.bound = scene.bound.union(mesh.bound)
+        single = isinstance(mesh, DeviceMeshScene)
+        try:
+            meshes = (mesh,) if single else tuple(mesh)
+        except TypeError:
+            raise ValueError(f"mesh must be a DeviceMeshScene, got {type(mesh).__name__}") from None
+        if not 1 <= len(meshes) <= self.MAX_MESHES:
+            raise ValueError(f"meshes: between 1 and {self.MAX_MESHES} DeviceMeshScenes, got {len(meshes)}")
+        for j, m in enumerate(meshes):
+            if not isinstance(m, DeviceMeshScene):
+                raise ValueError(f"mesh must be a DeviceMeshScene, got {type(m).__name__}" + ("" if single else f" (mesh {j})"))
+            if m.n_tris == 0:
+                raise ValueError("mesh must hold at least one triangle" + ("" if single else f" (mesh {j})"))
+        self.scene, self.meshes = scene, meshes
+        self.mesh = meshes[0] if len(meshes) == 1 else None
+        self.lights = scene.lights + [l for m in meshes for l in m.lights]
+        self.bound = scene.bound
+        for m in meshes:
+            self.bound = self.bound.union(m.bound)
 
     @property
     def has_unshaded(self):
